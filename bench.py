@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- the headline benchmark of BASELINE.json, on N GPUs of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Metric (BASELINE.json): "STFT+ISTFT Msamples/s at nfft=2048 hop=512".  One step = one pass
@@ -22,6 +22,11 @@ for B = 1024 signals x 10 s @ 48 kHz per GPU, valid frames only (934 per signal)
           box's host cores, bounded sample
 Multi-GPU: signals are sharded by signal across ranks, no collective on the data path
 (weak scaling: every rank owns B signals).  --impl reference times the CPU reference.
+
+--dump-outputs DIR writes what the last timed step returned on rank 0, for comparing two builds
+output for output (the inputs are seeded, so the same arguments give the same inputs): a fixed,
+seeded sample of DUMP_SIGNALS signals, as DIR/spectra.npy (float32 [signals][934][1025][2], real
+and imaginary parts) and DIR/reconstruction.npy (float32 [signals][480000]), 57.5 MB in all.
 """
 from __future__ import annotations
 
@@ -43,6 +48,19 @@ METRIC = "STFT+ISTFT Msamples/s at nfft=2048 hop=512"
 UNIT = "Msamples/s"
 WORKLOAD = ("configs[1]+[2]: batched STFT -> complex half spectra -> batched ISTFT (OLA, window-sum normalised), "
             "1024 synthetic mono signals x 10 s @48 kHz per GPU, nfft=2048 hop=512 Hann, 934 valid frames/signal")
+DUMP_SIGNALS, DUMP_SEED = 6, 0      # 6 x (7.66 MB spectra + 1.92 MB signal) stays under 64 MB
+
+
+def dump_outputs(out_dir, spec, y):
+    """The timed path's outputs for a fixed, seeded sample of signals, as float32 .npy files under out_dir."""
+    import numpy as np
+    import torch
+    B = spec.shape[0]
+    rows = np.sort(np.random.default_rng(DUMP_SEED).choice(B, min(B, DUMP_SIGNALS), replace=False))
+    idx = torch.as_tensor(rows, device=spec.device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "spectra.npy"), torch.view_as_real(spec.index_select(0, idx)).cpu().numpy())
+    np.save(os.path.join(out_dir, "reconstruction.npy"), y.index_select(0, idx).cpu().numpy())
 
 
 def measured_peaks():
@@ -243,7 +261,13 @@ def main():
     ap.add_argument("--e2e-steps", type=int, default=None)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-stream", action="store_true", help="skip the config-4 single-stream leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's spectra and reconstructed signals (seeded sample) to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -329,6 +353,8 @@ def main():
 
     # ---- sanity inside the bench: the timed outputs are the real thing (round trip on the interior)
     err = float(torch.linalg.vector_norm((y - x)[:, NFFT:-NFFT].double()) / torch.linalg.vector_norm(x[:, NFFT:-NFFT].double()))
+    if args.dump_outputs and rank == 0:             # before the legs below reuse spec
+        dump_outputs(args.dump_outputs, spec, y)
 
     # ---- power-spectrum variant (configs[1] as literally stated), device-resident, for the record
     pw = torch.empty((B, FRAMES, BINS), device=dev, dtype=torch.float32)

@@ -20,11 +20,9 @@ def oracle():
 
 @pytest.fixture(scope="session")
 def reference():
-    """The unmodified reference library; present where oracle/_ref was built (or travelled)."""
+    """The unmodified reference library where oracle/_ref was built (see oracle/Makefile), else None."""
     from oracle.oracle import Reference
-    if not Reference.available():
-        pytest.skip("oracle/_ref/libvvdsp_ref.so not built (no /root/reference here)")
-    return Reference()
+    return Reference() if Reference.available() else None
 
 
 @pytest.fixture(scope="session")

@@ -1,10 +1,14 @@
 """CPU tests (-m "not gpu"): pin the oracle restatement.
 
  (a) against sha256 digests and slices generated from the real reference (tests/golden/),
- (b) live, bit for bit, against oracle/_ref/libvvdsp_ref.so where it exists,
+ (b) bit for bit against the reference's outputs: digests recorded from it (tests/golden/reference_digests.json),
+     and live against oracle/_ref/libvvdsp_ref.so where it was built,
  (c) against the known answers in the reference's own tests (cited per test),
  (d) its accuracy envelope vs float64 (SURVEY.md section 8c).
 """
+import json
+import os
+
 import numpy as np
 import pytest
 
@@ -83,29 +87,130 @@ def test_golden_config1_voicebank(oracle, golden):
     assert rel_l2(y[1024:-1024], wav[1024:-1024]) < 5e-6
 
 
-# ------------------------------------------------------------------ (b) live vs reference
-@pytest.mark.parametrize("nfft,hop,win", [(2048, 512, "hann"), (1024, 256, "hamming"), (96, 40, "hann"), (8, 3, "boxcar")])
-def test_live_against_reference(oracle, reference, nfft, hop, win):
+# ------------------------------------------------------------------ (b) bit for bit vs reference
+# Each case is (key, what the oracle computes, what the reference library computes from the same input).  Where
+# oracle/_ref was built the reference side runs live; the oracle's result must also equal the sha256 digest (or status
+# code) recorded from the reference under that key in tests/golden/reference_digests.json, so that the comparison
+# holds in every checkout.
+def bits(v):
+    return int(v) if isinstance(v, (int, np.integer)) else sha(v)
+
+
+def check_against_reference(oracle, reference, recorded, cases):
+    for key, mine, theirs in cases:
+        got = bits(mine(oracle))
+        assert got == recorded[key], key
+        if reference is not None:
+            assert got == bits(theirs(reference)), key
+
+
+LIVE_STFT = [(2048, 512, "hann"), (1024, 256, "hamming"), (96, 40, "hann"), (8, 3, "boxcar")]
+
+
+def stft_cases(oracle, nfft, hop, win):
+    k = f"stft_n{nfft}_h{hop}_{win}/"
     x = np.stack([noise(100 + i, 6000) for i in range(3)])
-    assert oracle.batch_forward(x, nfft, hop, win).tobytes() == reference.batch_forward(x, nfft, hop, win, threads=2).tobytes()
-    assert oracle.batch_roundtrip(x, nfft, hop, win, threads=3).tobytes() == reference.batch_roundtrip(x, nfft, hop, win).tobytes()
-    assert oracle.batch_power(x, nfft, hop, win).tobytes() == reference.batch_power(x, nfft, hop, win).tobytes()
+    yield k + "batch_forward", lambda o: o.batch_forward(x, nfft, hop, win), lambda r: r.batch_forward(x, nfft, hop, win, threads=2)
+    yield k + "batch_roundtrip", lambda o: o.batch_roundtrip(x, nfft, hop, win, threads=3), lambda r: r.batch_roundtrip(x, nfft, hop, win)
+    yield k + "batch_power", lambda o: o.batch_power(x, nfft, hop, win), lambda r: r.batch_power(x, nfft, hop, win)
     for conv in ("valid", "spectrogram", "padded_tail", "center"):
-        a = oracle.stft(x[0, :1500], nfft, hop, win, convention=conv)
-        b = reference.stft(x[0, :1500], nfft, hop, win, convention=conv)
-        assert a.tobytes() == b.tobytes(), conv
+        yield (k + "stft_" + conv, lambda o, c=conv: o.stft(x[0, :1500], nfft, hop, win, convention=c),
+               lambda r, c=conv: r.stft(x[0, :1500], nfft, hop, win, convention=c))
     s = oracle.stft(x[1], nfft, hop, win)
     for norm in (True, False):
-        assert oracle.istft(s, nfft, hop, 6000, win, normalise=norm).tobytes() == \
-            reference.istft(s, nfft, hop, 6000, win, normalise=norm).tobytes()
+        yield (k + f"istft_normalise{int(norm)}", lambda o, m=norm: o.istft(s, nfft, hop, 6000, win, normalise=m),
+               lambda r, m=norm: r.istft(s, nfft, hop, 6000, win, normalise=m))
     f = noise(7, nfft)
-    assert oracle.process(f, nfft, hop, win).tobytes() == reference.process(f, nfft, hop, win).tobytes()
+    yield k + "process", lambda o: o.process(f, nfft, hop, win), lambda r: r.process(f, nfft, hop, win)
 
 
-def test_live_status_codes(oracle, reference):
-    """src/spectral/stft.c:31-34,21-28: NULL->1 (not reachable here), sizes->2, bad enum->3."""
+def status_cases(oracle):
     for args in [(0, 1, 1), (8, 0, 1), (8, 9, 1), (8, 4, 7), (2, 1, 0), (8, 8, 2)]:
-        assert oracle.create_status(*args) == reference.create_status(*args), args
+        yield "create_status_{}_{}_{}".format(*args), lambda o, a=args: o.create_status(*a), lambda r, a=args: r.create_status(*a)
+
+
+MEL_ARGS = [(2048, 80, 48000.0, 0.0, 24000.0), (2048, 128, 48000.0, 20.0, 20000.0), (1024, 40, 44100.0, 0.0, 22050.0),
+            (512, 26, 16000.0, 300.0, 8000.0)]
+MEL_BAD_ARGS = [(0, 10, 48000.0, 0.0, 100.0), (512, 0, 48000.0, 0.0, 100.0), (512, 300, 48000.0, 0.0, 100.0),
+                (512, 10, 48000.0, 0.0, 30000.0), (512, 10, 48000.0, 100.0, 50.0), (512, 10, 48000.0, 0.0, 8000.0, 1)]
+
+
+def mel_cases(oracle):
+    for args in MEL_ARGS:
+        k = "mel_n{}_m{}_sr{:g}_{:g}_{:g}/".format(*args)
+        yield k + "status", lambda o, a=args: o.mel_filterbank(*a)[0], lambda r, a=args: r.mel_filterbank(*a)[0]
+        yield k + "weights", lambda o, a=args: o.mel_filterbank(*a)[1], lambda r, a=args: r.mel_filterbank(*a)[1]
+        p = np.random.default_rng(1).uniform(0, 10, (5, args[0] // 2 + 1)).astype(np.float32)
+        yield (k + "log_mel", lambda o, a=args, p=p: o.log_mel(p, o.mel_filterbank(*a)[1], 1e-10),
+               lambda r, a=args, p=p: r.log_mel(p, r.mel_filterbank(*a)[1], 1e-10))
+    for bad in MEL_BAD_ARGS:
+        yield ("mel_bad_" + "_".join(f"{v:g}" for v in bad), lambda o, a=bad: o.mel_filterbank(*a)[0],
+               lambda r, a=bad: r.mel_filterbank(*a)[0])
+
+
+def mfcc_cases(oracle):
+    rng = np.random.default_rng(5)
+    for n_mels, n_coeffs, lifter in ((80, 13, 0.0), (40, 40, 22.0), (26, 12, 22.0), (7, 1, 3.5)):
+        lm = rng.normal(-3, 4, (17, n_mels)).astype(np.float32)
+        k = f"mfcc_m{n_mels}_c{n_coeffs}_l{lifter:g}/"
+        yield k + "status", lambda o, a=(lm, n_coeffs, lifter): o.mfcc(*a)[0], lambda r, a=(lm, n_coeffs, lifter): r.mfcc(*a)[0]
+        yield k + "coeffs", lambda o, a=(lm, n_coeffs, lifter): o.mfcc(*a)[1], lambda r, a=(lm, n_coeffs, lifter): r.mfcc(*a)[1]
+    lm = np.zeros((2, 8), np.float32)
+    for bad in ((0, 0.0, 2), (9, 0.0, 2), (4, -1.0, 2), (4, 0.0, 3), (4, 0.0, 4)):
+        yield "mfcc_bad_{}_{:g}_{}".format(*bad), lambda o, a=bad: o.mfcc(lm, *a)[0], lambda r, a=bad: r.mfcc(lm, *a)[0]
+    p = rng.uniform(0, 5, (9, 257)).astype(np.float32)
+    w = oracle.mel_filterbank(512, 40, 16000.0, 0.0, 8000.0)[1]
+    plan = (p, 512, 40, 13, 16000.0, 0.0, 8000.0, 22.0, 1e-10)
+    yield "mfcc_plan/status", lambda o: o.mfcc(o.log_mel(p, w, 1e-10), 13, 22.0)[0], lambda r: r.mfcc_plan_process(*plan)[0]
+    yield "mfcc_plan/coeffs", lambda o: o.mfcc(o.log_mel(p, w, 1e-10), 13, 22.0)[1], lambda r: r.mfcc_plan_process(*plan)[1]
+
+
+def write_wav(path, raw, fmt, channels, rate=48000):
+    import struct
+    bits = abs(fmt)
+    tag = 3 if fmt < 0 else 1
+    block = channels * bits // 8
+    hdr = b"RIFF" + struct.pack("<I", 36 + len(raw)) + b"WAVEfmt " + struct.pack("<IHHIIHH", 16, tag, channels, rate, rate * block,
+                                                                                 block, bits) + b"data" + struct.pack("<I", len(raw))
+    with open(path, "wb") as f:
+        f.write(hdr + raw)
+
+
+def pcm_cases(oracle, tmp_dir):
+    rng = np.random.default_rng(3)
+    for fmt in (16, 24, 32, -32):
+        for channels in (1, 2):
+            n = 1001
+            if fmt == -32:
+                raw = rng.uniform(-1, 1, n * channels).astype("<f4").tobytes()
+            elif fmt == 24:
+                v = rng.integers(-2**23, 2**23, n * channels, dtype=np.int64)
+                v[:4] = [-2**23, 2**23 - 1, -1, 0]
+                raw = b"".join(int(q & 0xFFFFFF).to_bytes(3, "little") for q in v)
+            else:
+                lim = 2 ** (fmt - 1)
+                v = rng.integers(-lim, lim, n * channels, dtype=np.int64)
+                v[:4] = [-lim, lim - 1, -1, 0]
+                raw = v.astype("<i2" if fmt == 16 else "<i4").tobytes()
+            path = os.path.join(tmp_dir, f"t_{fmt}_{channels}.wav")
+            write_wav(path, raw, fmt, channels)
+            yield (f"pcm_{fmt}_{channels}ch", lambda o, a=(raw, fmt, channels): o.pcm_to_planar(*a),
+                   lambda r, p=path: r.wav_read(p))
+
+
+@pytest.fixture(scope="module")
+def recorded():
+    return json.load(open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_digests.json")))["digests"]
+
+
+@pytest.mark.parametrize("nfft,hop,win", LIVE_STFT)
+def test_live_against_reference(oracle, reference, recorded, nfft, hop, win):
+    check_against_reference(oracle, reference, recorded, stft_cases(oracle, nfft, hop, win))
+
+
+def test_live_status_codes(oracle, reference, recorded):
+    """src/spectral/stft.c:31-34,21-28: NULL->1 (not reachable here), sizes->2, bad enum->3."""
+    check_against_reference(oracle, reference, recorded, status_cases(oracle))
     assert oracle.create_status(0, 1, 1) == 2 and oracle.create_status(8, 9, 1) == 2
     assert oracle.create_status(8, 4, 7) == 3 and oracle.create_status(2, 1, 0) == 0
 
@@ -232,75 +337,23 @@ def test_oracle_accuracy_envelope(oracle, nfft, bound):
 
 
 # ------------------------------------------------------------------ groundwork for SURVEY.md 8(f) rank 2
-def test_mel_oracle_against_reference(oracle, reference):
+def test_mel_oracle_against_reference(oracle, reference, recorded):
     """The mel filterbank / log-mel restatement (src/features/mel.c:14-245) is bit-exact against the
-    compiled reference; the GPU side of this row is not built yet (DESIGN.md section 7)."""
-    if not hasattr(reference.lib, "vv_dsp_mel_filterbank_create"):
-        pytest.skip("oracle/_ref was built without mel.c")
-    for args in [(2048, 80, 48000.0, 0.0, 24000.0), (2048, 128, 48000.0, 20.0, 20000.0), (1024, 40, 44100.0, 0.0, 22050.0),
-                 (512, 26, 16000.0, 300.0, 8000.0)]:
+    compiled reference."""
+    check_against_reference(oracle, reference, recorded, mel_cases(oracle))
+    for args in MEL_ARGS:
         so, wo = oracle.mel_filterbank(*args)
-        sr, wr = reference.mel_filterbank(*args)
-        assert so == sr == 0 and wo.tobytes() == wr.tobytes(), args
-        assert np.allclose(wo.sum(axis=1), 1.0, atol=1e-5)
-        p = np.random.default_rng(1).uniform(0, 10, (5, args[0] // 2 + 1)).astype(np.float32)
-        assert oracle.log_mel(p, wo, 1e-10).tobytes() == reference.log_mel(p, wr, 1e-10).tobytes()
-    for bad in [(0, 10, 48000.0, 0.0, 100.0), (512, 0, 48000.0, 0.0, 100.0), (512, 300, 48000.0, 0.0, 100.0),
-                (512, 10, 48000.0, 0.0, 30000.0), (512, 10, 48000.0, 100.0, 50.0), (512, 10, 48000.0, 0.0, 8000.0, 1)]:
-        assert oracle.mel_filterbank(*bad)[0] == reference.mel_filterbank(*bad)[0], bad
+        assert so == 0 and np.allclose(wo.sum(axis=1), 1.0, atol=1e-5), args
 
 
-def test_mfcc_oracle_against_reference(oracle, reference):
+def test_mfcc_oracle_against_reference(oracle, reference, recorded):
     """orc_mfcc (DCT-II of src/spectral/dct.c:21-30 + liftering, src/features/mel.c:249-310) is bit-exact against the
     reference, and so is the plan pipeline power -> log-mel -> MFCC (mel.c:333-450) rebuilt from the oracle's pieces."""
-    if not hasattr(reference.lib, "vv_dsp_mfcc"):
-        pytest.skip("oracle/_ref was built without mel.c")
-    rng = np.random.default_rng(5)
-    for n_mels, n_coeffs, lifter in ((80, 13, 0.0), (40, 40, 22.0), (26, 12, 22.0), (7, 1, 3.5)):
-        lm = rng.normal(-3, 4, (17, n_mels)).astype(np.float32)
-        so, co = oracle.mfcc(lm, n_coeffs, lifter)
-        sr, cr = reference.mfcc(lm, n_coeffs, lifter)
-        assert so == sr == 0 and co.tobytes() == cr.tobytes(), (n_mels, n_coeffs, lifter)
-    lm = np.zeros((2, 8), np.float32)
-    for bad in ((0, 0.0, 2), (9, 0.0, 2), (4, -1.0, 2), (4, 0.0, 3), (4, 0.0, 4)):
-        assert oracle.mfcc(lm, bad[0], bad[1], bad[2])[0] == reference.mfcc(lm, bad[0], bad[1], bad[2])[0], bad
-    p = rng.uniform(0, 5, (9, 257)).astype(np.float32)
-    st, ref = reference.mfcc_plan_process(p, 512, 40, 13, 16000.0, 0.0, 8000.0, 22.0, 1e-10)
-    _, w = oracle.mel_filterbank(512, 40, 16000.0, 0.0, 8000.0)
-    st2, mine = oracle.mfcc(oracle.log_mel(p, w, 1e-10), 13, 22.0)
-    assert st == st2 == 0 and mine.tobytes() == ref.tobytes()
+    check_against_reference(oracle, reference, recorded, mfcc_cases(oracle))
+    assert all(mine(oracle) == 0 for key, mine, _ in mfcc_cases(oracle) if key.endswith("/status"))
 
 
-def _write_wav(path, raw, fmt, channels, rate=48000):
-    import struct
-    bits = abs(fmt)
-    tag = 3 if fmt < 0 else 1
-    block = channels * bits // 8
-    hdr = b"RIFF" + struct.pack("<I", 36 + len(raw)) + b"WAVEfmt " + struct.pack("<IHHIIHH", 16, tag, channels, rate, rate * block,
-                                                                                 block, bits) + b"data" + struct.pack("<I", len(raw))
-    path.write_bytes(hdr + raw)
-
-
-def test_pcm_decode_oracle_against_reference(oracle, reference, tmp_path):
+def test_pcm_decode_oracle_against_reference(oracle, reference, recorded, tmp_path):
     """orc_pcm_to_planar (src/audio/wav.c:458-521) is bit-exact against vv_dsp_wav_read of the same bytes, for every
     sample format the reference reads, mono and interleaved stereo, including the extreme codes."""
-    if not hasattr(reference.lib, "vv_dsp_wav_read"):
-        pytest.skip("oracle/_ref was built without wav.c")
-    rng = np.random.default_rng(3)
-    for fmt in (16, 24, 32, -32):
-        for channels in (1, 2):
-            n = 1001
-            if fmt == -32:
-                raw = rng.uniform(-1, 1, n * channels).astype("<f4").tobytes()
-            elif fmt == 24:
-                v = rng.integers(-2**23, 2**23, n * channels, dtype=np.int64)
-                v[:4] = [-2**23, 2**23 - 1, -1, 0]
-                raw = b"".join(int(q & 0xFFFFFF).to_bytes(3, "little") for q in v)
-            else:
-                lim = 2 ** (fmt - 1)
-                v = rng.integers(-lim, lim, n * channels, dtype=np.int64)
-                v[:4] = [-lim, lim - 1, -1, 0]
-                raw = v.astype("<i2" if fmt == 16 else "<i4").tobytes()
-            path = tmp_path / f"t_{fmt}_{channels}.wav"
-            _write_wav(path, raw, fmt, channels)
-            assert oracle.pcm_to_planar(raw, fmt, channels).tobytes() == reference.wav_read(path).tobytes(), (fmt, channels)
+    check_against_reference(oracle, reference, recorded, pcm_cases(oracle, str(tmp_path)))
