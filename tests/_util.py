@@ -42,9 +42,43 @@ def rel_l2(y, x):
     return float(np.linalg.norm(y - x) / d) if d > 0 else float(np.linalg.norm(y - x))
 
 
-def stft_truth_f64(x, w, nfft, hop, frames):
-    """float64 STFT truth (valid frames) for accuracy-vs-truth reporting."""
+def reflect_index(idx, n):
+    """edge-inclusive reflection of any index into [0, n): ... 1 0 | 0 1 .. n-1 | n-1 n-2 ... (integer arithmetic)"""
+    m = np.mod(idx, 2 * n)
+    return np.where(m < n, m, 2 * n - 1 - m)
+
+
+def stft_truth_f64(x, w, nfft, hop, frames=None, convention="valid"):
+    """float64 STFT truth of x ([..., n]) in any of the four frame conventions: frame f starts at f*hop, or at
+    f*hop - nfft/2 with edge-inclusive reflection for "center"; samples past either end are zero otherwise.
+    frames defaults to the convention's frame count."""
+    from oracle.oracle import num_frames
     x = np.asarray(x, np.float64)
     w = np.asarray(w, np.float64)
+    n = x.shape[-1]
+    if frames is None:
+        frames = num_frames(n, nfft, hop, convention)
+    if n == 0:
+        return np.zeros(x.shape[:-1] + (frames, nfft // 2 + 1), np.complex128)
     idx = np.arange(nfft)[None, :] + hop * np.arange(frames)[:, None]
-    return np.fft.rfft(x[idx] * w[None, :], axis=-1)
+    if convention == "center":
+        fr = x[..., reflect_index(idx - nfft // 2, n)]
+    else:
+        inside = idx < n
+        fr = np.where(inside, x[..., np.where(inside, idx, 0)], 0.0)
+    return np.fft.rfft(fr * w, axis=-1)
+
+
+def istft_truth_f64(spec, w, nfft, hop, n_out):
+    """float64 overlap-add of irfft(spec) * w ([..., frames, bins] -> [..., n_out]) and the float64 window-sum
+    sum_f w(t - f*hop)^2 ([n_out]); frame f starts at sample f*hop, samples past n_out are dropped."""
+    spec = np.asarray(spec)
+    w = np.asarray(w, np.float64)
+    frames = spec.shape[-2]
+    span = max(n_out, (frames - 1) * hop + nfft if frames else 0)
+    acc = np.zeros(spec.shape[:-2] + (span,))
+    wsum = np.zeros(span)
+    for f in range(frames):
+        acc[..., f * hop:f * hop + nfft] += np.fft.irfft(spec[..., f, :].astype(np.complex128), nfft, axis=-1) * w
+        wsum[f * hop:f * hop + nfft] += w * w
+    return acc[..., :n_out], wsum[:n_out]

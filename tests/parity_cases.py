@@ -8,7 +8,7 @@ relative L2 <= 1e-5; frame counts, padding and indexing bit-exact.
 """
 import numpy as np
 
-from _util import ATOL, ROUNDTRIP_REL_L2, RTOL, noise, rel_l2, spectra_close, stft_truth_f64
+from _util import ATOL, ROUNDTRIP_REL_L2, RTOL, istft_truth_f64, noise, rel_l2, spectra_close, stft_truth_f64
 from vv_dsp_b200 import StftStream, FftPlan, Stft
 from vv_dsp_b200.api import VvDspError
 
@@ -105,10 +105,9 @@ def check_inverse_few_frames(lib, oracle, sizes, frame_counts=(1, 2, 3, 4, 5, 9)
                 spec = np.stack([oracle.stft(x[i], nfft, hop) for i in range(3)])
                 assert spec.shape[1] == F
                 for extra in (0, 7, nfft):
-                    nn = np.zeros(n + extra + nfft)
-                    for f in range(F):
-                        nn[f * hop:f * hop + nfft] += w * w
-                    good = np.broadcast_to(nn[:n + extra] > 1e-2, (3, n + extra))
+                    # float64 truth: overlap-add of irfft(spec) * w in double, and the double window-sum
+                    acc, nn = istft_truth_f64(spec, w, nfft, hop, n + extra)
+                    good = np.broadcast_to(nn > 1e-2, (3, n + extra))
                     for norm in (False, True):
                         if norm and 2 * hop > nfft:
                             continue
@@ -126,12 +125,8 @@ def check_inverse_few_frames(lib, oracle, sizes, frame_counts=(1, 2, 3, 4, 5, 9)
                         assert err < tol, (nfft, hop, F, extra, norm, err)
                         # ... so the binding check for this library is float64 truth at the north-star bound:
                         # overlap-add of irfft(spec) * w in double, divided by the double window-sum
-                        acc = np.zeros((3, n + extra + nfft))
-                        for f in range(F):
-                            acc[:, f * hop:f * hop + nfft] += np.fft.irfft(spec[:, f].astype(np.complex128), nfft, axis=-1) * w
-                        acc = acc[:, :n + extra]
                         if norm:
-                            truth = np.where(good, acc / np.where(nn[:n + extra] > 1e-2, nn[:n + extra], 1.0), 0.0)
+                            truth = np.where(good, acc / np.where(nn > 1e-2, nn, 1.0), 0.0)
                             terr = np.abs((y - truth)[good]).max() / max(np.abs(truth[good]).max(), 1e-30)
                             # a sample is divided by a window-sum >= 1e-2, which amplifies the float32 rounding of
                             # the synthesis (~2e-7 of max|x|) by up to 100
@@ -624,6 +619,225 @@ def check_accuracy_vs_truth(lib, oracle, nfft):
     return mine, theirs
 
 
+# Bounds against float64 truth, relative to the per-signal maximum of the truth: about 4 times the worst error of any
+# route (test_gpu_parity.py::test_route_vs_float64_truth lists them per kernel family).  The north-star parity bound
+# (5e-5) would let a wrong twiddle, a dropped halo frame or a small race through.
+TRUTH_COMPLEX = 1e-6          # complex and magnitude spectra
+TRUTH_POWER = 2e-6
+TRUTH_RAW = 1e-6              # overlap-add without normalisation
+TRUTH_NORM = 1e-5             # normalised ISTFT, samples whose window-sum is above 1e-2
+TRUTH_WEIGHTED = 2e-6         # normalised ISTFT, every sample with a window-sum above 1e-10, error times sqrt(window-sum)
+
+# kernel family -> the launcher that VVB_ROUTE_DEBUG names, and fft_size / (the M of its Cfg); None: no Cfg parameter
+ROUTE_LAUNCHERS = {
+    "stft_march_kernel": ("launch_fwd_march_t", 2),
+    "stft_forward_kernel": ("launch_forward_t", 2),
+    "istft_pair_kernel": ("launch_inv_pair_s", 1),
+    "istft_ws_kernel": ("launch_inv_ws_s", None),
+    "istft_march_kernel": ("launch_inv_march_s", 2),
+    "stft_inverse_kernel": ("launch_inverse_t", 2),          # the slot overlap-add (OLA = true) instantiation
+}
+
+
+def routed(capfd, fn):
+    """fn() with VVB_ROUTE_DEBUG=1: (its result, the library's stderr lines)"""
+    import os
+    capfd.readouterr()
+    os.environ["VVB_ROUTE_DEBUG"] = "1"
+    try:
+        r = fn()
+    finally:
+        del os.environ["VVB_ROUTE_DEBUG"]
+    return r, capfd.readouterr().err.splitlines()
+
+
+def launched(lines, family, nfft):
+    """did one of the VVB_ROUTE_DEBUG lines launch `family` in the configuration of this fft_size?"""
+    fn, div = ROUTE_LAUNCHERS[family]
+    for ln in lines:
+        if not ln.startswith("vvb: launch ") or f"vvb::{fn}(" not in ln:
+            continue
+        if div is not None and f"C = Cfg<{nfft // div}," not in ln:
+            continue
+        if family == "stft_inverse_kernel" and "bool OLA = true" not in ln:
+            continue
+        return True
+    return False
+
+
+def ola_chunks(lines):
+    """chunks per signal of the last stft_inverse_kernel overlap-add launch (VVB_ROUTE_DEBUG)"""
+    found = [int(ln.split("chunks_per_signal ")[1].split(",")[0]) for ln in lines if "chunks_per_signal" in ln]
+    assert found, lines
+    return found[-1]
+
+
+def _rel(got, truth, axis):
+    """worst over signals of max|got - truth| / max|truth|, both maxima per signal"""
+    got = np.asarray(got)
+    err = np.abs(got.astype(truth.dtype) - truth).max(axis=axis)
+    return float((err / np.maximum(np.abs(truth).max(axis=axis), 1e-30)).max())
+
+
+def check_route(lib, oracle, nfft, hop, win, n, batch=2, big_batch=64, capfd=None, fwd=None, inv=None, min_chunks=None,
+                device_views=False):
+    """One (fft_size, hop, window) against float64 truth, through whatever kernels the dispatcher picks for it:
+      - forward complex in all four frame conventions, power and magnitude of valid frames (stft_truth_f64);
+      - inverse raw and normalised (istft_truth_f64), fed with the library's own spectra and with the oracle's;
+        normalised samples are compared where the window-sum is above 1e-2, and wherever the library divides with the
+        error weighted by sqrt(window-sum); uncovered samples must be exactly zero;
+      - the interior round trip at ROUNDTRIP_REL_L2 where the window-sum has no near-zeros;
+      - batch invariance: signal 0 alone == signal 0 in a batch of big_batch, forward and inverse, bit for bit (the two
+        calls split the signal into different work ranges / overlap-add chunks);
+      - with device_views (GPU): input, spectra and output as torch views with odd row pitches (unaligned rows: the
+        scalar overlap-add combine and the 32-bit stores of the marching kernels) == the host-buffer results, bit for bit.
+    With capfd, the VVB_ROUTE_DEBUG lines of the single-signal calls must name the kernel families fwd / inv, and an
+    inverse through stft_inverse_kernel must cut the signal into at least min_chunks chunks.
+    Returns the worst error per check relative to the per-signal maximum of the truth."""
+    bins = nfft // 2 + 1
+    x = np.stack([noise(7000 + nfft + hop + i, n) for i in range(batch)])
+    w = oracle.window(win, nfft)[1]
+    worst = dict.fromkeys(("complex", "power", "magnitude", "raw", "norm", "weighted"), 0.0)
+
+    def bound(what, e, lim, *ctx):
+        worst[what] = max(worst[what], e)
+        assert e <= lim, (what, nfft, hop, win, *ctx, e)
+
+    with Stft(nfft, hop, win, lib=lib) as h:
+        for conv in ("valid", "spectrogram", "padded_tail", "center"):
+            s = h.batch_forward(x, "complex", conv)
+            truth = stft_truth_f64(x, w, nfft, hop, convention=conv)
+            assert s.shape == truth.shape == (batch, oracle.num_frames(n, nfft, hop, conv), bins), conv
+            bound("complex", _rel(s, truth, (1, 2)), TRUTH_COMPLEX, conv)
+            if conv == "valid":
+                spec, tv = s, truth
+        F = spec.shape[1]
+        bound("power", _rel(h.batch_forward(x, "power", "valid"), np.abs(tv) ** 2, (1, 2)), TRUTH_POWER)
+        bound("magnitude", _rel(h.batch_forward(x, "magnitude", "valid"), np.abs(tv), (1, 2)), TRUTH_COMPLEX)
+
+        cov = (F - 1) * hop + nfft
+        ospec = np.stack([oracle.stft(x[i], nfft, hop, win) for i in range(batch)])
+        for which, sp in (("own", spec), ("oracle", ospec)):
+            acc, wsum = istft_truth_f64(sp, w, nfft, hop, n)
+            raw = h.batch_inverse(sp, n, False)
+            y = h.batch_inverse(sp, n, True)
+            bound("raw", _rel(raw, acc, 1), TRUTH_RAW, which)
+            good = wsum > 1e-2
+            if good.any():
+                bound("norm", _rel(y[:, good], acc[:, good] / wsum[good], 1), TRUTH_NORM, which)
+            # every sample the library divides, the error weighted by sqrt(window-sum): the synthesis error at a sample
+            # scales with the windows that cover it, so this stays at the raw-sum level even where the divide
+            # amplifies it (the window tails at both ends of the signal)
+            div = wsum > 1e-10
+            sc = np.sqrt(wsum[div])
+            bound("weighted", _rel(y[:, div] * sc, acc[:, div] / sc, 1), TRUTH_WEIGHTED, which)
+            assert np.all(y[:, cov:] == 0) and np.all(raw[:, cov:] == 0), which
+            if which == "own":
+                own_y, own_raw = y, raw
+        lo, hi = nfft, n - nfft
+        if hi > lo and (2 * hop <= nfft or win == "boxcar"):
+            err = rel_l2(own_y[:, lo:hi], x[:, lo:hi])
+            assert err <= ROUNDTRIP_REL_L2, (nfft, hop, win, err)
+
+        # batch invariance (and, with capfd, the route of the single-signal calls)
+        call = (lambda f: routed(capfd, f)) if capfd is not None else (lambda f: (f(), []))
+        s1, lines_f = call(lambda: h.batch_forward(x[:1], "complex", "valid"))
+        y1, lines_i = call(lambda: h.batch_inverse(s1, n, True))
+        r1 = h.batch_inverse(s1, n, False)
+        assert np.array_equal(s1[0], spec[0]) and np.array_equal(y1[0], own_y[0]) and np.array_equal(r1[0], own_raw[0])
+        if big_batch:
+            xb = np.concatenate([x[:1], np.stack([noise(9000 + i, n) for i in range(big_batch - 1)])])
+            sb = h.batch_forward(xb, "complex", "valid")
+            assert np.array_equal(sb[0], s1[0]), (nfft, hop, win, "forward: alone != in a batch")
+            assert np.array_equal(h.batch_inverse(sb, n, True)[0], y1[0]), (nfft, hop, win, "inverse: alone != in a batch")
+            assert np.array_equal(h.batch_inverse(sb, n, False)[0], r1[0]), (nfft, hop, win, "raw: alone != in a batch")
+            del xb, sb
+        if capfd is not None:
+            assert fwd is None or launched(lines_f, fwd, nfft), (nfft, hop, fwd, lines_f)
+            assert inv is None or launched(lines_i, inv, nfft), (nfft, hop, inv, lines_i)
+            if min_chunks is not None:
+                assert ola_chunks(lines_i) >= min_chunks, (nfft, hop, lines_i)
+
+        if device_views:
+            import torch
+            assert batch > 1                                       # (a single row has no pitch)
+            px = n + (1 if n % 2 == 0 else 2)                      # odd row pitches: rows start at every alignment
+            xd = torch.zeros((batch, px), device="cuda")
+            xd[:, :n] = torch.from_numpy(x)
+            sd = torch.zeros((batch, F, bins + 2), dtype=torch.complex64, device="cuda")
+            yd = torch.zeros((batch, px), device="cuda")
+            rd = torch.zeros((batch, px), device="cuda")
+            h.batch_forward(xd[:, :n], "complex", "valid", out=sd[:, :, :bins])
+            h.batch_inverse(sd[:, :, :bins], n, True, out=yd[:, :n])
+            h.batch_inverse(sd[:, :, :bins], n, False, out=rd[:, :n])
+            torch.cuda.synchronize()
+            assert np.array_equal(sd[:, :, :bins].cpu().numpy(), spec) and float(sd[:, :, bins:].abs().max()) == 0.0
+            assert np.array_equal(yd[:, :n].cpu().numpy(), own_y) and float(yd[:, n:].abs().max()) == 0.0
+            assert np.array_equal(rd[:, :n].cpu().numpy(), own_raw) and float(rd[:, n:].abs().max()) == 0.0
+    return worst
+
+
+# Every STFT / ISTFT kernel family with the (fft_size, hop) rows that reach it: (fft_size, hop, forward family, inverse family).
+# Hops 441 and 75 are no multiple of 4 (scalar overlap-add combine); 441 is 10 ms at 44.1 kHz.
+ROUTES = ([(2048, h, "stft_march_kernel", "istft_ws_kernel") for h in (256, 512, 1024)]
+          + [(N, N // d, "stft_march_kernel", "istft_march_kernel") for N in (4096, 8192) for d in (8, 4, 2)]
+          + [(N, N // d, "stft_forward_kernel", "istft_pair_kernel") for N in (256, 512, 1024) for d in (8, 4, 2)]
+          + [(N, h, "stft_forward_kernel", "stft_inverse_kernel") for N, h in
+             ((256, 100), (512, 75), (1024, 100), (2048, 480), (2048, 441), (4096, 1000), (4096, 441), (4096, 4096),
+              (8192, 441), (8192, 3000), (400, 160), (640, 160))])
+
+# frames per round (teams G per CTA) of stft_inverse_kernel at each fft_size: 256 threads / (fft_size/2 / points per thread)
+OLA_TEAMS = {256: 32, 512: 16, 1024: 16, 2048: 8, 4096: 4, 8192: 2, 400: 64, 640: 16}
+
+
+def route_length(nfft, hop, inv, chunks=4):
+    """Signal length for a route row.  Where the inverse is stft_inverse_kernel: enough frames for the slot overlap-add
+    to cut ONE signal into `chunks` chunks (it keeps >= 16 rounds of G frames per chunk), with a ragged last chunk;
+    elsewhere 41 frames.  A ragged tail after the last frame either way."""
+    frames = 16 * OLA_TEAMS[nfft] * chunks + OLA_TEAMS[nfft] // 2 + 3 if inv == "stft_inverse_kernel" else 41
+    return (frames - 1) * hop + nfft + hop // 3
+
+
+MEL_SWITCHES = ("VVB_MEL_NO_TMA", "VVB_MEL_UNIT4", "VVB_MEL_NO_GENERIC", "VVB_MEL_ROW_SPREAD_OFF")
+
+
+def check_mel_switches(lib, cases=((2048, 512, 80, 48000.0), (2048, 256, 40, 16000.0), (512, 128, 40, 16000.0), (400, 160, 80, 16000.0),
+                                   (1024, 256, 64, 44100.0)), n=20000, batch=3):
+    """The log-mel diagnostic switches are documented as bit-identical to the default path: log-mel and MFCC rows of the
+    batched chain (each switch alone and on top of VVB_MEL_UNFUSED, where the log-mel kernel of the chain runs), and
+    log_mel_spectrogram on a dense power matrix (logmel_tma_kernel against the register-transposing kernel)."""
+    import os
+    from vv_dsp_b200 import log_mel_spectrogram, mel_filterbank
+    for nfft, hop, n_mels, sr in cases:
+        st, w = mel_filterbank(nfft, n_mels, sr, 0.0, sr / 2, lib=lib)
+        assert st == 0
+        x = np.stack([noise(4000 + nfft + i, n) for i in range(batch)])
+
+        def rows(*envs):
+            for e in envs:
+                os.environ[e] = "1"
+            try:
+                with Stft(nfft, hop, "hann", lib=lib) as h:       # (VVB_MEL_UNIT4 is read when a handle builds its schedules)
+                    return (h.batch_logmel(x, w, 1e-6, "center"), h.batch_logmel(x, w, 1e-6, "valid"),
+                            h.batch_mfcc(x, w, 13, lifter=22.0, log_epsilon=1e-6, convention="center"))
+            finally:
+                for e in envs:
+                    del os.environ[e]
+        fused, chained = rows(), rows("VVB_MEL_UNFUSED")
+        for env in MEL_SWITCHES:
+            for base, got in ((fused, rows(env)), (chained, rows("VVB_MEL_UNFUSED", env))):
+                for a, b in zip(base, got):
+                    assert a.shape == b.shape and np.array_equal(a, b, equal_nan=True), (nfft, hop, env)
+        p = np.random.default_rng(nfft).uniform(0, 3, (77, nfft // 2 + 1)).astype(np.float32)
+        a = log_mel_spectrogram(p, w, 1e-10, lib=lib)
+        os.environ["VVB_MEL_NO_TMA"] = "1"
+        try:
+            b = log_mel_spectrogram(p, w, 1e-10, lib=lib)
+        finally:
+            del os.environ["VVB_MEL_NO_TMA"]
+        assert np.array_equal(a, b), (nfft, "log_mel_spectrogram")
+
+
 def check_bluestein(lib, oracle, sizes):
     """Sizes served by the chirp-z path (no Stockham kernel, 32 <= n <= 4096).  The reference serves them with an O(n^2)
     float32 DFT whose own error grows with n (measured here: 2.5e-5 at n=400, 6e-5 at 1000, 1.5e-4 at 2000 of max|X|),
@@ -653,12 +867,7 @@ def check_bluestein(lib, oracle, sizes):
                 # synthesis: float64 overlap-add of irfft(spec) * w, divided by sum(w^2) where > 1e-12
                 y = h.batch_inverse(ref, n, True)
                 raw = h.batch_inverse(ref, n, False)
-                acc = np.zeros((2, n + nfft)); norm = np.zeros(n + nfft)
-                for f in range(F):
-                    fr = np.fft.irfft(ref[:, f].astype(np.complex128), nfft, axis=-1) * w.astype(np.float64)
-                    acc[:, f * hop:f * hop + nfft] += fr
-                    norm[f * hop:f * hop + nfft] += w.astype(np.float64) ** 2
-                acc, norm = acc[:, :n], norm[:n]
+                acc, norm = istft_truth_f64(ref, w, nfft, hop, n)
                 assert np.abs(raw - acc).max() <= 3e-6 * np.abs(acc).max()
                 cov = (F - 1) * hop + nfft
                 assert np.all(y[:, cov:] == 0) and np.all(raw[:, cov:] == 0)

@@ -174,3 +174,39 @@ def test_staged_chunks_do_not_overlap(emu, monkeypatch):
 @pytest.mark.parametrize("nfft,hop", [(2048, 512), (4096, 1024), (512, 256), (1024, 128)])
 def test_stream_sharding_bit_identical(emu, nfft, hop):
     pc.check_stream_sharding(emu, nfft, hop, nfft + hop * 45 + 17, shard_counts=(1, 2, 3))
+
+
+# reduced route matrix: every kernel family, Hann plus one other window (the full matrix runs in test_gpu_parity.py)
+EMU_ROUTES = [(2048, 512, "hamming"), (4096, 1024, "boxcar"), (8192, 2048, "hann"), (1024, 512, "hann"), (256, 32, "hamming"),
+              (2048, 441, "hamming"), (512, 75, "boxcar"), (4096, 1000, "hann"), (8192, 441, "hann"), (1024, 100, "hamming")]
+
+
+@pytest.mark.parametrize("nfft,hop,win", EMU_ROUTES)
+def test_route_vs_float64_truth(emu, oracle, capfd, nfft, hop, win):
+    """one (fft_size, hop) per kernel family against float64 truth (parity_cases.check_route); the route is asserted from
+    the library's VVB_ROUTE_DEBUG lines, and the slot overlap-add cuts one signal into at least 4 chunks"""
+    fwd, inv = next((r[2], r[3]) for r in pc.ROUTES if r[:2] == (nfft, hop))
+    n = pc.route_length(nfft, hop, inv)
+    worst = pc.check_route(emu, oracle, nfft, hop, win, n, batch=2, big_batch=5, capfd=capfd, fwd=fwd, inv=inv,
+                           min_chunks=4 if inv == "stft_inverse_kernel" else None)
+    print("route", nfft, hop, win, fwd, inv, worst)
+
+
+@pytest.mark.parametrize("env,nfft,hop,inv", [("VVB_NO_WS", 2048, 256, "istft_march_kernel"),
+                                              ("VVB_NO_PAIR", 512, 64, "istft_march_kernel"), ("VVB_NO_PAIR", 1024, 512, "istft_march_kernel"),
+                                              ("VVB_NO_PAIR", 256, 128, "stft_inverse_kernel"),
+                                              ("VVB_NO_MARCH", 8192, 1024, "stft_inverse_kernel"), ("VVB_NO_MARCH", 1024, 256, "stft_inverse_kernel")])
+def test_cross_check_switch_routes(emu, oracle, capfd, monkeypatch, env, nfft, hop, inv):
+    """the cross-check kernels behind VVB_NO_WS / VVB_NO_PAIR / VVB_NO_MARCH against float64 truth"""
+    monkeypatch.setenv(env, "1")
+    fwd = "stft_forward_kernel" if env == "VVB_NO_MARCH" or nfft <= 1024 else "stft_march_kernel"
+    pc.check_route(emu, oracle, nfft, hop, "hann", pc.route_length(nfft, hop, None), big_batch=3, capfd=capfd, fwd=fwd, inv=inv)
+
+
+def test_mel_switches_bit_identical(emu):
+    pc.check_mel_switches(emu, cases=((2048, 512, 80, 48000.0), (512, 128, 40, 16000.0), (400, 160, 80, 16000.0)), n=9000)
+
+
+def test_stream_sharding_without_graphs(emu, monkeypatch):
+    monkeypatch.setenv("VVB_STREAM_NO_GRAPH", "1")
+    pc.check_stream_sharding(emu, 2048, 512, 2048 + 512 * 45 + 17, shard_counts=(1, 3))

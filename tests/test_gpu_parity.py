@@ -78,9 +78,10 @@ def test_marching_istft_partitions(lib, oracle):
     pc.check_batch_inverse(lib, oracle, 2048, 512, "hann", 2048 + 511, batch=1)
 
 
-def test_many_signals_chunking(lib, oracle):
-    """more work items than resident CTAs, several chunks per signal in the ISTFT"""
-    nfft, hop, n, B = 1024, 256, 200000, 7
+def test_many_signals_chunking(lib, oracle, capfd):
+    """more work items than resident CTAs, several chunks per signal in the ISTFT (hop 100: the slot overlap-add of
+    stft_inverse_kernel, which cuts every signal into chunks that re-synthesise their halo frames)"""
+    nfft, hop, n, B = 1024, 100, 200000, 7
     x = np.stack([noise(300 + i, n) for i in range(B)])
     from vv_dsp_b200 import Stft
     with Stft(nfft, hop, "hann", lib=lib) as h:
@@ -88,7 +89,8 @@ def test_many_signals_chunking(lib, oracle):
         ref = oracle.batch_forward(x, nfft, hop, threads=4)
         ok, frac = spectra_close(s, ref)
         assert ok, frac
-        y = h.batch_inverse(ref, n, True)
+        y, lines = pc.routed(capfd, lambda: h.batch_inverse(ref, n, True))
+        assert pc.launched(lines, "stft_inverse_kernel", nfft) and pc.ola_chunks(lines) >= 2, lines
         refy = np.stack([oracle.istft(ref[i], nfft, hop, n) for i in range(B)])
         assert rel_l2(y[:, nfft:-nfft], refy[:, nfft:-nfft]) < 5e-5
         assert rel_l2(h.batch_inverse(s, n, True)[:, nfft:-nfft], x[:, nfft:-nfft]) < ROUNDTRIP_REL_L2
@@ -562,3 +564,68 @@ def test_stream_sharding_over_all_visible_gpus(lib):
         assert np.array_equal(s.download_spectra(), spec)
         assert np.array_equal(s.download(), y)
         assert {s.shard(d).device for d in range(g)} == set(range(g))
+
+
+@pytest.mark.parametrize("win", ["hann", "hamming", "boxcar"])
+@pytest.mark.parametrize("nfft,hop,fwd,inv", pc.ROUTES)
+def test_route_vs_float64_truth(lib, oracle, capfd, nfft, hop, fwd, inv, win):
+    """Every kernel family at the (fft_size, hop) rows that reach it (parity_cases.ROUTES) against float64 truth, with
+    the route read from VVB_ROUTE_DEBUG; stft_inverse_kernel rows cut one signal into >= 4 overlap-add chunks.
+    Worst error against truth over the three windows, relative to the per-signal maximum, measured on one NVIDIA B200
+    (power limit 1000 W); bounds in parity_cases.TRUTH_*:
+      stft_march_kernel    complex 2.3e-7, magnitude 2.4e-7, power 4.3e-7
+      stft_forward_kernel  complex 2.4e-7, magnitude 2.9e-7, power 4.9e-7
+      istft_ws_kernel      raw 3.4e-7, normalised 1.4e-6, weighted 4.0e-7
+      istft_march_kernel   raw 3.9e-7, normalised 1.7e-6, weighted 4.4e-7
+      istft_pair_kernel    raw 3.4e-7, normalised 1.2e-6, weighted 3.7e-7
+      stft_inverse_kernel  raw 4.1e-7, normalised 1.9e-6, weighted 4.3e-7
+    (istft_pair_kernel was at 6.5e-6 normalised and up to 5e-4 weighted before its unpaired last frame stopped adding
+    the transform's rounding noise to the tail samples.)"""
+    worst = pc.check_route(lib, oracle, nfft, hop, win, pc.route_length(nfft, hop, inv), batch=2, big_batch=64, capfd=capfd,
+                           fwd=fwd, inv=inv, min_chunks=4 if inv == "stft_inverse_kernel" else None, device_views=True)
+    with capfd.disabled():
+        print("route", nfft, hop, win, fwd, inv, " ".join(f"{k} {v:.2e}" for k, v in worst.items()))
+
+
+@pytest.mark.parametrize("hop", [256, 512, 1024])
+def test_no_ws_switch(lib, oracle, capfd, monkeypatch, hop):
+    """VVB_NO_WS: the ISTFT of fft_size 2048 through istft_march_kernel<Cfg1024> instead of istft_ws_kernel, within the
+    truth bounds.  Not bit-identical to the default path: measured on a B200, the raw overlap-add differs in the last bits
+    (up to 2.4e-7 of max|y|) and the normalised output by up to 1.3e-6 where the window-sum is above 1e-2."""
+    monkeypatch.setenv("VVB_NO_WS", "1")
+    for win in ("hann", "hamming", "boxcar"):
+        pc.check_route(lib, oracle, 2048, hop, win, pc.route_length(2048, hop, None), capfd=capfd,
+                       fwd="stft_march_kernel", inv="istft_march_kernel", device_views=True)
+
+
+@pytest.mark.parametrize("nfft,hop", [(N, N // d) for N in (256, 512, 1024) for d in (8, 4, 2)])
+def test_no_pair_switch(lib, oracle, capfd, monkeypatch, nfft, hop):
+    """VVB_NO_PAIR: unsharded ISTFT of fft_size 512 / 1024 through the whole-warp marching kernel, of 256 through the slot
+    overlap-add -- within the truth bounds (not claimed bit-identical to istft_pair_kernel)"""
+    monkeypatch.setenv("VVB_NO_PAIR", "1")
+    inv = "stft_inverse_kernel" if nfft == 256 else "istft_march_kernel"
+    for win in ("hann", "hamming", "boxcar"):
+        pc.check_route(lib, oracle, nfft, hop, win, pc.route_length(nfft, hop, None), capfd=capfd,
+                       fwd="stft_forward_kernel", inv=inv, device_views=True)
+
+
+@pytest.mark.parametrize("nfft,hop", [(r[0], r[1]) for r in pc.ROUTES if r[3] != "stft_inverse_kernel"])
+def test_no_march_switch(lib, oracle, capfd, monkeypatch, nfft, hop):
+    """VVB_NO_MARCH: the generic forward kernel and the slot overlap-add for every (fft_size, hop) that normally takes a
+    marching, warp-specialised or pair kernel -- within the truth bounds"""
+    monkeypatch.setenv("VVB_NO_MARCH", "1")
+    for win in ("hann", "hamming", "boxcar"):
+        pc.check_route(lib, oracle, nfft, hop, win, pc.route_length(nfft, hop, None), capfd=capfd,
+                       fwd="stft_forward_kernel", inv="stft_inverse_kernel", device_views=True)
+
+
+def test_mel_switches_bit_identical(lib):
+    pc.check_mel_switches(lib)
+
+
+@pytest.mark.parametrize("nfft,hop", [(2048, 512), (4096, 1024), (1024, 256)])
+def test_stream_sharding_without_graphs(lib, monkeypatch, nfft, hop):
+    """VVB_STREAM_NO_GRAPH: the stream handle's launches enqueued one by one instead of replaying a CUDA graph -- still
+    bit-identical to the unsharded calls"""
+    monkeypatch.setenv("VVB_STREAM_NO_GRAPH", "1")
+    pc.check_stream_sharding(lib, nfft, hop, nfft + hop * 997 + 123, shard_counts=(1, 2, 5))

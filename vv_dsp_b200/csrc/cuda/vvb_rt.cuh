@@ -24,16 +24,26 @@ int rt_num_sms();                                                 /* SMs of the 
 
 enum { VVB_MAX_DEVICES = 32 };
 
+/* VVB_ROUTE_DEBUG=1: one stderr line per launch naming the kernel and the function that launches it.  Inside the
+ * per-family launchers (vvb_tu_*.cu, vvb_launch_march.cuh) the function's signature carries the kernel family and its
+ * compile-time configuration, so a test can tell which kernel a (fft_size, hop) reached. */
+inline void rt_route_debug(const char* kern, const char* where)
+{
+    if (getenv("VVB_ROUTE_DEBUG")) fprintf(stderr, "vvb: launch %s in %s\n", kern, where);
+}
+
 #ifdef VVB_EMU
 #define CK(expr) do { if ((expr) != 0) return ::vvb::rt_fail(4, #expr, "emu"); } while (0)
 #define VVB_LAUNCH(kern, grid, block, smem, stream, ...) \
-    do { ::vvb::g_launches++; vvb_emu::launch(dim3(grid), dim3(block), smem, [&] { kern(__VA_ARGS__); }); } while (0)
+    do { ::vvb::g_launches++; ::vvb::rt_route_debug(#kern, __PRETTY_FUNCTION__); \
+         vvb_emu::launch(dim3(grid), dim3(block), smem, [&] { kern(__VA_ARGS__); }); } while (0)
 inline int rt_device() { return 0; }
 template <class K> static int rt_blocks_per_sm(K, int, size_t) { return 1; }
 #else
 #define CK(expr) do { cudaError_t e_ = (expr); if (e_ != cudaSuccess) return ::vvb::rt_fail(4, #expr, cudaGetErrorString(e_)); } while (0)
 #define VVB_LAUNCH(kern, grid, block, smem, stream, ...) \
-    do { ::vvb::g_launches++; kern<<<(grid), (block), (smem), (cudaStream_t)(stream)>>>(__VA_ARGS__); CK(cudaGetLastError()); } while (0)
+    do { ::vvb::g_launches++; ::vvb::rt_route_debug(#kern, __PRETTY_FUNCTION__); \
+         kern<<<(grid), (block), (smem), (cudaStream_t)(stream)>>>(__VA_ARGS__); CK(cudaGetLastError()); } while (0)
 inline int rt_device() { int d = 0; return cudaGetDevice(&d) == cudaSuccess ? d : 0; }
 /* opt in to the dynamic shared memory the kernel needs (a per-device attribute) and ask how many CTAs fit per SM */
 template <class K> static int rt_blocks_per_sm(K kern, int threads, size_t smem)

@@ -1453,14 +1453,19 @@ __global__ void __launch_bounds__(32 * G, MINB) istft_pair_kernel(const PairArgs
                         const float2 z = v[q * L::R + ct_bitrev(r, L::R)];
                         acc[sl] = fmaf(z.y, w[sl], acc[sl]);
                     }
+                /* an odd frame count leaves the last pair without its second frame: the imaginary part is then only the
+                 * transform's rounding noise, which must not reach the tail samples (after the divide by a window-sum
+                 * that falls towards 0 there it would be amplified without bound) */
+                if (have1) {
 #pragma unroll
-                for (int q = 0; q < L::NQ; ++q)
+                    for (int q = 0; q < L::NQ; ++q)
 #pragma unroll
-                    for (int r = 0; r < L::R; ++r) {
-                        const int sl = q + r * (L::NS / 32);
-                        const float2 z = v[q * L::R + ct_bitrev(r, L::R)];
-                        acc[sl + HS] = fmaf(z.x, w[sl], acc[sl + HS]);
-                    }
+                        for (int r = 0; r < L::R; ++r) {
+                            const int sl = q + r * (L::NS / 32);
+                            const float2 z = v[q * L::R + ct_bitrev(r, L::R)];
+                            acc[sl + HS] = fmaf(z.x, w[sl], acc[sl + HS]);
+                        }
+                }
             }
             /* the two oldest hop-blocks are complete: blocks f0 (slots 0..HS-1) and f0+1 (slots HS..2HS-1) */
 #pragma unroll

@@ -27,6 +27,8 @@ template <class C, bool OLA> static int launch_inverse_t(InvArgs a, long long ba
         a.chunk_frames = (int)cf;
         a.chunks_per_signal = (int)((a.frames + cf - 1) / cf);
         items = batch * a.chunks_per_signal;
+        if (getenv("VVB_ROUTE_DEBUG"))
+            fprintf(stderr, "vvb: stft_inverse_kernel overlap-add: chunks_per_signal %d, chunk_frames %d\n", a.chunks_per_signal, a.chunk_frames);
     } else {
         items = (a.frames + G - 1) / G;
     }
