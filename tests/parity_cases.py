@@ -640,29 +640,67 @@ ROUTE_LAUNCHERS = {
 
 
 def routed(capfd, fn):
-    """fn() with VVB_ROUTE_DEBUG=1: (its result, the library's stderr lines)"""
+    """fn() with VVB_ROUTE_DEBUG=1 and VVB_MEL_DEBUG=1: (its result, the library's stderr lines)"""
     import os
     capfd.readouterr()
     os.environ["VVB_ROUTE_DEBUG"] = "1"
+    os.environ["VVB_MEL_DEBUG"] = "1"
     try:
         r = fn()
     finally:
-        del os.environ["VVB_ROUTE_DEBUG"]
+        del os.environ["VVB_ROUTE_DEBUG"], os.environ["VVB_MEL_DEBUG"]
     return r, capfd.readouterr().err.splitlines()
 
 
-def launched(lines, family, nfft):
-    """did one of the VVB_ROUTE_DEBUG lines launch `family` in the configuration of this fft_size?"""
-    fn, div = ROUTE_LAUNCHERS[family]
-    for ln in lines:
-        if not ln.startswith("vvb: launch ") or f"vvb::{fn}(" not in ln:
-            continue
-        if div is not None and f"C = Cfg<{nfft // div}," not in ln:
-            continue
-        if family == "stft_inverse_kernel" and "bool OLA = true" not in ln:
-            continue
-        return True
-    return False
+def chirp_m(nfft):
+    """length of the chirp-z convolution of a size without a Stockham kernel: the power of two >= 2 fft_size - 1, at least 128"""
+    m = 128
+    while m < 2 * nfft - 1:
+        m *= 2
+    return m
+
+
+def route_needles(family, nfft, frames=False):
+    """What VVB_ROUTE_DEBUG prints when `family` runs at this fft_size: a list of groups of substrings, every group on one
+    line.  Besides the Stockham families of ROUTE_LAUNCHERS:
+      chirp_fused_fwd / chirp_fused_inv: chirp_fused_kernel on the M-point plan (M = chirp_m), MODE 0 analysis / MODE 1
+        synthesis;
+      chirp_staged_fwd / chirp_staged_inv: the multi-kernel chirp-z pipeline (pre-multiply, M-point transforms, chirp_mul,
+        post-multiply) with a four-step plan underneath when M > 8192;
+      stft_forward_direct_kernel / stft_inverse_direct_kernel: the O(n^2) kernels;
+      logmel_march / logmel_generic: the fused STFT -> log-mel instantiations of stft_march_kernel (fft_size 2048) and of
+        the generic forward kernel; logmel_tma_kernel / logmel_kernel: the log-mel kernel of the chained path.
+    Inverses of the non-Stockham families end in overlap_add_kernel.  frames: the per-frame synthesis
+    (vvb_stft_inverse_frames), which has no overlap-add."""
+    if family in ROUTE_LAUNCHERS:
+        fn, div = ROUTE_LAUNCHERS[family]
+        group = ["vvb: launch ", f"vvb::{fn}("] + ([f"C = Cfg<{nfft // div},"] if div is not None else [])
+        if family == "stft_inverse_kernel":
+            group.append("bool OLA = false" if frames else "bool OLA = true")
+        return [group]
+    M = chirp_m(nfft)
+    ola = [] if frames else [["vvb: launch overlap_add_kernel in", "vvb_stft_inverse("]]
+    fused = lambda mode: [["vvb: launch kern in", "vvb::launch_chirp_fused_m(", f"C = Cfg<{M},", f"int MODE = {mode}]"]]  # noqa: E731
+    m_point = [["vvb: launch fourstep_transpose_kernel in"]] if M > 8192 else [["vvb::launch_c2c(", f"C = Cfg<{M},"]]
+    staged = lambda pre, post: [[f"vvb: launch {pre} in"], ["vvb: launch chirp_mul_kernel in"], [f"vvb: launch {post} in"]] + m_point  # noqa: E731
+    return {
+        "chirp_fused_fwd": fused(0),
+        "chirp_fused_inv": fused(1) + ola,
+        "chirp_staged_fwd": staged("chirp_pre_stft_kernel", "chirp_post_stft_kernel"),
+        "chirp_staged_inv": staged("chirp_pre_spec_kernel", "chirp_post_frames_kernel") + ola,
+        "stft_forward_direct_kernel": [["vvb: launch stft_forward_direct_kernel in", "vvb_stft_forward("]],
+        "stft_inverse_direct_kernel": [["vvb: launch stft_inverse_direct_kernel in",
+                                        "vvb_stft_inverse_frames(" if frames else "vvb_stft_inverse("]] + ola,
+        "logmel_march": [["vvb: launch kern in", "vvb::launch_fwd_march_t(", "C = Cfg<1024,", "int OUT = 3]"]],
+        "logmel_generic": [["vvb: launch kern in", "vvb::launch_forward_logmel(", f"C = Cfg<{nfft // 2},"]],
+        "logmel_tma_kernel": [["vvb: launch (logmel_tma_kernel<"]],
+        "logmel_kernel": [["vvb: launch logmel_kernel in"]],
+    }[family]
+
+
+def launched(lines, family, nfft, frames=False):
+    """did the VVB_ROUTE_DEBUG lines launch `family` in the configuration of this fft_size?  (route_needles)"""
+    return all(any(all(s in ln for s in group) for ln in lines) for group in route_needles(family, nfft, frames))
 
 
 def ola_chunks(lines):
@@ -709,6 +747,8 @@ def check_route(lib, oracle, nfft, hop, win, n, batch=2, big_batch=64, capfd=Non
             truth = stft_truth_f64(x, w, nfft, hop, convention=conv)
             assert s.shape == truth.shape == (batch, oracle.num_frames(n, nfft, hop, conv), bins), conv
             bound("complex", _rel(s, truth, (1, 2)), TRUTH_COMPLEX, conv)
+            # the spectrum of a real frame is real at DC and, for an even fft_size, at Nyquist: exactly, not to rounding
+            assert np.all(s[..., 0].imag == 0) and (nfft % 2 == 1 or np.all(s[..., -1].imag == 0)), (nfft, hop, win, conv)
             if conv == "valid":
                 spec, tv = s, truth
         F = spec.shape[1]
@@ -784,10 +824,23 @@ ROUTES = ([(2048, h, "stft_march_kernel", "istft_ws_kernel") for h in (256, 512,
           + [(N, N // d, "stft_forward_kernel", "istft_pair_kernel") for N in (256, 512, 1024) for d in (8, 4, 2)]
           + [(N, h, "stft_forward_kernel", "stft_inverse_kernel") for N, h in
              ((256, 100), (512, 75), (1024, 100), (2048, 480), (2048, 441), (4096, 1000), (4096, 441), (4096, 4096),
-              (8192, 441), (8192, 3000), (400, 160), (640, 160))])
+              (8192, 441), (8192, 3000), (400, 160), (640, 160))]
+          # mixed radix (3- and 5-point leaves): 320 and 480 besides 400 / 640 above; hop = fft_size leaves window-sum zeros
+          + [(N, h, "stft_forward_kernel", "stft_inverse_kernel") for N, h in ((320, 80), (320, 160), (480, 120), (480, 160), (400, 400))]
+          # chirp-z in one kernel per transform (M <= 8192), the powers of two below 256 included
+          + [(N, h, "chirp_fused_fwd", "chirp_fused_inv") for N, h in
+             ((64, 16), (128, 32), (100, 25), (440, 110), (1000, 250), (2047, 512), (4095, 1365), (1000, 1000))]
+          # chirp-z through the multi-kernel pipeline on four-step plans (M = 16384, 32768)
+          + [(N, h, "chirp_staged_fwd", "chirp_staged_inv") for N, h in ((5000, 1250), (16384, 4096))]
+          # O(n^2) kernels (n < 32)
+          + [(N, h, "stft_forward_direct_kernel", "stft_inverse_direct_kernel") for N, h in ((12, 5), (24, 6), (31, 9), (30, 30))])
+
+# rows that reach a family only under a selection switch (read when a handle is created): (switch, fft_size, hop, fwd, inv)
+SWITCH_ROUTES = [("VVB_BLUESTEIN_UNFUSED", 440, 110, "chirp_staged_fwd", "chirp_staged_inv"),
+                 ("VVB_NO_BLUESTEIN", 100, 25, "stft_forward_direct_kernel", "stft_inverse_direct_kernel")]
 
 # frames per round (teams G per CTA) of stft_inverse_kernel at each fft_size: 256 threads / (fft_size/2 / points per thread)
-OLA_TEAMS = {256: 32, 512: 16, 1024: 16, 2048: 8, 4096: 4, 8192: 2, 400: 64, 640: 16}
+OLA_TEAMS = {256: 32, 512: 16, 1024: 16, 2048: 8, 4096: 4, 8192: 2, 320: 32, 400: 64, 480: 64, 640: 16}
 
 
 def route_length(nfft, hop, inv, chunks=4):
@@ -796,6 +849,199 @@ def route_length(nfft, hop, inv, chunks=4):
     elsewhere 41 frames.  A ragged tail after the last frame either way."""
     frames = 16 * OLA_TEAMS[nfft] * chunks + OLA_TEAMS[nfft] // 2 + 3 if inv == "stft_inverse_kernel" else 41
     return (frames - 1) * hop + nfft + hop // 3
+
+
+def check_per_frame_route(lib, oracle, nfft, hop, win, frames=5, capfd=None, fwd=None, inv=None):
+    """vv_dsp_stft_process / reconstruct against float64 truth at the TRUTH_* bounds: the spectrum of each frame (all fft_size
+    bins) against the float64 DFT of the windowed frame, and the frame that reconstruct adds (vvb_stft_inverse_frames: the
+    synthesis without overlap-add) against the float64 inverse DFT of the same spectrum times the window; the window-sum it
+    adds is the float32 w*w.  With capfd the VVB_ROUTE_DEBUG lines must name fwd and inv (its per-frame flavour)."""
+    w = oracle.window(win, nfft)[1]
+    x = noise(1300 + nfft + hop, (frames - 1) * hop + nfft)
+    worst = {"complex": 0.0, "raw": 0.0}
+    call = (lambda f: routed(capfd, f)) if capfd is not None else (lambda f: (f(), []))
+    with Stft(nfft, hop, win, lib=lib) as h:
+        for f in range(frames):
+            fr = x[f * hop: f * hop + nfft]
+            s, lines_f = call(lambda: h.process(fr))
+            truth = np.fft.fft(fr.astype(np.float64) * w)
+            e = _rel(s, truth, None)
+            worst["complex"] = max(worst["complex"], e)
+            assert e <= TRUTH_COMPLEX, ("process", nfft, hop, win, f, e)
+            assert s[0].imag == 0 and (nfft % 2 == 1 or s[nfft // 2].imag == 0), ("process", nfft, hop, win, f)
+            out = np.zeros(nfft, np.float32)
+            norm = np.zeros(nfft, np.float32)
+            _, lines_i = call(lambda: h.reconstruct(s, out, norm))
+            frame_truth = np.fft.ifft(s.astype(np.complex128)).real * w
+            e = _rel(out, frame_truth, None)
+            worst["raw"] = max(worst["raw"], e)
+            assert e <= TRUTH_RAW, ("reconstruct", nfft, hop, win, f, e)
+            assert np.array_equal(norm, w * w)
+            if capfd is not None:
+                assert fwd is None or launched(lines_f, fwd, nfft), (nfft, hop, fwd, lines_f)
+                assert inv is None or launched(lines_i, inv, nfft, frames=True), (nfft, hop, inv, lines_i)
+    return worst
+
+
+def check_multipass(lib, oracle, nfft, hop, batch, frames, win="hann", capfd=None, min_passes=2):
+    """The staged chirp-z pipeline over more transforms than its work buffer holds (chirp_reserve caps it at 256 MB, the
+    four-step plans underneath alike): device-resident signals, so one call carries batch * frames transforms and the pass
+    boundaries fall inside a signal.  Spectra, raw and normalised ISTFT against float64 truth at the TRUTH_* bounds, and bit
+    for bit equal to each signal run alone.  With capfd: the pipeline ran min_passes passes or more, forward and inverse."""
+    import torch
+    n = (frames - 1) * hop + nfft + hop // 3
+    x = np.stack([noise(1700 + nfft + i, n) for i in range(batch)])
+    w = oracle.window(win, nfft)[1]
+    xd = torch.from_numpy(x).cuda()
+    call = (lambda f: routed(capfd, f)) if capfd is not None else (lambda f: (f(), []))
+    worst = {}
+    with Stft(nfft, hop, win, lib=lib) as h:
+        def fwd():
+            r = h.batch_forward(xd, "complex", "valid")
+            torch.cuda.synchronize()
+            return r
+        sd, lines_f = call(fwd)
+        assert tuple(sd.shape) == (batch, frames, nfft // 2 + 1)
+
+        def inv(norm):
+            r = h.batch_inverse(sd, n, norm)
+            torch.cuda.synchronize()
+            return r.cpu().numpy()
+        y, lines_i = call(lambda: inv(True))
+        raw = inv(False)
+        s = sd.cpu().numpy()
+        if capfd is not None:
+            assert launched(lines_f, "chirp_staged_fwd", nfft) and launched(lines_i, "chirp_staged_inv", nfft), (lines_f, lines_i)
+            for lines, kern in ((lines_f, "chirp_pre_stft_kernel"), (lines_i, "chirp_pre_spec_kernel")):
+                passes = sum(f"vvb: launch {kern} in" in ln for ln in lines)
+                assert passes >= min_passes, (nfft, kern, passes)
+        worst["complex"] = _rel(s, stft_truth_f64(x, w, nfft, hop), (1, 2))
+        assert worst["complex"] <= TRUTH_COMPLEX, worst
+        acc, wsum = istft_truth_f64(s, w, nfft, hop, n)
+        worst["raw"] = _rel(raw, acc, 1)
+        assert worst["raw"] <= TRUTH_RAW, worst
+        good = wsum > 1e-2
+        worst["norm"] = _rel(y[:, good], acc[:, good] / wsum[good], 1)
+        assert worst["norm"] <= TRUTH_NORM, worst
+        assert np.all(y[:, (frames - 1) * hop + nfft:] == 0)
+        for i in range(batch):
+            one = h.batch_forward(xd[i:i + 1].contiguous(), "complex", "valid")
+            y1 = h.batch_inverse(one, n, True)
+            torch.cuda.synchronize()
+            assert np.array_equal(one.cpu().numpy()[0], s[i]), (nfft, i, "forward: alone != in the batch")
+            assert np.array_equal(y1.cpu().numpy()[0], y[i]), (nfft, i, "inverse: alone != in the batch")
+    return worst
+
+
+# Bound of the log-mel routes against float64 truth, per band and frame:
+#   |exp(lm) - (mel + eps)| <= TRUTH_LOGMEL * sum_k |w_mk| |X_k| * max|X|  +  2^-22 * max(|log(mel + eps)|, 1) * (mel + eps)
+# The first term is the float32 error of |X_k|^2 (about max|X| |X_k| times the spectrum's relative error) carried through
+# the band's weights; the second is two units in the last place of the float32 logarithm itself, which is all a band with
+# no power (log(eps)) may differ by.  A flat bound on the log would hold quiet bands (a few 1e-6 of the frame's power)
+# to the error of the loud bins around them.  About 6 times the worst error in the CPU emulator (3.4e-7); the worst on a B200
+# is not measured yet (test_logmel_route_vs_float64_truth).
+TRUTH_LOGMEL = 2e-6
+
+
+def logmel_truth(x, w, nfft, hop, convention, weights, eps):
+    """float64 mel + eps of |X_truth|^2 under the library's float32 filterbank, and the propagated bound above"""
+    X = stft_truth_f64(x, w, nfft, hop, convention=convention)
+    A = np.abs(X)
+    W = np.asarray(weights, np.float64)
+    mel = (A * A) @ W.T + eps
+    bound = TRUTH_LOGMEL * (A @ np.abs(W).T) * A.max(axis=(-2, -1), keepdims=True)
+    return mel, bound + 2.0 ** -22 * np.maximum(np.abs(np.log(mel)), 1.0) * mel
+
+
+def mfcc_truth(mel, bound, n_coeffs, lifter):
+    """float64 DCT-II (cos(pi (n + 1/2) k / n_mels), unnormalised) of log(mel + eps) with the lifter 1 + L/2 sin(pi k / L), and
+    a bound propagated from the log-mel bound: a log-mel error below bound/(mel+eps) <= 1/2 is at most twice that in the log;
+    plus the float32 cosine table (angle rounded to float32), the float32 sum over n_mels terms and the float32 lifter."""
+    n_mels = mel.shape[-1]
+    k = np.arange(n_coeffs)[:, None]
+    ang = np.pi * (np.arange(n_mels)[None, :] + 0.5) * k / n_mels
+    D = np.cos(ang)
+    lif = np.ones(n_coeffs)
+    if lifter > 0:
+        lif[1:] = 1.0 + lifter / 2.0 * np.sin(np.pi * np.arange(1, n_coeffs) / lifter)
+    lm = np.log(mel)
+    r = bound / mel
+    assert r.max() <= 0.5, r.max()
+    c = (lm @ D.T) * lif
+    absl = np.abs(lm)
+    err = (2 * r) @ np.abs(D).T + absl @ (2.0 ** -22 * (1 + np.abs(ang))).T + n_mels * 2.0 ** -23 * absl.sum(-1, keepdims=True)
+    return c, np.abs(lif) * err + 2.0 ** -21 * np.abs(c)
+
+
+LOGMEL_MODES = {"pair": "one fused kernel, two frames per band-sum phase", "single": "one fused kernel, one frame per band-sum phase",
+                "warp": "one fused kernel, band sums per warp", "chained": "power kernel + log-mel kernel"}
+
+
+def check_logmel_route(lib, oracle, nfft, hop, n_mels, sr, win, route=None, mode=None, capfd=None, batch=2, n=None, eps=1e-10,
+                       n_coeffs=13, lifter=22.0):
+    """batch_logmel and batch_mfcc in all four frame conventions against float64 truth (logmel_truth, mfcc_truth), through
+    whatever path the handle picks for this filterbank.  With capfd the call must launch `route` (route_needles) and the
+    VVB_MEL_DEBUG line must name `mode` (LOGMEL_MODES).  Returns the worst error over TRUTH_LOGMEL's term (relative to
+    sum |w||X| max|X|) and the worst MFCC error as a fraction of its bound."""
+    from vv_dsp_b200 import mel_filterbank
+    st, weights = mel_filterbank(nfft, n_mels, sr, 0.0, sr / 2, lib=lib)
+    assert st == 0
+    n = n or nfft + 40 * hop + hop // 3
+    x = np.stack([noise(2900 + nfft + hop + i, n) for i in range(batch)])
+    w = oracle.window(win, nfft)[1]
+    worst = {"logmel": 0.0, "mfcc": 0.0}
+    call = (lambda f: routed(capfd, f)) if capfd is not None else (lambda f: (f(), []))
+    with Stft(nfft, hop, win, lib=lib) as h:
+        for conv in ("valid", "spectrogram", "padded_tail", "center"):
+            lm, lines = call(lambda: h.batch_logmel(x, weights, eps, conv))
+            if capfd is not None:
+                assert route is None or launched(lines, route, nfft), (nfft, hop, n_mels, route, lines)
+                assert mode is None or f"vvb: STFT -> log-mel: {LOGMEL_MODES[mode]}" in lines, (nfft, hop, n_mels, mode, lines)
+            mel, bound = logmel_truth(x, w, nfft, hop, conv, weights, eps)
+            assert lm.shape == mel.shape == (batch, h.num_frames(n, conv), n_mels), conv
+            err = np.abs(np.exp(lm.astype(np.float64)) - mel)
+            assert np.all(err <= bound), (nfft, hop, n_mels, win, conv, float((err / bound).max()))
+            prop = (bound - 2.0 ** -22 * np.maximum(np.abs(np.log(mel)), 1.0) * mel) / TRUTH_LOGMEL
+            worst["logmel"] = max(worst["logmel"], float((err / np.maximum(prop, 1e-300)).max()))
+            mf = h.batch_mfcc(x, weights, n_coeffs, lifter=lifter, log_epsilon=eps, convention=conv)
+            c, cb = mfcc_truth(mel, bound, n_coeffs, lifter)
+            e = np.abs(mf - c)
+            assert np.all(e <= cb), (nfft, hop, n_mels, win, conv, "mfcc", float((e / cb).max()))
+            worst["mfcc"] = max(worst["mfcc"], float((e / cb).max()))
+    return worst
+
+
+def check_logmel_pcm_truth(lib, oracle, nfft=2048, hop=512, n_mels=80, sr=48000.0, n=30000, batch=3, eps=1e-10):
+    """batch_logmel_pcm (16-bit samples decoded on the device) against the float64 truth of the decoded samples"""
+    from vv_dsp_b200 import mel_filterbank
+    st, weights = mel_filterbank(nfft, n_mels, sr, 0.0, sr / 2, lib=lib)
+    raw = np.random.default_rng(41).integers(-32768, 32768, (batch, n), dtype=np.int16)
+    x = raw.astype(np.float64) / 32768.0
+    w = oracle.window("hann", nfft)[1]
+    with Stft(nfft, hop, "hann", lib=lib) as h:
+        for conv in ("valid", "center"):
+            lm = h.batch_logmel_pcm(raw, weights, 16, eps, conv)
+            mel, bound = logmel_truth(x, w, nfft, hop, conv, weights, eps)
+            err = np.abs(np.exp(lm.astype(np.float64)) - mel)
+            assert lm.shape == mel.shape and np.all(err <= bound), (conv, float((err / bound).max()))
+
+
+# Every log-mel path: (fft_size, hop, n_mels, sample rate, route, mode, switch).  The fused marching kernel at fft_size 2048
+# sums two frames per band-sum phase where shared memory allows; the generic forward kernel fuses the sizes <= 1024 and the
+# mixed-radix ones; every other size, and filterbanks the fused kernels cannot hold, chain the power kernel and a log-mel kernel
+# (logmel_tma_kernel up to 512 bands, logmel_kernel above).
+LOGMEL_ROUTES = ([(2048, h, 80, 48000.0, "logmel_march", "pair", None) for h in (256, 512, 1024)]
+                 + [(2048, 1024, 40, 48000.0, "logmel_march", "single", None)]          # (its short schedule leaves no room for a pair)
+                 + [(2048, 512, 80, 48000.0, "logmel_march", "single", "VVB_MEL_SINGLE"), (2048, 256, 40, 16000.0, "logmel_march", "single", "VVB_MEL_SINGLE")]
+                 + [(N, h, m, sr, "logmel_generic", "warp", None) for N, h, m, sr in
+                    ((256, 64, 40, 8000.0), (512, 128, 40, 16000.0), (1024, 256, 64, 44100.0), (320, 80, 40, 16000.0), (400, 160, 80, 16000.0),
+                     (480, 160, 64, 16000.0), (640, 160, 80, 16000.0))]
+                 + [(N, h, m, sr, "logmel_tma_kernel", "chained", None) for N, h, m, sr in
+                    ((4096, 1024, 128, 48000.0), (8192, 2048, 256, 48000.0), (1000, 250, 40, 16000.0))]
+                 + [(4096, 1024, 600, 48000.0, "logmel_kernel", "chained", None)]
+                 # the filterbanks of check_mel_fused_fallback
+                 + [(400, 160, 200, 16000.0, "logmel_tma_kernel", "chained", None), (400, 160, 128, 16000.0, "logmel_generic", "warp", None),
+                    (1024, 256, 400, 48000.0, "logmel_tma_kernel", "chained", None), (256, 64, 128, 8000.0, "logmel_generic", "warp", None)])
 
 
 MEL_SWITCHES = ("VVB_MEL_NO_TMA", "VVB_MEL_UNIT4", "VVB_MEL_NO_GENERIC", "VVB_MEL_ROW_SPREAD_OFF")

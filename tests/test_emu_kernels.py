@@ -178,7 +178,8 @@ def test_stream_sharding_bit_identical(emu, nfft, hop):
 
 # reduced route matrix: every kernel family, Hann plus one other window (the full matrix runs in test_gpu_parity.py)
 EMU_ROUTES = [(2048, 512, "hamming"), (4096, 1024, "boxcar"), (8192, 2048, "hann"), (1024, 512, "hann"), (256, 32, "hamming"),
-              (2048, 441, "hamming"), (512, 75, "boxcar"), (4096, 1000, "hann"), (8192, 441, "hann"), (1024, 100, "hamming")]
+              (2048, 441, "hamming"), (512, 75, "boxcar"), (4096, 1000, "hann"), (8192, 441, "hann"), (1024, 100, "hamming"),
+              (480, 160, "hamming"), (100, 25, "hann"), (1000, 1000, "hamming"), (31, 9, "hamming")]
 
 
 @pytest.mark.parametrize("nfft,hop,win", EMU_ROUTES)
@@ -190,6 +191,37 @@ def test_route_vs_float64_truth(emu, oracle, capfd, nfft, hop, win):
     worst = pc.check_route(emu, oracle, nfft, hop, win, n, batch=2, big_batch=5, capfd=capfd, fwd=fwd, inv=inv,
                            min_chunks=4 if inv == "stft_inverse_kernel" else None)
     print("route", nfft, hop, win, fwd, inv, worst)
+
+
+@pytest.mark.parametrize("env,nfft,hop,fwd,inv", pc.SWITCH_ROUTES)
+def test_switch_route_vs_float64_truth(emu, oracle, capfd, monkeypatch, env, nfft, hop, fwd, inv):
+    """the separate-kernel chirp-z pipeline and the O(n^2) kernels, selected by their switches, against float64 truth"""
+    monkeypatch.setenv(env, "1")
+    pc.check_route(emu, oracle, nfft, hop, "hann", pc.route_length(nfft, hop, inv), big_batch=5, capfd=capfd, fwd=fwd, inv=inv)
+
+
+@pytest.mark.parametrize("env,nfft,hop,fwd,inv", [(None, 512, 128, "stft_forward_kernel", "stft_inverse_kernel"),
+                                                  (None, 400, 160, "stft_forward_kernel", "stft_inverse_kernel"),
+                                                  (None, 1000, 250, "chirp_fused_fwd", "chirp_fused_inv"),
+                                                  (None, 12, 5, "stft_forward_direct_kernel", "stft_inverse_direct_kernel")]
+                         + pc.SWITCH_ROUTES)
+def test_per_frame_route_vs_float64_truth(emu, oracle, capfd, monkeypatch, env, nfft, hop, fwd, inv):
+    """vv_dsp_stft_process / reconstruct against float64 truth, one row per family (the staged chirp-z one by its switch)"""
+    if env:
+        monkeypatch.setenv(env, "1")
+    pc.check_per_frame_route(emu, oracle, nfft, hop, "hamming", frames=3, capfd=capfd, fwd=fwd, inv=inv)
+
+
+# one row per log-mel path: fused marching kernel (pair, single), fused generic kernel, chained logmel_tma_kernel (a chirp-z
+# size), chained logmel_kernel (> 512 bands)
+EMU_LOGMEL_ROUTES = [r for r in pc.LOGMEL_ROUTES if r[:3] in ((2048, 512, 80), (2048, 1024, 40), (400, 160, 80), (1000, 250, 40), (4096, 1024, 600))
+                     and r[6] is None]
+
+
+@pytest.mark.parametrize("nfft,hop,n_mels,sr,route,mode,env", EMU_LOGMEL_ROUTES)
+def test_logmel_route_vs_float64_truth(emu, oracle, capfd, nfft, hop, n_mels, sr, route, mode, env):
+    win = "hamming" if nfft in (400, 4096) else "hann"
+    print(pc.check_logmel_route(emu, oracle, nfft, hop, n_mels, sr, win, route, mode, capfd=capfd, n=nfft + 12 * hop + hop // 3))
 
 
 @pytest.mark.parametrize("env,nfft,hop,inv", [("VVB_NO_WS", 2048, 256, "istft_march_kernel"),

@@ -592,7 +592,13 @@ static vv_dsp_status batch_mel_chain(vv_dsp_stft* h, const void* signals_v, int 
     /* one kernel from samples to log-mel rows where the plan has it (fft_size 2048 marching kernel): the power spectrogram
      * then never exists in HBM and there is no scratch; chunks only bound the host staging buffers */
     fused = !st && h->mel.d_fw && vvb_stft_forward_logmel_ok(h->eng, h->mel.f_segments, h->mel.f_prow, h->mel.f_unit, n_mels);
-    if (getenv("VVB_MEL_DEBUG")) fprintf(stderr, "vvb: STFT -> log-mel: %s\n", fused ? "one fused kernel" : "power kernel + log-mel kernel");
+    if (getenv("VVB_MEL_DEBUG")) {
+        /* 2 / 1: marching kernel with two frames / one frame per band-sum phase; 3: generic kernel, band sums per warp */
+        const int mode = fused ? vvb_stft_forward_logmel_ok(h->eng, h->mel.f_segments, h->mel.f_prow, h->mel.f_unit, n_mels) : 0;
+        fprintf(stderr, "vvb: STFT -> log-mel: %s\n", mode == 2 ? "one fused kernel, two frames per band-sum phase"
+                                                    : mode == 1 ? "one fused kernel, one frame per band-sum phase"
+                                                    : mode ? "one fused kernel, band sums per warp" : "power kernel + log-mel kernel");
+    }
     if (fused) {
         const size_t stage_target = h->stage_target;                   /* VVB_STAGE_TARGET_BYTES applies here too */
         cs = batch;
