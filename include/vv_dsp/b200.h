@@ -242,6 +242,44 @@ VV_DSP_NODISCARD vv_dsp_status vv_dsp_b200_pcm_to_planar(const void* interleaved
                                                          size_t num_samples, size_t channels, vv_dsp_real* planar,
                                                          vv_dsp_mem_space out_space, size_t planar_pitch, void* cuda_stream);
 
+/* ---------------------------------------------------------------------------------------------------------------
+ * Batched FIR filtering by FFT convolution (overlap-save), one fused kernel per filter partition.
+ *
+ *   out[b][i] = sum_{j < num_taps} h_b[j] x_b[i - j],   0 <= i < n_out,
+ * where x_b[k] = 0 outside [0, n) and h_b = filters[num_filters == 1 ? 0 : b] (rows of num_taps taps).
+ * n_out = n is causal FIR filtering (scipy.signal.lfilter(h, 1, x)); n_out = n + num_taps - 1 is the full linear
+ * convolution; samples beyond that are 0.  Pitches (in elements) of 0 mean dense.  Memory spaces as above: if every
+ * buffer is DEVICE the call only enqueues on the handle's stream, otherwise it returns once the results are in host
+ * memory.  `out` must not overlap `signals`; an identical base pointer is rejected with VV_DSP_ERROR_UNSUPPORTED.
+ *
+ * Plan: a handle is created for a tap count M and picks, as a pure function of M, a complex transform size
+ * N in {128, 256, ..., 8192} and P partitions of Lp = ceil(M / P) <= N taps: the smallest P N log2(N) / (N - Lp + 1)
+ * (transform work per output sample), ties to the smaller N and then the fewer partitions.  That gives N = 128 for
+ * M <= 29, 256 to M = 52, 512 to 94, 1024 to 171, 2048 to 316, 4096 to 586 and 8192 from M = 587; one partition up to
+ * M = 5462, two from 5463, 12 at 48 000.  Every M >= 1 runs on the GPU: partition p (taps p Lp ... (p+1) Lp) is one
+ * pass of the kernel delayed by p Lp samples that adds into `out`, in ascending p, so results are deterministic.
+ * The filter spectra are built on the device in every call (filters change per batch in augmentation); per-signal
+ * filters are processed in chunks of signals whose spectra fit a bounded scratch of the handle.
+ *
+ * Status: NULL pointer -> VV_DSP_ERROR_NULL_POINTER; num_taps == 0 (or above 2^31 - 1), num_filters not in {1, batch}
+ * or a pitch smaller than its row -> VV_DSP_ERROR_INVALID_SIZE; a bad memory space -> VV_DSP_ERROR_OUT_OF_RANGE;
+ * out == signals -> VV_DSP_ERROR_UNSUPPORTED; batch == 0 or n_out == 0 -> VV_DSP_OK with no work; CUDA failures
+ * -> VV_DSP_ERROR_INTERNAL (no usable device at creation: VV_DSP_ERROR_UNSUPPORTED).
+ * ------------------------------------------------------------------------------------------------------------- */
+typedef struct vv_dsp_fir vv_dsp_fir;
+VV_DSP_NODISCARD vv_dsp_status vv_dsp_fir_create(size_t num_taps, vv_dsp_fir** out);
+vv_dsp_status vv_dsp_fir_destroy(vv_dsp_fir* f);
+/* same rules as vv_dsp_stft_set_stream (NULL = the handle's own stream) */
+vv_dsp_status vv_dsp_fir_set_stream(vv_dsp_fir* f, void* cuda_stream);
+vv_dsp_status vv_dsp_fir_synchronize(vv_dsp_fir* f);
+/* the transform size N and the number of filter partitions P (passes) the handle uses */
+vv_dsp_status vv_dsp_fir_get_config(const vv_dsp_fir* f, size_t* fft_size, size_t* partitions);
+VV_DSP_NODISCARD vv_dsp_status vv_dsp_fir_filter_batch(
+    vv_dsp_fir* f,
+    const vv_dsp_real* filters, vv_dsp_mem_space filters_space, size_t num_filters, size_t filter_pitch,
+    const vv_dsp_real* signals, vv_dsp_mem_space signals_space, size_t batch, size_t n, size_t signal_pitch,
+    vv_dsp_real* out, vv_dsp_mem_space out_space, size_t n_out, size_t out_pitch);
+
 /* Library / device introspection */
 const char* vv_dsp_b200_version(void);
 /* last CUDA error text seen by the calling thread ("" if none) */

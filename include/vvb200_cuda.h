@@ -127,6 +127,21 @@ void vvb_fft_engine_destroy(vvb_fft_engine* e);
 int vvb_fft_engine_is_single_kernel(const vvb_fft_engine* e);   /* one kernel that reads its input once */
 int vvb_fft_exec(vvb_fft_engine* e, const void* d_in, void* d_out, size_t batch, void* stream);
 
+/* ---- FIR by overlap-save (csrc/host/fir.c): m = transform size, a power of two in [128, 8192] */
+typedef struct vvb_fir_engine vvb_fir_engine;
+int vvb_fir_engine_create(size_t m, vvb_fir_engine** out);
+void vvb_fir_engine_destroy(vvb_fir_engine* e);
+/* filter spectra: d_spec [filters][parts][m] = FFT_m of the zero-padded partition h_f[p lp .. (p+1) lp) (taps beyond
+ * num_taps read as 0), times 1/m.  d_h: [filters][h_pitch] floats. */
+int vvb_fir_spectra(vvb_fir_engine* e, const float* d_h, size_t filters, size_t h_pitch, size_t num_taps, size_t lp,
+                    size_t parts, vvb_cpx* d_spec, void* stream);
+/* d_y[b][i] = sum_j h_b[j] x_b[i - j], i < n_out (0 from n + num_taps - 1 on), by `parts` passes of the overlap-save
+ * kernel in ascending partition order (pass p delayed by p lp, passes after the first add into d_y).  d_spec as built by
+ * vvb_fir_spectra; spec_stride: complex values from one signal's spectra to the next's (0: one filter for all). */
+int vvb_fir_filter(vvb_fir_engine* e, const vvb_cpx* d_spec, size_t spec_stride, size_t num_taps, size_t lp, size_t parts,
+                   const float* d_x, size_t batch, size_t n, size_t x_pitch, float* d_y, size_t n_out, size_t y_pitch,
+                   void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -109,13 +109,21 @@ class Library:
         "vv_dsp_stft_stream_download": (C.c_int, [_vp, _vp]),
         "vv_dsp_stft_stream_download_spectra": (C.c_int, [_vp, _vp]),
         "vv_dsp_stft_stream_time_roundtrip": (C.c_int, [_vp, _sz, _sz, C.POINTER(C.c_double)]),
+        "vv_dsp_fir_create": (C.c_int, [_sz, C.POINTER(_vp)]),
+        "vv_dsp_fir_destroy": (C.c_int, [_vp]),
+        "vv_dsp_fir_set_stream": (C.c_int, [_vp, _vp]),
+        "vv_dsp_fir_synchronize": (C.c_int, [_vp]),
+        "vv_dsp_fir_get_config": (C.c_int, [_vp, C.POINTER(_sz), C.POINTER(_sz)]),
+        "vv_dsp_fir_filter_batch": (C.c_int, [_vp, _vp, C.c_int, _sz, _sz, _vp, C.c_int, _sz, _sz, _sz, _vp, C.c_int, _sz, _sz]),
     }
     # entry points newer than round 1: absent from an old library variant loaded for an A/B measurement
     OPTIONAL = {"vv_dsp_b200_sm_clock_mhz", "vv_dsp_stft_shard_inverse", "vv_dsp_stft_device", "vv_dsp_stft_get_stream",
                 "vv_dsp_stft_stream_create", "vv_dsp_stft_stream_destroy", "vv_dsp_stft_stream_num_frames",
                 "vv_dsp_stft_stream_get_shard", "vv_dsp_stft_stream_upload", "vv_dsp_stft_stream_forward",
                 "vv_dsp_stft_stream_inverse", "vv_dsp_stft_stream_roundtrip", "vv_dsp_stft_stream_synchronize",
-                "vv_dsp_stft_stream_download", "vv_dsp_stft_stream_download_spectra", "vv_dsp_stft_stream_time_roundtrip"}
+                "vv_dsp_stft_stream_download", "vv_dsp_stft_stream_download_spectra", "vv_dsp_stft_stream_time_roundtrip",
+                "vv_dsp_fir_create", "vv_dsp_fir_destroy", "vv_dsp_fir_set_stream", "vv_dsp_fir_synchronize", "vv_dsp_fir_get_config",
+                "vv_dsp_fir_filter_batch"}
 
     def __init__(self, path: str | None = None):
         path = path or DEFAULT_LIB
@@ -696,6 +704,103 @@ class StftStream:
         _check(self.lib, self.lib.vv_dsp_stft_stream_time_roundtrip(self._s, warmup, steps, C.byref(ms)),
                "vv_dsp_stft_stream_time_roundtrip")
         return float(ms.value)
+
+
+# ----------------------------------------------------------------------------- FIR filtering
+class FirFilter:
+    """vv_dsp_fir handle (include/vv_dsp/b200.h): batched FIR filtering by FFT convolution on the device.
+    out[b][i] = sum_j h_b[j] x_b[i - j] for i < n_out; n_out = n is lfilter(h, 1, x), n + num_taps - 1 the full convolution."""
+
+    def __init__(self, num_taps, lib: Library | None = None):
+        self.lib = lib or default_library()
+        self.num_taps = int(num_taps)
+        self._f = _vp()
+        _check(self.lib, self.lib.vv_dsp_fir_create(self.num_taps, C.byref(self._f)), "vv_dsp_fir_create")
+        n, p = _sz(0), _sz(0)
+        _check(self.lib, self.lib.vv_dsp_fir_get_config(self._f, C.byref(n), C.byref(p)), "vv_dsp_fir_get_config")
+        self.fft_size, self.partitions = int(n.value), int(p.value)
+        self._stream_pinned = False
+        self._bound_stream = None
+
+    def close(self):
+        if getattr(self, "_f", None) is not None and self._f.value:
+            self.lib.vv_dsp_fir_destroy(self._f)
+            self._f = _vp()
+
+    __del__ = close
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def set_stream(self, cuda_stream):
+        """Pin the handle to a stream (a cudaStream_t as an integer; 0 = the legacy default stream); None = its own
+        stream and back to automatic binding to torch's current stream (see Stft.set_stream)."""
+        self._stream_pinned = cuda_stream is not None
+        self._set_stream_raw(cuda_stream)
+
+    def _set_stream_raw(self, cuda_stream):
+        arg = None if cuda_stream is None else _vp(int(cuda_stream) or 1)
+        _check(self.lib, self.lib.vv_dsp_fir_set_stream(self._f, arg), "vv_dsp_fir_set_stream")
+        self._bound_stream = None if cuda_stream is None else (int(cuda_stream) or 1)
+
+    def _bind_torch_stream(self, tensor):
+        """device calls are enqueued on torch's current stream of the tensor's device, as Stft._bind_torch_stream does"""
+        if self._stream_pinned:
+            return
+        import torch
+        cur = int(torch.cuda.current_stream(tensor.device).cuda_stream) or 1
+        if cur != self._bound_stream:
+            self._set_stream_raw(cur)
+
+    def synchronize(self):
+        _check(self.lib, self.lib.vv_dsp_fir_synchronize(self._f), "vv_dsp_fir_synchronize")
+
+    @staticmethod
+    def _rows(a, what):
+        """(container, rows, row length, row pitch in elements); device tensors keep their layout (odd pitches of views
+        included), host arrays are made dense float32"""
+        if _is_device(a):
+            Stft._check_device_tensor(a, "float32", what)
+            if a.ndim != 2:
+                raise ValueError(f"{what}: expected a 2-D tensor")
+            return a, int(a.shape[0]), int(a.shape[1]), (int(a.stride(0)) if a.shape[0] > 1 else 0)
+        a = np.ascontiguousarray(a, np.float32)
+        if a.ndim != 2:
+            raise ValueError(f"{what}: expected a 2-D array")
+        return a, int(a.shape[0]), int(a.shape[1]), 0
+
+    def filter(self, filters, signals, n_out=None, out=None):
+        """filters: [1 or batch, num_taps], signals: [batch, n] float32 (numpy, or torch CUDA tensors).  Returns
+        [batch, n_out] float32 (default n_out = n) in the container of `signals` unless `out` is given."""
+        filters, nf, taps, fpitch = self._rows(filters, "filters")
+        signals, batch, n, spitch = self._rows(signals, "signals")
+        if taps != self.num_taps:
+            raise ValueError(f"filters: rows of {taps} taps, the handle was created for {self.num_taps}")
+        n_out = n if n_out is None else int(n_out)
+        if out is None:
+            if _is_device(signals):
+                import torch
+                out = torch.empty((batch, n_out), device=signals.device, dtype=torch.float32)
+            else:
+                out = np.empty((batch, n_out), np.float32)
+        elif not _is_device(out):
+            assert out.dtype == np.float32 and out.flags.c_contiguous
+        opitch = 0
+        if _is_device(out):
+            Stft._check_device_tensor(out, "float32", "out")
+            assert out.ndim == 2 and int(out.shape[0]) == batch and int(out.shape[1]) == n_out
+            opitch = int(out.stride(0)) if batch > 1 else 0
+        dev = next((t for t in (out, signals, filters) if _is_device(t)), None)
+        if dev is not None:
+            self._bind_torch_stream(dev)
+        st = self.lib.vv_dsp_fir_filter_batch(self._f, _ptr(filters), DEVICE if _is_device(filters) else HOST, nf, fpitch,
+                                              _ptr(signals), DEVICE if _is_device(signals) else HOST, batch, n, spitch,
+                                              _ptr(out), DEVICE if _is_device(out) else HOST, n_out, opitch)
+        _check(self.lib, st, "vv_dsp_fir_filter_batch")
+        return out
 
 
 # ----------------------------------------------------------------------------- FFT plan

@@ -9,6 +9,7 @@
  */
 #include "vvb_rt.cuh"
 #include "vvb_direct_kernels.cuh"
+#include "vvb_fir_kernels.cuh"
 
 #include <algorithm>
 #include <cmath>
@@ -805,6 +806,70 @@ extern "C" int vvb_fft_exec(vvb_fft_engine* e, const void* d_in, void* d_out, si
     if (e->type == 1)   /* R2C: one frame per transform, boxcar window, complex half spectrum */
         return vvb_stft_forward(e->real, (const float*)d_in, batch, e->n, e->n, 1, PAD_ZERO, OUT_COMPLEX, d_out, bins, stream);
     return vvb_stft_inverse_frames(e->real, (const vvb_cpx*)d_in, batch, bins, (float*)d_out, stream);   /* C2R */
+}
+
+/* ------------------------------------------------------------------ FIR by overlap-save */
+/* the forward C2C plan of the transform size: its tables feed fir_ols_kernel, its kernel makes the filter spectra */
+struct vvb_fir_engine {
+    vvb_fft_engine* fwd = nullptr;
+};
+
+extern "C" int vvb_fir_engine_create(size_t m, vvb_fir_engine** out)
+{
+    if (!out) return fail(1, "vvb_fir_engine_create", "null");
+    *out = nullptr;
+    if (m < 128 || m > 8192 || (m & (m - 1)) != 0) return fail(6, "vvb_fir_engine_create", "no Stockham kernel for this size");
+    vvb_fir_engine* e = new (std::nothrow) vvb_fir_engine();
+    if (!e) return fail(4, "vvb_fir_engine_create", "oom");
+    if (int st = vvb_fft_engine_create(m, 0, 1, &e->fwd)) { delete e; return st; }
+    *out = e;
+    return 0;
+}
+
+extern "C" void vvb_fir_engine_destroy(vvb_fir_engine* e)
+{
+    if (!e) return;
+    vvb_fft_engine_destroy(e->fwd);
+    delete e;
+}
+
+extern "C" int vvb_fir_spectra(vvb_fir_engine* e, const float* d_h, size_t filters, size_t h_pitch, size_t num_taps, size_t lp,
+                               size_t parts, vvb_cpx* d_spec, void* stream)
+{
+    if (!e || !d_h || !d_spec) return fail(1, "vvb_fir_spectra", "null");
+    if (filters == 0) return 0;
+    const size_t m = e->fwd->n;
+    if (lp == 0 || lp > m || parts == 0) return fail(2, "vvb_fir_spectra", "partition");
+    FirPadArgs a;
+    a.h = d_h; a.h_pitch = (long long)h_pitch; a.taps = (long long)num_taps; a.out = (float2*)d_spec;
+    a.total = (long long)(filters * parts * m); a.m = (int)m; a.lp = (int)lp; a.parts = (int)parts;
+    if (int st = tu_fir_pad(a, e->fwd->sms, stream)) return st;
+    return vvb_fft_exec(e->fwd, d_spec, d_spec, filters * parts, stream);      /* in place: each team reads before it writes */
+}
+
+extern "C" int vvb_fir_filter(vvb_fir_engine* e, const vvb_cpx* d_spec, size_t spec_stride, size_t num_taps, size_t lp, size_t parts,
+                              const float* d_x, size_t batch, size_t n, size_t x_pitch, float* d_y, size_t n_out, size_t y_pitch,
+                              void* stream)
+{
+    if (!e || !d_spec || !d_x || !d_y) return fail(1, "vvb_fir_filter", "null");
+    if (batch == 0 || n_out == 0) return 0;
+    const size_t m = e->fwd->n;
+    if (lp == 0 || lp > m || parts == 0 || (parts - 1) * lp >= num_taps) return fail(2, "vvb_fir_filter", "partition");
+    FirArgs a;
+    a.x = d_x; a.x_pitch = (long long)x_pitch; a.n = (long long)n;
+    a.y = d_y; a.y_pitch = (long long)y_pitch; a.n_out = (long long)n_out; a.n_full = (long long)(n + num_taps - 1);
+    a.h_stride = (long long)spec_stride;
+    a.lp = (int)lp; a.L = (int)(m - lp + 1);
+    a.blocks = ((long long)n_out + a.L - 1) / a.L;
+    a.pairs = (a.blocks + 1) / 2;
+    a.count = (long long)batch * a.pairs;
+    a.tables = e->fwd->d_tables;
+    for (size_t p = 0; p < parts; ++p) {          /* ascending partitions: every output sample sums its passes in one order */
+        a.H = (const float2*)d_spec + p * m;
+        a.delay = (long long)(p * lp);
+        if (int st = tu_fir((int)m, a, p > 0, e->fwd->sms, stream)) return st;
+    }
+    return 0;
 }
 
 /* ---------------------------------------------------------------------- Bluestein plumbing */

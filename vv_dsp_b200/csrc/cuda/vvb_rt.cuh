@@ -140,5 +140,9 @@ int tu_inv_march_8192(size_t hop, const InvArgs& a, long long batch, int sms, vo
 int tu_inv_pair(int nfft, size_t hop, const InvArgs& a, long long batch, int sms, const float* tables_p, const float* tables_real, void* stream);
 int tu_c2c(int n, const C2CArgs& a, int sms, void* stream);
 int tu_chirp_fused(size_t M, const ChirpFusedArgs& a, int sms, void* stream);
+struct FirArgs;
+struct FirPadArgs;
+int tu_fir(int m, const FirArgs& a, bool accum, int sms, void* stream);    /* one overlap-save pass (vvb_fir_kernels.cuh) */
+int tu_fir_pad(const FirPadArgs& a, int sms, void* stream);
 
 }  // namespace vvb
