@@ -280,6 +280,46 @@ VV_DSP_NODISCARD vv_dsp_status vv_dsp_fir_filter_batch(
     const vv_dsp_real* signals, vv_dsp_mem_space signals_space, size_t batch, size_t n, size_t signal_pitch,
     vv_dsp_real* out, vv_dsp_mem_space out_space, size_t n_out, size_t out_pitch);
 
+/* ---------------------------------------------------------------------------------------------------------------
+ * Batched rational-ratio resampling by a polyphase FIR: scipy.signal.resample_poly(x, up, down, window=..., padtype=
+ * 'constant') row by row.  up / down are first divided by their gcd.  With K taps w, h = up w and half = (K - 1) / 2:
+ *
+ *   y[m] = sum_k h[k] xu[m down + half - k],   0 <= m < n_out = ceil(n up / down),
+ *   xu[q] = x[q / up] if up divides q and 0 <= q / up < n, else 0.
+ *
+ * taps == NULL (num_taps 0) designs scipy's default filter, firwin(2 half + 1, 1 / max(up, down), window=('kaiser', 5.0))
+ * with half = 10 max(up, down), in double; otherwise the num_taps host floats are the window argument of resample_poly.
+ * The bank of T = ceil(K / up) taps per phase is rounded to float32 once and lives on the device.  up == down == 1 after
+ * reduction copies the input bit for bit and ignores the filter.  Every output sums its T products in one fixed order,
+ * so a signal gives the same bits alone or inside any batch, from HOST or DEVICE buffers.
+ *
+ * Pitches (in elements) of 0 mean dense.  Memory spaces as above: if both buffers are DEVICE the call only enqueues on
+ * the handle's stream, otherwise it returns once the results are in host memory.  `out` must not overlap `signals`; an
+ * identical base pointer is rejected with VV_DSP_ERROR_UNSUPPORTED.  *out_len receives n_out.
+ *
+ * Status: NULL handle / signals / out / out_len, or taps == NULL with num_taps > 0 -> VV_DSP_ERROR_NULL_POINTER; up or
+ * down == 0, taps with num_taps == 0, a bank up T above 65 536 taps, up or down above 2^31 - 1 after reduction, a pitch
+ * smaller than its row or n up >= 2^62 -> VV_DSP_ERROR_INVALID_SIZE; a bad memory space -> VV_DSP_ERROR_OUT_OF_RANGE;
+ * out == signals -> VV_DSP_ERROR_UNSUPPORTED; batch == 0 or n == 0 -> VV_DSP_OK with no work; CUDA failures ->
+ * VV_DSP_ERROR_INTERNAL (no usable device at creation: VV_DSP_ERROR_UNSUPPORTED).
+ * ------------------------------------------------------------------------------------------------------------- */
+typedef struct vv_dsp_resample_poly vv_dsp_resample_poly;
+VV_DSP_NODISCARD vv_dsp_status vv_dsp_resample_poly_create(size_t up, size_t down, const vv_dsp_real* taps /* HOST or NULL */,
+                                                           size_t num_taps, vv_dsp_resample_poly** out);
+vv_dsp_status vv_dsp_resample_poly_destroy(vv_dsp_resample_poly* r);
+/* same rules as vv_dsp_stft_set_stream (NULL = the handle's own stream) */
+vv_dsp_status vv_dsp_resample_poly_set_stream(vv_dsp_resample_poly* r, void* cuda_stream);
+vv_dsp_status vv_dsp_resample_poly_synchronize(vv_dsp_resample_poly* r);
+/* the reduced up / down, the filter length K and the taps per phase T */
+vv_dsp_status vv_dsp_resample_poly_get_config(const vv_dsp_resample_poly* r, size_t* up, size_t* down, size_t* num_taps,
+                                              size_t* taps_per_phase);
+/* ceil(n up / down); 0 for a NULL handle */
+size_t vv_dsp_resample_poly_output_length(const vv_dsp_resample_poly* r, size_t n);
+VV_DSP_NODISCARD vv_dsp_status vv_dsp_resample_poly_batch(
+    vv_dsp_resample_poly* r,
+    const vv_dsp_real* signals, vv_dsp_mem_space signals_space, size_t batch, size_t n, size_t signal_pitch,
+    vv_dsp_real* out, vv_dsp_mem_space out_space, size_t out_pitch, size_t* out_len);
+
 /* Library / device introspection */
 const char* vv_dsp_b200_version(void);
 /* last CUDA error text seen by the calling thread ("" if none) */

@@ -39,6 +39,7 @@ int vvb_memcpy_h2d(void* dst, const void* src, size_t bytes, void* stream);
 int vvb_memcpy_d2h(void* dst, const void* src, size_t bytes, void* stream);
 int vvb_memcpy2d_h2d(void* dst, size_t dpitch, const void* src, size_t spitch, size_t width, size_t height, void* stream);
 int vvb_memcpy2d_d2h(void* dst, size_t dpitch, const void* src, size_t spitch, size_t width, size_t height, void* stream);
+int vvb_memcpy2d_d2d(void* dst, size_t dpitch, const void* src, size_t spitch, size_t width, size_t height, void* stream);
 int vvb_memset(void* dst, int value, size_t bytes, void* stream);
 int vvb_stream_create(void** stream);
 int vvb_stream_destroy(void* stream);
@@ -141,6 +142,14 @@ int vvb_fir_spectra(vvb_fir_engine* e, const float* d_h, size_t filters, size_t 
 int vvb_fir_filter(vvb_fir_engine* e, const vvb_cpx* d_spec, size_t spec_stride, size_t num_taps, size_t lp, size_t parts,
                    const float* d_x, size_t batch, size_t n, size_t x_pitch, float* d_y, size_t n_out, size_t y_pitch,
                    void* stream);
+
+/* ---- polyphase resampling (csrc/host/resample.c): up, down coprime; d_bank [taps_per_phase][up] (phase-minor) holds
+ * h[phi + j up], the filter already scaled by up, 0 past its end; half = (num_taps - 1) / 2.
+ *   d_y[b][m] = sum_{j < T} d_bank[j][phi] x_b[i0 - j],  q0 = m down + half, phi = q0 mod up, i0 = q0 div up,  m < n_out,
+ * x_b = 0 outside [0, n); every output sums its products in one fixed order, whatever the batch. */
+int vvb_resample_poly(const float* d_bank, size_t up, size_t down, size_t taps_per_phase, size_t half,
+                      const float* d_x, size_t batch, size_t n, size_t x_pitch, float* d_y, size_t n_out, size_t y_pitch,
+                      void* stream);
 
 #ifdef __cplusplus
 }

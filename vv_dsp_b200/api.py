@@ -115,6 +115,13 @@ class Library:
         "vv_dsp_fir_synchronize": (C.c_int, [_vp]),
         "vv_dsp_fir_get_config": (C.c_int, [_vp, C.POINTER(_sz), C.POINTER(_sz)]),
         "vv_dsp_fir_filter_batch": (C.c_int, [_vp, _vp, C.c_int, _sz, _sz, _vp, C.c_int, _sz, _sz, _sz, _vp, C.c_int, _sz, _sz]),
+        "vv_dsp_resample_poly_create": (C.c_int, [_sz, _sz, _vp, _sz, C.POINTER(_vp)]),
+        "vv_dsp_resample_poly_destroy": (C.c_int, [_vp]),
+        "vv_dsp_resample_poly_set_stream": (C.c_int, [_vp, _vp]),
+        "vv_dsp_resample_poly_synchronize": (C.c_int, [_vp]),
+        "vv_dsp_resample_poly_get_config": (C.c_int, [_vp, C.POINTER(_sz), C.POINTER(_sz), C.POINTER(_sz), C.POINTER(_sz)]),
+        "vv_dsp_resample_poly_output_length": (_sz, [_vp, _sz]),
+        "vv_dsp_resample_poly_batch": (C.c_int, [_vp, _vp, C.c_int, _sz, _sz, _sz, _vp, C.c_int, _sz, C.POINTER(_sz)]),
     }
     # entry points newer than round 1: absent from an old library variant loaded for an A/B measurement
     OPTIONAL = {"vv_dsp_b200_sm_clock_mhz", "vv_dsp_stft_shard_inverse", "vv_dsp_stft_device", "vv_dsp_stft_get_stream",
@@ -123,7 +130,9 @@ class Library:
                 "vv_dsp_stft_stream_inverse", "vv_dsp_stft_stream_roundtrip", "vv_dsp_stft_stream_synchronize",
                 "vv_dsp_stft_stream_download", "vv_dsp_stft_stream_download_spectra", "vv_dsp_stft_stream_time_roundtrip",
                 "vv_dsp_fir_create", "vv_dsp_fir_destroy", "vv_dsp_fir_set_stream", "vv_dsp_fir_synchronize", "vv_dsp_fir_get_config",
-                "vv_dsp_fir_filter_batch"}
+                "vv_dsp_fir_filter_batch", "vv_dsp_resample_poly_create", "vv_dsp_resample_poly_destroy",
+                "vv_dsp_resample_poly_set_stream", "vv_dsp_resample_poly_synchronize", "vv_dsp_resample_poly_get_config",
+                "vv_dsp_resample_poly_output_length", "vv_dsp_resample_poly_batch"}
 
     def __init__(self, path: str | None = None):
         path = path or DEFAULT_LIB
@@ -800,6 +809,95 @@ class FirFilter:
                                               _ptr(signals), DEVICE if _is_device(signals) else HOST, batch, n, spitch,
                                               _ptr(out), DEVICE if _is_device(out) else HOST, n_out, opitch)
         _check(self.lib, st, "vv_dsp_fir_filter_batch")
+        return out
+
+
+# ----------------------------------------------------------------------------- resampling
+class Resampler:
+    """vv_dsp_resample_poly handle (include/vv_dsp/b200.h): batched rational-ratio resampling by a polyphase FIR on the
+    device, scipy.signal.resample_poly(x, up, down, window=taps, padtype='constant') row by row.  taps=None designs scipy's
+    default Kaiser (beta 5) filter; up / down are reduced by their gcd."""
+
+    def __init__(self, up, down, taps=None, lib: Library | None = None):
+        self.lib = lib or default_library()
+        self._r = _vp()
+        t = None if taps is None else np.ascontiguousarray(np.asarray(taps, np.float32).ravel())
+        st = self.lib.vv_dsp_resample_poly_create(int(up), int(down), None if t is None else t.ctypes.data_as(_vp),
+                                                  0 if t is None else t.size, C.byref(self._r))
+        _check(self.lib, st, "vv_dsp_resample_poly_create")
+        u, d, k, tp = _sz(0), _sz(0), _sz(0), _sz(0)
+        _check(self.lib, self.lib.vv_dsp_resample_poly_get_config(self._r, C.byref(u), C.byref(d), C.byref(k), C.byref(tp)),
+               "vv_dsp_resample_poly_get_config")
+        self.up, self.down, self.num_taps, self.taps_per_phase = int(u.value), int(d.value), int(k.value), int(tp.value)
+        self._stream_pinned = False
+        self._bound_stream = None
+
+    def close(self):
+        if getattr(self, "_r", None) is not None and self._r.value:
+            self.lib.vv_dsp_resample_poly_destroy(self._r)
+            self._r = _vp()
+
+    __del__ = close
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def output_length(self, n) -> int:
+        """ceil(n up / down)"""
+        return int(self.lib.vv_dsp_resample_poly_output_length(self._r, int(n)))
+
+    def set_stream(self, cuda_stream):
+        """Pin the handle to a stream (a cudaStream_t as an integer; 0 = the legacy default stream); None = its own
+        stream and back to automatic binding to torch's current stream (see Stft.set_stream)."""
+        self._stream_pinned = cuda_stream is not None
+        self._set_stream_raw(cuda_stream)
+
+    def _set_stream_raw(self, cuda_stream):
+        arg = None if cuda_stream is None else _vp(int(cuda_stream) or 1)
+        _check(self.lib, self.lib.vv_dsp_resample_poly_set_stream(self._r, arg), "vv_dsp_resample_poly_set_stream")
+        self._bound_stream = None if cuda_stream is None else (int(cuda_stream) or 1)
+
+    def _bind_torch_stream(self, tensor):
+        if self._stream_pinned:
+            return
+        import torch
+        cur = int(torch.cuda.current_stream(tensor.device).cuda_stream) or 1
+        if cur != self._bound_stream:
+            self._set_stream_raw(cur)
+
+    def synchronize(self):
+        _check(self.lib, self.lib.vv_dsp_resample_poly_synchronize(self._r), "vv_dsp_resample_poly_synchronize")
+
+    def resample(self, signals, out=None):
+        """signals: [batch, n] float32 (numpy, or a torch CUDA tensor, views with a row pitch included).  Returns
+        [batch, output_length(n)] float32 in the container of `signals` unless `out` is given."""
+        signals, batch, n, spitch = FirFilter._rows(signals, "signals")
+        n_out = self.output_length(n)
+        if out is None:
+            if _is_device(signals):
+                import torch
+                out = torch.empty((batch, n_out), device=signals.device, dtype=torch.float32)
+            else:
+                out = np.empty((batch, n_out), np.float32)
+        elif not _is_device(out):
+            if not (isinstance(out, np.ndarray) and out.dtype == np.float32 and out.flags.c_contiguous):
+                raise ValueError("out: expected a C-contiguous float32 numpy array")
+        opitch = 0
+        if _is_device(out):
+            Stft._check_device_tensor(out, "float32", "out")
+            opitch = int(out.stride(0)) if batch > 1 else 0
+        if tuple(out.shape) != (batch, n_out):
+            raise ValueError(f"out: expected shape {(batch, n_out)}, got {tuple(out.shape)}")
+        dev = next((t for t in (out, signals) if _is_device(t)), None)
+        if dev is not None:
+            self._bind_torch_stream(dev)
+        got = _sz(0)
+        st = self.lib.vv_dsp_resample_poly_batch(self._r, _ptr(signals), DEVICE if _is_device(signals) else HOST, batch, n, spitch,
+                                                 _ptr(out), DEVICE if _is_device(out) else HOST, opitch, C.byref(got))
+        _check(self.lib, st, "vv_dsp_resample_poly_batch")
         return out
 
 

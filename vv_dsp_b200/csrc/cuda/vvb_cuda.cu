@@ -10,6 +10,7 @@
 #include "vvb_rt.cuh"
 #include "vvb_direct_kernels.cuh"
 #include "vvb_fir_kernels.cuh"
+#include "vvb_resample_kernels.cuh"
 
 #include <algorithm>
 #include <cmath>
@@ -56,6 +57,7 @@ static int emu_copy2d(void* d, size_t dp, const void* s, size_t sp, size_t w, si
 }
 extern "C" int vvb_memcpy2d_h2d(void* d, size_t dp, const void* s, size_t sp, size_t w, size_t h, void*) { return emu_copy2d(d, dp, s, sp, w, h); }
 extern "C" int vvb_memcpy2d_d2h(void* d, size_t dp, const void* s, size_t sp, size_t w, size_t h, void*) { return emu_copy2d(d, dp, s, sp, w, h); }
+extern "C" int vvb_memcpy2d_d2d(void* d, size_t dp, const void* s, size_t sp, size_t w, size_t h, void*) { return emu_copy2d(d, dp, s, sp, w, h); }
 extern "C" int vvb_memset(void* d, int v, size_t n, void*) { memset(d, v, n); return 0; }
 extern "C" int vvb_stream_create(void** s) { *s = malloc(1); return 0; }
 extern "C" int vvb_stream_destroy(void* s) { free(s); return 0; }
@@ -116,6 +118,10 @@ extern "C" int vvb_memcpy2d_h2d(void* d, size_t dp, const void* s, size_t sp, si
 extern "C" int vvb_memcpy2d_d2h(void* d, size_t dp, const void* s, size_t sp, size_t w, size_t h, void* st)
 {
     CK(cudaMemcpy2DAsync(d, dp, s, sp, w, h, cudaMemcpyDeviceToHost, (cudaStream_t)st)); return 0;
+}
+extern "C" int vvb_memcpy2d_d2d(void* d, size_t dp, const void* s, size_t sp, size_t w, size_t h, void* st)
+{
+    CK(cudaMemcpy2DAsync(d, dp, s, sp, w, h, cudaMemcpyDeviceToDevice, (cudaStream_t)st)); return 0;
 }
 extern "C" int vvb_memset(void* d, int v, size_t n, void* st) { CK(cudaMemsetAsync(d, v, n, (cudaStream_t)st)); return 0; }
 extern "C" int vvb_stream_create(void** s) { cudaStream_t st; CK(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking)); *s = st; return 0; }
@@ -870,6 +876,40 @@ extern "C" int vvb_fir_filter(vvb_fir_engine* e, const vvb_cpx* d_spec, size_t s
         if (int st = tu_fir((int)m, a, p > 0, e->fwd->sms, stream)) return st;
     }
     return 0;
+}
+
+/* ------------------------------------------------------------------ polyphase resampling */
+/* the largest shared-memory input span a launch stages; beyond it the kernel reads its inputs through L1 */
+#define VVB_RESAMPLE_SMEM_MAX ((size_t)200 << 10)
+
+extern "C" int vvb_resample_poly(const float* d_bank, size_t up, size_t down, size_t taps_per_phase, size_t half,
+                                 const float* d_x, size_t batch, size_t n, size_t x_pitch, float* d_y, size_t n_out,
+                                 size_t y_pitch, void* stream)
+{
+    if (!d_bank || !d_x || !d_y) return fail(1, "vvb_resample_poly", "null");
+    if (up == 0 || down == 0 || taps_per_phase == 0) return fail(2, "vvb_resample_poly", "ratio");
+    if (batch == 0 || n_out == 0) return 0;
+    ResampleArgs a;
+    a.x = d_x; a.x_pitch = (long long)x_pitch; a.n = (long long)n;
+    a.y = d_y; a.y_pitch = (long long)y_pitch; a.n_out = (long long)n_out;
+    a.bank = d_bank;
+    a.up = (long long)up; a.down = (long long)down; a.half = (long long)half;
+    a.half_mod = (long long)(half % up);
+    a.taps = (int)taps_per_phase;
+    {   /* down^-1 mod up by the extended Euclidean algorithm (gcd(up, down) == 1) */
+        long long r0 = a.up, r1 = a.down % a.up, t0 = 0, t1 = 1;
+        while (r1) { const long long qq = r0 / r1, r2 = r0 - qq * r1, t2 = t0 - qq * t1; r0 = r1; r1 = r2; t0 = t1; t1 = t2; }
+        if (r0 != 1 && up != 1) return fail(2, "vvb_resample_poly", "up and down are not coprime");
+        a.dinv = up == 1 ? 0 : ((t0 % a.up) + a.up) % a.up;
+    }
+    const long long band = (long long)RS_RUN * a.up;
+    const long long bands = (a.n_out + band - 1) / band;
+    a.tiles = (bands * a.up + RS_THREADS - 1) / RS_THREADS;
+    a.count = (long long)batch * a.tiles;
+    /* a tile's runs lie in at most (RS_THREADS - 1) / up + 2 bands, which read at most that times R down inputs plus T */
+    const double span = ((double)((RS_THREADS - 1) / a.up) + 2.0) * RS_RUN * (double)down + (double)taps_per_phase + 1.0;
+    a.span = span < 1e8 && resample_smem_bytes((long long)span) <= VVB_RESAMPLE_SMEM_MAX ? (int)span : 0;
+    return tu_resample(a, rt_num_sms(), stream);
 }
 
 /* ---------------------------------------------------------------------- Bluestein plumbing */

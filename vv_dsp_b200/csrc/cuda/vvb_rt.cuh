@@ -144,5 +144,7 @@ struct FirArgs;
 struct FirPadArgs;
 int tu_fir(int m, const FirArgs& a, bool accum, int sms, void* stream);    /* one overlap-save pass (vvb_fir_kernels.cuh) */
 int tu_fir_pad(const FirPadArgs& a, int sms, void* stream);
+struct ResampleArgs;
+int tu_resample(const ResampleArgs& a, int sms, void* stream);   /* polyphase resampling (vvb_resample_kernels.cuh) */
 
 }  // namespace vvb
