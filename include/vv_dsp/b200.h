@@ -320,6 +320,67 @@ VV_DSP_NODISCARD vv_dsp_status vv_dsp_resample_poly_batch(
     const vv_dsp_real* signals, vv_dsp_mem_space signals_space, size_t batch, size_t n, size_t signal_pitch,
     vv_dsp_real* out, vv_dsp_mem_space out_space, size_t out_pitch, size_t* out_len);
 
+/* ---------------------------------------------------------------------------------------------------------------
+ * Batched IIR filtering by a cascade of S second-order sections: scipy.signal.sosfilt / sosfiltfilt row by row.  Row s
+ * of sos[S][6] is (b0, b1, b2, 1, a1, a2); every section runs transposed direct form II in scipy's order,
+ *
+ *   y = b0 u + z0,   z0 <- b1 u - a1 y + z1,   z1 <- b2 u - a2 y,   (the input u of section s + 1 is y of section s)
+ *
+ * filter:   sosfilt(sos, x, zi=zi) row by row.  zi and zf have scipy's layout [S][batch][2] (row pitch 2, section
+ *           pitch 2 batch); zi == NULL is the zero state, zf == NULL does not write zf.  zf may be zi.
+ * filtfilt: sosfiltfilt(sos, x, padtype, padlen) row by row.  padtype is VV_DSP_PAD_NONE (padlen is then 0), _ODD,
+ *           _EVEN or _CONSTANT; padlen == (size_t)-1 is scipy's default 3 (2S + 1 - min(#{b2 == 0}, #{a2 == 0})).  The
+ *           forward pass runs over the padded signal from sosfilt_zi(sos) x_ext[0], the backward pass from
+ *           sosfilt_zi(sos) y_fwd[last], and the result is trimmed by padlen at both ends.  The padding is an index rule
+ *           of the kernel's loads; the forward pass writes n + 2 padlen floats per row to a device scratch of the handle.
+ *
+ * Arithmetic is float32 on the float32-rounded coefficients (sos is rounded once, at creation): exactly the filter
+ * scipy applies to float32 sos and x, but not the float64 arithmetic scipy uses when sos is float64.  The device runs the
+ * recurrence as a blocked scan: tiles of VV_DSP_SOS_TILE samples whose per-thread runs are joined by the constant maps
+ * A^k of each section (tables computed on the host in double; the join itself runs in float64).  Rows longer than the segment length (VV_DSP_SOS_SEGMENT
+ * samples unless the handle reports another, a multiple of the tile) are cut into segments that are joined through the
+ * cascade's state transition over one segment, so a few long rows still fill the device.  Output bits depend only on
+ * (sos, n, zi, x) of a row: not on the batch, the memory spaces or the staging chunks.
+ *
+ * Rejected filters: a section whose poles are not strictly inside the unit circle (|a2| < 1 and |a1| < 1 + a2 fails)
+ * is rejected with VV_DSP_ERROR_OUT_OF_RANGE.  scipy runs such a filter and diverges; the scan has no error bound for it.
+ *
+ * Pitches (in elements) of 0 mean dense.  Memory spaces as above: if every buffer is DEVICE the call only enqueues on
+ * the handle's stream, otherwise it returns once the results are in host memory.  `out` must not overlap `signals`; an
+ * identical base pointer is rejected with VV_DSP_ERROR_UNSUPPORTED.
+ *
+ * Status: NULL handle / signals / out / sos -> VV_DSP_ERROR_NULL_POINTER; S outside [1, 64], a pitch smaller than its
+ * row, or 0 < n <= padlen in filtfilt -> VV_DSP_ERROR_INVALID_SIZE; a coefficient that is not finite ->
+ * VV_DSP_ERROR_NAN_INF; a0 != 1, a pole on or outside the unit circle, a bad memory space or a bad padtype ->
+ * VV_DSP_ERROR_OUT_OF_RANGE; out == signals -> VV_DSP_ERROR_UNSUPPORTED; batch == 0 or n == 0 -> VV_DSP_OK with no
+ * filtering (filter then writes zf = zi, or zeros); CUDA failures -> VV_DSP_ERROR_INTERNAL (no usable device at
+ * creation: VV_DSP_ERROR_UNSUPPORTED).
+ * ------------------------------------------------------------------------------------------------------------- */
+#define VV_DSP_SOS_MAX_SECTIONS 64
+#define VV_DSP_SOS_TILE 4096                      /* samples per tile: 256 threads x 16 */
+#define VV_DSP_SOS_SEGMENT ((size_t)1 << 20)      /* samples per segment of a long row */
+enum { VV_DSP_PAD_NONE = 0, VV_DSP_PAD_ODD = 1, VV_DSP_PAD_EVEN = 2, VV_DSP_PAD_CONSTANT = 3 };
+typedef struct vv_dsp_sos vv_dsp_sos;
+VV_DSP_NODISCARD vv_dsp_status vv_dsp_sos_create(const vv_dsp_real* sos /* HOST [S][6] */, size_t n_sections,
+                                                 vv_dsp_sos** out);
+vv_dsp_status vv_dsp_sos_destroy(vv_dsp_sos* h);
+/* same rules as vv_dsp_stft_set_stream (NULL = the handle's own stream) */
+vv_dsp_status vv_dsp_sos_set_stream(vv_dsp_sos* h, void* cuda_stream);
+vv_dsp_status vv_dsp_sos_synchronize(vv_dsp_sos* h);
+/* S and the segment length in samples */
+vv_dsp_status vv_dsp_sos_get_config(const vv_dsp_sos* h, size_t* n_sections, size_t* segment_length);
+VV_DSP_NODISCARD vv_dsp_status vv_dsp_sos_filter_batch(
+    vv_dsp_sos* h,
+    const vv_dsp_real* signals, vv_dsp_mem_space signals_space, size_t batch, size_t n, size_t signal_pitch,
+    const vv_dsp_real* zi, vv_dsp_mem_space zi_space,     /* [S][batch][2] or NULL */
+    vv_dsp_real* zf, vv_dsp_mem_space zf_space,           /* [S][batch][2] or NULL */
+    vv_dsp_real* out, vv_dsp_mem_space out_space, size_t out_pitch);
+VV_DSP_NODISCARD vv_dsp_status vv_dsp_sos_filtfilt_batch(
+    vv_dsp_sos* h,
+    const vv_dsp_real* signals, vv_dsp_mem_space signals_space, size_t batch, size_t n, size_t signal_pitch,
+    int padtype, size_t padlen,
+    vv_dsp_real* out, vv_dsp_mem_space out_space, size_t out_pitch);
+
 /* Library / device introspection */
 const char* vv_dsp_b200_version(void);
 /* last CUDA error text seen by the calling thread ("" if none) */

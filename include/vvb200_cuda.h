@@ -151,6 +151,34 @@ int vvb_resample_poly(const float* d_bank, size_t up, size_t down, size_t taps_p
                       const float* d_x, size_t batch, size_t n, size_t x_pitch, float* d_y, size_t n_out, size_t y_pitch,
                       void* stream);
 
+/* ---- IIR second-order sections (csrc/host/sos.c).  A tile is VVB_IIR_THREADS runs of VVB_IIR_RUN samples.
+ * d_table [S][VVB_IIR_TABLE] (double): b0 b1 b2 a1 a2 0 0 0 (float32 values), then A^(RUN 2^d) row-major for d < VVB_IIR_LEVELS, A = [[-a1, 1],
+ * [-a2, 0]].  d_phi [2S][2S]: the cascade's state transition over one segment (state index 2 s + c).  The kernels run
+ * the cascade over the virtual rows v_b[j], 0 <= j < nv:
+ *   VVB_IIR_IN_PLAIN: x_b[j] (nv = n);  VVB_IIR_IN_EXT: x_b padded by `pad` samples at both ends by `padtype` (scipy's
+ *   odd_ext / even_ext / const_ext; nv = n + 2 pad);  VVB_IIR_IN_REV: x_b[nv - 1 - j] (x rows of nv samples).
+ * and store output j at y_b[j] (VVB_IIR_OUT_DIRECT) or at y_b[nv - 1 - j - pad] when that lies in [0, n)
+ * (VVB_IIR_OUT_REVTRIM).  The entering state of section s is zi[s zi_sstride + b zi_rstride + c] (0 when zi is NULL),
+ * times v_b[0] when zi_scale_first; the state after the last sample goes to zf[s zf_sstride + 2 b + c] unless zf is NULL.
+ * Rows longer than `segment` samples take three launches and need d_seg [batch][ceil(nv / segment)][2S] of scratch. */
+#define VVB_IIR_THREADS 256
+#define VVB_IIR_RUN 16
+#define VVB_IIR_LEVELS 8             /* log2(VVB_IIR_THREADS) */
+#define VVB_IIR_TABLE (8 + 4 * VVB_IIR_LEVELS)
+enum { VVB_IIR_IN_PLAIN = 0, VVB_IIR_IN_EXT = 1, VVB_IIR_IN_REV = 2 };
+enum { VVB_IIR_OUT_DIRECT = 0, VVB_IIR_OUT_REVTRIM = 1 };
+enum { VVB_IIR_PAD_ODD = 1, VVB_IIR_PAD_EVEN = 2, VVB_IIR_PAD_CONSTANT = 3 };   /* the values of VV_DSP_PAD_* */
+typedef struct {
+    const double* d_table; const float* d_phi; size_t sections, segment;
+    const float* x; size_t x_pitch, n; int in_mode, padtype; size_t pad, nv;
+    float* y; size_t y_pitch; int out_mode;
+    const float* zi; size_t zi_sstride, zi_rstride; int zi_scale_first;
+    float* zf; size_t zf_sstride;
+    float* d_seg;
+    size_t batch;
+} vvb_iir_call;
+int vvb_iir_sos(const vvb_iir_call* c, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

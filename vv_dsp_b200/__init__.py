@@ -8,9 +8,9 @@ follow the reference's ``vv_dsp_stft_*`` / ``vv_dsp_fft_*`` interface
 fails loudly when the CUDA library has not been built.
 """
 from .api import (  # noqa: F401
-    CONVENTIONS, KINDS, WINDOWS, FftPlan, FirFilter, Library, Resampler, Stft, StftStream, VvDspError, default_library,
+    CONVENTIONS, KINDS, WINDOWS, FftPlan, FirFilter, Library, Resampler, SosFilter, Stft, StftStream, VvDspError, default_library,
     fetch_frame, get_num_frames, overlap_add, window, mel_filterbank, log_mel_spectrogram, mfcc, MfccPlan, pcm_to_planar,
 )
 
-__all__ = ["Stft", "StftStream", "FftPlan", "FirFilter", "Resampler", "Library", "VvDspError", "default_library", "window", "get_num_frames",
+__all__ = ["Stft", "StftStream", "FftPlan", "FirFilter", "Resampler", "SosFilter", "Library", "VvDspError", "default_library", "window", "get_num_frames",
            "fetch_frame", "overlap_add", "WINDOWS", "CONVENTIONS", "KINDS"]

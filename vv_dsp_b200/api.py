@@ -122,6 +122,13 @@ class Library:
         "vv_dsp_resample_poly_get_config": (C.c_int, [_vp, C.POINTER(_sz), C.POINTER(_sz), C.POINTER(_sz), C.POINTER(_sz)]),
         "vv_dsp_resample_poly_output_length": (_sz, [_vp, _sz]),
         "vv_dsp_resample_poly_batch": (C.c_int, [_vp, _vp, C.c_int, _sz, _sz, _sz, _vp, C.c_int, _sz, C.POINTER(_sz)]),
+        "vv_dsp_sos_create": (C.c_int, [_vp, _sz, C.POINTER(_vp)]),
+        "vv_dsp_sos_destroy": (C.c_int, [_vp]),
+        "vv_dsp_sos_set_stream": (C.c_int, [_vp, _vp]),
+        "vv_dsp_sos_synchronize": (C.c_int, [_vp]),
+        "vv_dsp_sos_get_config": (C.c_int, [_vp, C.POINTER(_sz), C.POINTER(_sz)]),
+        "vv_dsp_sos_filter_batch": (C.c_int, [_vp, _vp, C.c_int, _sz, _sz, _sz, _vp, C.c_int, _vp, C.c_int, _vp, C.c_int, _sz]),
+        "vv_dsp_sos_filtfilt_batch": (C.c_int, [_vp, _vp, C.c_int, _sz, _sz, _sz, C.c_int, _sz, _vp, C.c_int, _sz]),
     }
     # entry points newer than round 1: absent from an old library variant loaded for an A/B measurement
     OPTIONAL = {"vv_dsp_b200_sm_clock_mhz", "vv_dsp_stft_shard_inverse", "vv_dsp_stft_device", "vv_dsp_stft_get_stream",
@@ -132,7 +139,9 @@ class Library:
                 "vv_dsp_fir_create", "vv_dsp_fir_destroy", "vv_dsp_fir_set_stream", "vv_dsp_fir_synchronize", "vv_dsp_fir_get_config",
                 "vv_dsp_fir_filter_batch", "vv_dsp_resample_poly_create", "vv_dsp_resample_poly_destroy",
                 "vv_dsp_resample_poly_set_stream", "vv_dsp_resample_poly_synchronize", "vv_dsp_resample_poly_get_config",
-                "vv_dsp_resample_poly_output_length", "vv_dsp_resample_poly_batch"}
+                "vv_dsp_resample_poly_output_length", "vv_dsp_resample_poly_batch", "vv_dsp_sos_create", "vv_dsp_sos_destroy",
+                "vv_dsp_sos_set_stream", "vv_dsp_sos_synchronize", "vv_dsp_sos_get_config", "vv_dsp_sos_filter_batch",
+                "vv_dsp_sos_filtfilt_batch"}
 
     def __init__(self, path: str | None = None):
         path = path or DEFAULT_LIB
@@ -898,6 +907,137 @@ class Resampler:
         st = self.lib.vv_dsp_resample_poly_batch(self._r, _ptr(signals), DEVICE if _is_device(signals) else HOST, batch, n, spitch,
                                                  _ptr(out), DEVICE if _is_device(out) else HOST, opitch, C.byref(got))
         _check(self.lib, st, "vv_dsp_resample_poly_batch")
+        return out
+
+
+# ----------------------------------------------------------------------------- IIR second-order sections
+PADTYPES = {None: 0, "none": 0, "odd": 1, "even": 2, "constant": 3}
+
+
+class SosFilter:
+    """vv_dsp_sos handle (include/vv_dsp/b200.h): batched IIR filtering by a cascade of second-order sections on the
+    device, scipy.signal.sosfilt / sosfiltfilt row by row.  sos: [S][6] rows (b0, b1, b2, 1, a1, a2), rounded to float32
+    once; every section must have its poles strictly inside the unit circle."""
+
+    def __init__(self, sos, lib: Library | None = None):
+        self.lib = lib or default_library()
+        self._h = _vp()
+        s = np.ascontiguousarray(np.asarray(sos, np.float32))
+        if s.ndim != 2 or s.shape[1] != 6:
+            raise ValueError("sos: expected an array of shape (n_sections, 6)")
+        _check(self.lib, self.lib.vv_dsp_sos_create(s.ctypes.data_as(_vp), s.shape[0], C.byref(self._h)), "vv_dsp_sos_create")
+        ns, seg = _sz(0), _sz(0)
+        _check(self.lib, self.lib.vv_dsp_sos_get_config(self._h, C.byref(ns), C.byref(seg)), "vv_dsp_sos_get_config")
+        self.n_sections, self.segment_length = int(ns.value), int(seg.value)
+        self._stream_pinned = False
+        self._bound_stream = None
+
+    def close(self):
+        if getattr(self, "_h", None) is not None and self._h.value:
+            self.lib.vv_dsp_sos_destroy(self._h)
+            self._h = _vp()
+
+    __del__ = close
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def set_stream(self, cuda_stream):
+        """Pin the handle to a stream (a cudaStream_t as an integer; 0 = the legacy default stream); None = its own
+        stream and back to automatic binding to torch's current stream (see Stft.set_stream)."""
+        self._stream_pinned = cuda_stream is not None
+        self._set_stream_raw(cuda_stream)
+
+    def _set_stream_raw(self, cuda_stream):
+        arg = None if cuda_stream is None else _vp(int(cuda_stream) or 1)
+        _check(self.lib, self.lib.vv_dsp_sos_set_stream(self._h, arg), "vv_dsp_sos_set_stream")
+        self._bound_stream = None if cuda_stream is None else (int(cuda_stream) or 1)
+
+    def _bind_torch_stream(self, tensor):
+        if self._stream_pinned:
+            return
+        import torch
+        cur = int(torch.cuda.current_stream(tensor.device).cuda_stream) or 1
+        if cur != self._bound_stream:
+            self._set_stream_raw(cur)
+
+    def synchronize(self):
+        _check(self.lib, self.lib.vv_dsp_sos_synchronize(self._h), "vv_dsp_sos_synchronize")
+
+    def _out(self, signals, batch, n, out):
+        """the output container ([batch, n] float32 like `signals` unless given) and its row pitch"""
+        if out is None:
+            if _is_device(signals):
+                import torch
+                out = torch.empty((batch, n), device=signals.device, dtype=torch.float32)
+            else:
+                out = np.empty((batch, n), np.float32)
+        elif not _is_device(out):
+            if not (isinstance(out, np.ndarray) and out.dtype == np.float32 and out.flags.c_contiguous):
+                raise ValueError("out: expected a C-contiguous float32 numpy array")
+        opitch = 0
+        if _is_device(out):
+            Stft._check_device_tensor(out, "float32", "out")
+            opitch = int(out.stride(0)) if batch > 1 else 0
+        if tuple(out.shape) != (batch, n):
+            raise ValueError(f"out: expected shape {(batch, n)}, got {tuple(out.shape)}")
+        return out, opitch
+
+    def _state(self, z, batch, what):
+        """a [S, batch, 2] float32 state in either space, dense"""
+        if _is_device(z):
+            Stft._check_device_tensor(z, "float32", what)
+            if not z.is_contiguous():
+                raise ValueError(f"{what}: expected a contiguous tensor")
+        else:
+            z = np.ascontiguousarray(z, np.float32)
+        if tuple(z.shape) != (self.n_sections, batch, 2):
+            raise ValueError(f"{what}: expected shape {(self.n_sections, batch, 2)}, got {tuple(z.shape)}")
+        return z
+
+    def filter(self, signals, zi=None, return_zf=False, out=None):
+        """scipy.signal.sosfilt(sos, signals, zi=zi) row by row.  signals: [batch, n] float32 (numpy, or a torch CUDA
+        tensor, views with a row pitch included); zi: [S, batch, 2] or None (zero state).  Returns the output in the
+        container of `signals` unless `out` is given, and (output, zf) when return_zf."""
+        signals, batch, n, spitch = FirFilter._rows(signals, "signals")
+        out, opitch = self._out(signals, batch, n, out)
+        if zi is not None:
+            zi = self._state(zi, batch, "zi")
+        zf = None
+        if return_zf:
+            if _is_device(signals):
+                import torch
+                zf = torch.empty((self.n_sections, batch, 2), device=signals.device, dtype=torch.float32)
+            else:
+                zf = np.empty((self.n_sections, batch, 2), np.float32)
+        dev = next((t for t in (out, signals, zi, zf) if t is not None and _is_device(t)), None)
+        if dev is not None:
+            self._bind_torch_stream(dev)
+        space = lambda t: DEVICE if t is not None and _is_device(t) else HOST      # noqa: E731
+        st = self.lib.vv_dsp_sos_filter_batch(self._h, _ptr(signals), space(signals), batch, n, spitch,
+                                              None if zi is None else _ptr(zi), space(zi),
+                                              None if zf is None else _ptr(zf), space(zf),
+                                              _ptr(out), space(out), opitch)
+        _check(self.lib, st, "vv_dsp_sos_filter_batch")
+        return (out, zf) if return_zf else out
+
+    def filtfilt(self, signals, padtype="odd", padlen=None, out=None):
+        """scipy.signal.sosfiltfilt(sos, signals, padtype=padtype, padlen=padlen) row by row; padlen=None is scipy's
+        default.  Returns the output in the container of `signals` unless `out` is given."""
+        if padtype not in PADTYPES:
+            raise ValueError(f"padtype: expected one of {sorted(k for k in PADTYPES if k)} or None")
+        signals, batch, n, spitch = FirFilter._rows(signals, "signals")
+        out, opitch = self._out(signals, batch, n, out)
+        dev = next((t for t in (out, signals) if _is_device(t)), None)
+        if dev is not None:
+            self._bind_torch_stream(dev)
+        st = self.lib.vv_dsp_sos_filtfilt_batch(self._h, _ptr(signals), DEVICE if _is_device(signals) else HOST, batch, n,
+                                                spitch, PADTYPES[padtype], (1 << 64) - 1 if padlen is None else int(padlen),
+                                                _ptr(out), DEVICE if _is_device(out) else HOST, opitch)
+        _check(self.lib, st, "vv_dsp_sos_filtfilt_batch")
         return out
 
 

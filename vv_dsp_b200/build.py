@@ -17,7 +17,7 @@ ROOT = os.path.dirname(PKG)
 INC = os.path.join(ROOT, "include")
 LIB = os.path.join(PKG, "lib", "libvvdsp_b200.so")
 OBJ = os.path.join(PKG, "lib", "obj")
-HOST_SRCS = [os.path.join(PKG, "csrc", "host", f) for f in ("window.c", "framing.c", "fft.c", "stft.c", "stream.c", "mel.c", "pcm.c", "fir.c", "resample.c")]
+HOST_SRCS = [os.path.join(PKG, "csrc", "host", f) for f in ("window.c", "framing.c", "fft.c", "stft.c", "stream.c", "mel.c", "pcm.c", "fir.c", "resample.c", "sos.c")]
 CUDA_DIR = os.path.join(PKG, "csrc", "cuda")
 # one kernel family per translation unit (vvb_tu_*.cu) + the C-ABI / runtime unit: compiled in parallel
 CUDA_SRCS = sorted(os.path.join(CUDA_DIR, f) for f in os.listdir(CUDA_DIR) if f.endswith(".cu"))

@@ -11,6 +11,7 @@
 #include "vvb_direct_kernels.cuh"
 #include "vvb_fir_kernels.cuh"
 #include "vvb_resample_kernels.cuh"
+#include "vvb_iir_kernels.cuh"
 
 #include <algorithm>
 #include <cmath>
@@ -910,6 +911,38 @@ extern "C" int vvb_resample_poly(const float* d_bank, size_t up, size_t down, si
     const double span = ((double)((RS_THREADS - 1) / a.up) + 2.0) * RS_RUN * (double)down + (double)taps_per_phase + 1.0;
     a.span = span < 1e8 && resample_smem_bytes((long long)span) <= VVB_RESAMPLE_SMEM_MAX ? (int)span : 0;
     return tu_resample(a, rt_num_sms(), stream);
+}
+
+/* ------------------------------------------------------------------ IIR second-order sections */
+extern "C" int vvb_iir_sos(const vvb_iir_call* c, void* stream)
+{
+    if (!c || !c->d_table || !c->x || !c->y) return fail(1, "vvb_iir_sos", "null");
+    if (c->sections == 0 || 2 * c->sections > (size_t)IIR_CHAIN_THREADS || c->segment == 0 ||
+        c->segment % ((size_t)IIR_THREADS * VVB_IIR_RUN) != 0)
+        return fail(2, "vvb_iir_sos", "sections / segment");
+    if (c->batch == 0 || c->nv == 0) return 0;
+    IirArgs a;
+    a.x = c->x; a.x_pitch = (long long)c->x_pitch; a.n = (long long)c->n;
+    a.in_mode = c->in_mode; a.padtype = c->padtype; a.pad = (long long)c->pad; a.nv = (long long)c->nv;
+    a.y = c->y; a.y_pitch = (long long)c->y_pitch; a.out_mode = c->out_mode;
+    a.table = c->d_table; a.sections = (int)c->sections; a.phi = c->d_phi;
+    a.zi = c->zi; a.zi_sstride = (long long)c->zi_sstride; a.zi_rstride = (long long)c->zi_rstride;
+    a.zi_scale_first = c->zi_scale_first;
+    a.zf = c->zf; a.zf_sstride = (long long)c->zf_sstride;
+    a.seg = c->d_seg;
+    a.segment = (long long)c->segment;
+    a.segs = (a.nv + a.segment - 1) / a.segment;
+    const long long batch = (long long)c->batch;
+    const int sms = rt_num_sms();
+    if (a.segs > 1) {
+        if (!c->d_seg || !c->d_phi) return fail(1, "vvb_iir_sos", "segment scratch");
+        a.count = batch * (a.segs - 1);               /* A: end states of every segment but the last, from zero */
+        if (int st = tu_iir('A', a, sms, stream)) return st;
+        a.count = batch;                              /* B: the true entering state of every segment */
+        if (int st = tu_iir('B', a, sms, stream)) return st;
+    }
+    a.count = batch * a.segs;                         /* C: every segment from its entering state */
+    return tu_iir('C', a, sms, stream);
 }
 
 /* ---------------------------------------------------------------------- Bluestein plumbing */

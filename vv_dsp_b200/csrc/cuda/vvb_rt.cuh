@@ -146,5 +146,7 @@ int tu_fir(int m, const FirArgs& a, bool accum, int sms, void* stream);    /* on
 int tu_fir_pad(const FirPadArgs& a, int sms, void* stream);
 struct ResampleArgs;
 int tu_resample(const ResampleArgs& a, int sms, void* stream);   /* polyphase resampling (vvb_resample_kernels.cuh) */
+struct IirArgs;
+int tu_iir(char pass, const IirArgs& a, int sms, void* stream);   /* IIR launch 'A', 'B' or 'C' (vvb_iir_kernels.cuh) */
 
 }  // namespace vvb
