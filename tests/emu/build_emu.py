@@ -6,9 +6,14 @@ The product package never loads this file.
 """
 import os
 import subprocess
+import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
+if ROOT not in sys.path:
+    sys.path.insert(0, ROOT)
+from vv_dsp_b200.build import HOST_DEPS, HOST_SRCS  # noqa: E402
+
 PKG = os.path.join(ROOT, "vv_dsp_b200")
 INC = os.path.join(ROOT, "include")
 LIB = os.path.join(HERE, "libvvdsp_b200_emu.so")
@@ -17,10 +22,10 @@ OBJ = os.path.join(HERE, "obj")
 
 def build(force=False):
     os.makedirs(OBJ, exist_ok=True)
-    host = [os.path.join(PKG, "csrc", "host", f) for f in ("window.c", "framing.c", "fft.c", "stft.c", "stream.c", "mel.c", "pcm.c")]
+    host = HOST_SRCS
     cudir = os.path.join(PKG, "csrc", "cuda")
     cus = sorted(os.path.join(cudir, f) for f in os.listdir(cudir) if f.endswith(".cu"))
-    deps = host + cus + [os.path.join(HERE, "cuda_emu.h")]
+    deps = host + HOST_DEPS + cus + [os.path.join(HERE, "cuda_emu.h")]
     for d, _, fs in list(os.walk(INC)) + list(os.walk(os.path.join(PKG, "csrc", "cuda"))):
         deps += [os.path.join(d, f) for f in fs]
     if not force and os.path.exists(LIB) and all(os.path.getmtime(d) <= os.path.getmtime(LIB) for d in deps):

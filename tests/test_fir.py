@@ -31,36 +31,12 @@ PLAN_EDGES = {29: (128, 1), 30: (256, 1), 52: (256, 1), 53: (512, 1), 94: (512, 
 FIR_C = 4e-8
 
 
-def build_fir_emu():
-    """The emulator library of tests/emu/build_emu.py plus the FIR host unit: build_emu.py compiles every kernel unit
-    (vvb_tu_fir.cu included) but only the host sources it lists, so csrc/host/fir.c is compiled here and linked with
-    build_emu's objects into a library of its own (tests/emu/libvvdsp_b200_fir_emu.so)."""
-    import glob
-    import subprocess
-    sys.path.insert(0, os.path.join(HERE, "emu"))
-    import build_emu
-    build_emu.build()
-    objs = sorted(glob.glob(os.path.join(build_emu.OBJ, "*.o")))
-    if not objs:                                      # a library left without its objects
-        build_emu.build(force=True)
-        objs = sorted(glob.glob(os.path.join(build_emu.OBJ, "*.o")))
-    src = os.path.join(build_emu.PKG, "csrc", "host", "fir.c")
-    obj_dir = os.path.join(HERE, "emu", "obj_fir")
-    obj = os.path.join(obj_dir, "fir.c.o")
-    lib = os.path.join(HERE, "emu", "libvvdsp_b200_fir_emu.so")
-    deps = [src, build_emu.LIB] + objs + glob.glob(os.path.join(build_emu.INC, "**", "*.h"), recursive=True)
-    if os.path.exists(lib) and all(os.path.getmtime(d) <= os.path.getmtime(lib) for d in deps):
-        return lib
-    os.makedirs(obj_dir, exist_ok=True)
-    subprocess.run(["gcc", "-std=c99", "-O1", "-fPIC", "-I" + build_emu.INC, "-c", src, "-o", obj], check=True)
-    subprocess.run(["g++", "-shared", "-o", lib, *objs, obj, "-lm"], check=True)
-    return lib
-
-
 @pytest.fixture(scope="module")
 def emu():
+    sys.path.insert(0, os.path.join(HERE, "emu"))
+    import build_emu
     from vv_dsp_b200 import Library
-    return Library(build_fir_emu())
+    return Library(build_emu.build())
 
 
 @pytest.fixture(scope="module")
@@ -281,6 +257,8 @@ def check_status_codes(lib):
         y[:] = 3.0
         assert call(*ok[:2], 1, *ok[3:6], 0, *ok[7:]) == 0 and np.all(y == 3.0)     # batch == 0
         assert call(*ok[:11], 0, 0) == 0 and np.all(y == 3.0)          # n_out == 0
+        with pytest.raises(ValueError):                                # a HOST out of another shape
+            f.filter(h, x, out=np.zeros((3, 101), np.float32))
 
 
 def check_plan_edges(lib):

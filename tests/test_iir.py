@@ -59,36 +59,12 @@ def sos32(name):
     return np.asarray(FILTERS[name], np.float32)
 
 
-def build_iir_emu():
-    """The emulator library of tests/emu/build_emu.py plus the IIR host unit: build_emu.py compiles every kernel unit
-    (vvb_tu_iir.cu included) but only the host sources it lists, so csrc/host/sos.c is compiled here and linked with
-    build_emu's objects into a library of its own (tests/emu/libvvdsp_b200_iir_emu.so)."""
-    import glob
-    import subprocess
-    sys.path.insert(0, os.path.join(HERE, "emu"))
-    import build_emu
-    build_emu.build()
-    objs = sorted(glob.glob(os.path.join(build_emu.OBJ, "*.o")))
-    if not objs:                                      # a library left without its objects
-        build_emu.build(force=True)
-        objs = sorted(glob.glob(os.path.join(build_emu.OBJ, "*.o")))
-    src = os.path.join(build_emu.PKG, "csrc", "host", "sos.c")
-    obj_dir = os.path.join(HERE, "emu", "obj_iir")
-    obj = os.path.join(obj_dir, "sos.c.o")
-    lib = os.path.join(HERE, "emu", "libvvdsp_b200_iir_emu.so")
-    deps = [src, build_emu.LIB] + objs + glob.glob(os.path.join(build_emu.INC, "**", "*.h"), recursive=True)
-    if os.path.exists(lib) and all(os.path.getmtime(d) <= os.path.getmtime(lib) for d in deps):
-        return lib
-    os.makedirs(obj_dir, exist_ok=True)
-    subprocess.run(["gcc", "-std=c99", "-O1", "-fPIC", "-I" + build_emu.INC, "-c", src, "-o", obj], check=True)
-    subprocess.run(["g++", "-shared", "-o", lib, *objs, obj, "-lm"], check=True)
-    return lib
-
-
 @pytest.fixture(scope="module")
 def emu():
+    sys.path.insert(0, os.path.join(HERE, "emu"))
+    import build_emu
     from vv_dsp_b200 import Library
-    return Library(build_iir_emu())
+    return Library(build_emu.build())
 
 
 @pytest.fixture(scope="module")

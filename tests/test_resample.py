@@ -29,36 +29,12 @@ ROWS = {(1, 3): (1, 3, 61, 61, True), (3, 1): (3, 1, 61, 21, True), (160, 441): 
         (2560, 147): (2560, 147, 51201, 21, True), (1, 24): (1, 24, 481, 481, False)}
 
 
-def build_resample_emu():
-    """The emulator library of tests/emu/build_emu.py plus the resampling host unit: build_emu.py compiles every kernel
-    unit (vvb_tu_resample.cu included) but only the host sources it lists, so csrc/host/resample.c is compiled here and
-    linked with build_emu's objects into a library of its own (tests/emu/libvvdsp_b200_resample_emu.so)."""
-    import glob
-    import subprocess
-    sys.path.insert(0, os.path.join(HERE, "emu"))
-    import build_emu
-    build_emu.build()
-    objs = sorted(glob.glob(os.path.join(build_emu.OBJ, "*.o")))
-    if not objs:                                      # a library left without its objects
-        build_emu.build(force=True)
-        objs = sorted(glob.glob(os.path.join(build_emu.OBJ, "*.o")))
-    src = os.path.join(build_emu.PKG, "csrc", "host", "resample.c")
-    obj_dir = os.path.join(HERE, "emu", "obj_resample")
-    obj = os.path.join(obj_dir, "resample.c.o")
-    lib = os.path.join(HERE, "emu", "libvvdsp_b200_resample_emu.so")
-    deps = [src, build_emu.LIB] + objs + glob.glob(os.path.join(build_emu.INC, "**", "*.h"), recursive=True)
-    if os.path.exists(lib) and all(os.path.getmtime(d) <= os.path.getmtime(lib) for d in deps):
-        return lib
-    os.makedirs(obj_dir, exist_ok=True)
-    subprocess.run(["gcc", "-std=c99", "-O1", "-fPIC", "-I" + build_emu.INC, "-c", src, "-o", obj], check=True)
-    subprocess.run(["g++", "-shared", "-o", lib, *objs, obj, "-lm"], check=True)
-    return lib
-
-
 @pytest.fixture(scope="module")
 def emu():
+    sys.path.insert(0, os.path.join(HERE, "emu"))
+    import build_emu
     from vv_dsp_b200 import Library
-    return Library(build_resample_emu())
+    return Library(build_emu.build())
 
 
 @pytest.fixture(scope="module")

@@ -215,6 +215,54 @@ def _ptr(a):
     return a.ctypes.data_as(_vp)
 
 
+def _space(t):
+    return DEVICE if _is_device(t) else HOST
+
+
+def _check_device_tensor(t, dtype_name, what):
+    """device tensors are handed to the C API as raw pointers: the layout has to be what it expects"""
+    import torch
+    want = {"float32": torch.float32, "complex64": torch.complex64}[dtype_name]
+    if t.dtype != want:
+        raise TypeError(f"{what}: expected a {dtype_name} CUDA tensor, got {t.dtype}")
+    if t.stride(-1) != 1:
+        raise ValueError(f"{what}: the innermost dimension must be contiguous (stride {t.stride(-1)})")
+
+
+def _rows(a, what):
+    """(container, rows, row length, row pitch in elements); device tensors keep their layout (odd pitches of views
+    included), host arrays are made dense float32"""
+    if _is_device(a):
+        _check_device_tensor(a, "float32", what)
+        if a.ndim != 2:
+            raise ValueError(f"{what}: expected a 2-D tensor")
+        return a, int(a.shape[0]), int(a.shape[1]), (int(a.stride(0)) if a.shape[0] > 1 else 0)
+    a = np.ascontiguousarray(a, np.float32)
+    if a.ndim != 2:
+        raise ValueError(f"{what}: expected a 2-D array")
+    return a, int(a.shape[0]), int(a.shape[1]), 0
+
+
+def _out_rows(out, like, batch, n):
+    """the output container ([batch, n] float32 in the container of `like` unless given) and its row pitch"""
+    if out is None:
+        if _is_device(like):
+            import torch
+            out = torch.empty((batch, n), device=like.device, dtype=torch.float32)
+        else:
+            out = np.empty((batch, n), np.float32)
+    elif not _is_device(out):
+        if not (isinstance(out, np.ndarray) and out.dtype == np.float32 and out.flags.c_contiguous):
+            raise ValueError("out: expected a C-contiguous float32 numpy array")
+    opitch = 0
+    if _is_device(out):
+        _check_device_tensor(out, "float32", "out")
+        opitch = int(out.stride(0)) if batch > 1 else 0
+    if tuple(out.shape) != (batch, n):
+        raise ValueError(f"out: expected shape {(batch, n)}, got {tuple(out.shape)}")
+    return out, opitch
+
+
 def _win_id(w):
     return WINDOWS[w] if isinstance(w, str) else int(w)
 
@@ -291,7 +339,7 @@ def pcm_to_planar(raw, fmt, channels, out=None, stream=0, lib: Library | None = 
             out = np.empty((channels, n), np.float32)
     pitch = int(out.stride(0)) if _is_device(out) else n
     st = lib.vv_dsp_b200_pcm_to_planar(_ptr(raw), DEVICE if dev_in else HOST, fmt, n, channels, _ptr(out),
-                                       DEVICE if _is_device(out) else HOST, pitch, stream)
+                                       _space(out), pitch, stream)
     _check(lib, st, "vv_dsp_b200_pcm_to_planar")
     return out
 
@@ -337,24 +385,26 @@ class MfccPlan:
         self.close()
 
 
-# ----------------------------------------------------------------------------- STFT handle
-class Stft:
-    """vv_dsp_stft handle: create / process / reconstruct / spectrogram + the batched extension."""
+# ----------------------------------------------------------------------------- stream-bound handles
+class _StreamHandle:
+    """A handle of include/vv_dsp/b200.h that enqueues its device work on one CUDA stream: vv_dsp_<_prefix>_destroy,
+    _set_stream and _synchronize, and the binding to torch's current stream."""
 
-    def __init__(self, fft_size, hop_size, window="hann", lib: Library | None = None):
+    _prefix = ""
+
+    def __init__(self, lib: Library | None):
         self.lib = lib or default_library()
-        self.nfft, self.hop = int(fft_size), int(hop_size)
-        self.bins = self.nfft // 2 + 1
         self._h = _vp()
-        p = StftParams(self.nfft, self.hop, _win_id(window))
-        st = self.lib.vv_dsp_stft_create(C.byref(p), C.byref(self._h))
-        _check(self.lib, st, "vv_dsp_stft_create")
         self._stream_pinned = False      # set_stream() called by the user: never rebind behind their back
         self._bound_stream = None        # what the handle is bound to right now (None = its own stream)
 
+    def _call(self, what, *args):
+        name = f"vv_dsp_{self._prefix}_{what}"
+        _check(self.lib, getattr(self.lib, name)(self._h, *args), name)
+
     def close(self):
         if getattr(self, "_h", None) is not None and self._h.value:
-            self.lib.vv_dsp_stft_destroy(self._h)
+            getattr(self.lib, f"vv_dsp_{self._prefix}_destroy")(self._h)
             self._h = _vp()
 
     __del__ = close
@@ -364,6 +414,54 @@ class Stft:
 
     def __exit__(self, *exc):
         self.close()
+
+    def set_stream(self, cuda_stream):
+        """Pin the handle to a stream.  cuda_stream: a cudaStream_t as an integer.  None = the handle's own stream
+        (and back to automatic binding, see _bind_torch_stream); 0 (the legacy default stream, what torch reports
+        for its default stream) is passed as cudaStreamLegacy (0x1), because the C API reserves NULL for "the
+        handle's own stream"."""
+        self._stream_pinned = cuda_stream is not None
+        self._set_stream_raw(cuda_stream)
+
+    def _set_stream_raw(self, cuda_stream):
+        self._call("set_stream", None if cuda_stream is None else _vp(int(cuda_stream) or 1))
+        self._bound_stream = None if cuda_stream is None else (int(cuda_stream) or 1)
+
+    def _bind_torch_stream(self, tensor):
+        """Stream contract of the device path: calls whose buffers are torch CUDA tensors are enqueued on torch's
+        CURRENT stream of that device (like any torch op), so they are ordered after the ops that produced the
+        inputs and before the ops that consume the outputs -- unless the user pinned a stream with set_stream(),
+        in which case ordering against torch's streams is theirs to establish."""
+        if self._stream_pinned:
+            return
+        import torch
+        cur = int(torch.cuda.current_stream(tensor.device).cuda_stream) or 1
+        if cur != self._bound_stream:
+            self._set_stream_raw(cur)
+
+    def _bind(self, *tensors):
+        """_bind_torch_stream to the first device tensor among `tensors` (None entries allowed), if there is one"""
+        dev = next((t for t in tensors if _is_device(t)), None)
+        if dev is not None:
+            self._bind_torch_stream(dev)
+
+    def synchronize(self):
+        self._call("synchronize")
+
+
+# ----------------------------------------------------------------------------- STFT handle
+class Stft(_StreamHandle):
+    """vv_dsp_stft handle: create / process / reconstruct / spectrogram + the batched extension."""
+
+    _prefix = "stft"
+
+    def __init__(self, fft_size, hop_size, window="hann", lib: Library | None = None):
+        super().__init__(lib)
+        self.nfft, self.hop = int(fft_size), int(hop_size)
+        self.bins = self.nfft // 2 + 1
+        p = StftParams(self.nfft, self.hop, _win_id(window))
+        st = self.lib.vv_dsp_stft_create(C.byref(p), C.byref(self._h))
+        _check(self.lib, st, "vv_dsp_stft_create")
 
     # --- reference per-frame API
     def process(self, frame):
@@ -394,47 +492,6 @@ class Stft:
     def num_frames(self, n, convention="valid") -> int:
         return int(self.lib.vv_dsp_stft_num_frames(self._h, n, CONVENTIONS[convention]))
 
-    def set_stream(self, cuda_stream):
-        """Pin the handle to a stream.  cuda_stream: a cudaStream_t as an integer.  None = the handle's own stream
-        (and back to automatic binding, see _bind_torch_stream); 0 (the legacy default stream, what torch reports
-        for its default stream) is passed as cudaStreamLegacy (0x1), because the C API reserves NULL for "the
-        handle's own stream"."""
-        self._stream_pinned = cuda_stream is not None
-        self._set_stream_raw(cuda_stream)
-
-    def _set_stream_raw(self, cuda_stream):
-        if cuda_stream is None:
-            arg = None
-        else:
-            arg = _vp(int(cuda_stream) or 1)
-        _check(self.lib, self.lib.vv_dsp_stft_set_stream(self._h, arg), "vv_dsp_stft_set_stream")
-        self._bound_stream = None if cuda_stream is None else (int(cuda_stream) or 1)
-
-    def _bind_torch_stream(self, tensor):
-        """Stream contract of the device path: calls whose buffers are torch CUDA tensors are enqueued on torch's
-        CURRENT stream of that device (like any torch op), so they are ordered after the ops that produced the
-        inputs and before the ops that consume the outputs -- unless the user pinned a stream with set_stream(),
-        in which case ordering against torch's streams is theirs to establish."""
-        if self._stream_pinned:
-            return
-        import torch
-        cur = int(torch.cuda.current_stream(tensor.device).cuda_stream) or 1
-        if cur != self._bound_stream:
-            self._set_stream_raw(cur)
-
-    @staticmethod
-    def _check_device_tensor(t, dtype_name, what):
-        """device tensors are handed to the C API as raw pointers: the layout has to be what it expects"""
-        import torch
-        want = {"float32": torch.float32, "complex64": torch.complex64}[dtype_name]
-        if t.dtype != want:
-            raise TypeError(f"{what}: expected a {dtype_name} CUDA tensor, got {t.dtype}")
-        if t.stride(-1) != 1:
-            raise ValueError(f"{what}: the innermost dimension must be contiguous (stride {t.stride(-1)})")
-
-    def synchronize(self):
-        _check(self.lib, self.lib.vv_dsp_stft_synchronize(self._h), "vv_dsp_stft_synchronize")
-
     def set_async(self, enable=True):
         """stream-ordered mode for HOST-buffer calls (see include/vv_dsp/b200.h); finish with synchronize()"""
         _check(self.lib, self.lib.vv_dsp_stft_set_async(self._h, int(bool(enable))), "vv_dsp_stft_set_async")
@@ -458,18 +515,16 @@ class Stft:
                 out = np.empty((batch, frames, self.bins), np.complex64 if kind == "complex" else np.float32)
         spec_pitch = 0
         if dev_in:
-            self._check_device_tensor(signals, "float32", "signals")
+            _check_device_tensor(signals, "float32", "signals")
         if _is_device(out):
-            self._check_device_tensor(out, "complex64" if kind == "complex" else "float32", "out")
+            _check_device_tensor(out, "complex64" if kind == "complex" else "float32", "out")
             assert tuple(out.shape) == (batch, frames, self.bins), (tuple(out.shape), (batch, frames, self.bins))
             spec_pitch = self._spec_pitch(out)
-            self._bind_torch_stream(out)
-        elif dev_in:
-            self._bind_torch_stream(signals)
+        self._bind(out, signals)
         nf = _sz(0)
         st = self.lib.vv_dsp_stft_batch_forward(self._h, _ptr(signals), DEVICE if dev_in else HOST, batch, n, pitch,
                                                 CONVENTIONS[convention], KINDS[kind], _ptr(out),
-                                                DEVICE if _is_device(out) else HOST, spec_pitch, C.byref(nf))
+                                                _space(out), spec_pitch, C.byref(nf))
         _check(self.lib, st, "vv_dsp_stft_batch_forward")
         assert nf.value == frames
         return out
@@ -486,13 +541,13 @@ class Stft:
             out = np.empty((batch, frames, self.bins), np.complex64 if kind == "complex" else np.float32)
         spec_pitch = 0
         if _is_device(out):
-            self._check_device_tensor(out, "complex64" if kind == "complex" else "float32", "out")
+            _check_device_tensor(out, "complex64" if kind == "complex" else "float32", "out")
             assert tuple(out.shape) == (batch, frames, self.bins)
             spec_pitch = self._spec_pitch(out)
             self._bind_torch_stream(out)
         nf = _sz(0)
         st = self.lib.vv_dsp_stft_batch_forward_pcm(self._h, _ptr(pcm), fmt, batch, n, n, CONVENTIONS[convention], KINDS[kind],
-                                                    _ptr(out), DEVICE if _is_device(out) else HOST, spec_pitch, C.byref(nf))
+                                                    _ptr(out), _space(out), spec_pitch, C.byref(nf))
         _check(self.lib, st, "vv_dsp_stft_batch_forward_pcm")
         assert nf.value == frames
         return out
@@ -500,14 +555,12 @@ class Stft:
     def _prepare_device_args(self, signals, out):
         """dtype / layout checks and stream binding of the feature chains (dense float32 output)"""
         if _is_device(signals):
-            self._check_device_tensor(signals, "float32", "signals")
+            _check_device_tensor(signals, "float32", "signals")
         if _is_device(out):
-            self._check_device_tensor(out, "float32", "out")
+            _check_device_tensor(out, "float32", "out")
             if not out.is_contiguous():
                 raise ValueError("out: must be contiguous")
-            self._bind_torch_stream(out)
-        elif _is_device(signals):
-            self._bind_torch_stream(signals)
+        self._bind(out, signals)
 
     def _spec_pitch(self, t):
         """row pitch (elements) of a [batch, frames, bins] device tensor whose rows follow each other at one pitch;
@@ -539,7 +592,7 @@ class Stft:
         nf = _sz(0)
         st = self.lib.vv_dsp_stft_batch_logmel(self._h, _ptr(signals), DEVICE if dev_in else HOST, batch, n, pitch,
                                                CONVENTIONS[convention], _ptr(weights), weights.shape[0], log_epsilon,
-                                               _ptr(out), DEVICE if _is_device(out) else HOST, C.byref(nf))
+                                               _ptr(out), _space(out), C.byref(nf))
         _check(self.lib, st, "vv_dsp_stft_batch_logmel")
         return out
 
@@ -555,11 +608,11 @@ class Stft:
         if out is None:
             out = np.empty((batch, frames, weights.shape[0]), np.float32)
         if _is_device(out):
-            self._check_device_tensor(out, "float32", "out")
+            _check_device_tensor(out, "float32", "out")
             self._bind_torch_stream(out)
         nf = _sz(0)
         st = self.lib.vv_dsp_stft_batch_logmel_pcm(self._h, _ptr(pcm), fmt, batch, n, n, CONVENTIONS[convention], _ptr(weights),
-                                                   weights.shape[0], log_epsilon, _ptr(out), DEVICE if _is_device(out) else HOST, C.byref(nf))
+                                                   weights.shape[0], log_epsilon, _ptr(out), _space(out), C.byref(nf))
         _check(self.lib, st, "vv_dsp_stft_batch_logmel_pcm")
         return out
 
@@ -583,7 +636,7 @@ class Stft:
         nf = _sz(0)
         st = self.lib.vv_dsp_stft_batch_mfcc(self._h, _ptr(signals), DEVICE if dev_in else HOST, batch, n, pitch,
                                              CONVENTIONS[convention], _ptr(weights), weights.shape[0], log_epsilon,
-                                             num_coeffs, lifter, _ptr(out), DEVICE if _is_device(out) else HOST, C.byref(nf))
+                                             num_coeffs, lifter, _ptr(out), _space(out), C.byref(nf))
         _check(self.lib, st, "vv_dsp_stft_batch_mfcc")
         return out
 
@@ -603,17 +656,15 @@ class Stft:
         keep = spectra if frames else None
         spec_pitch = out_pitch = 0
         if dev_in:
-            self._check_device_tensor(spectra, "complex64", "spectra")
+            _check_device_tensor(spectra, "complex64", "spectra")
             spec_pitch = self._spec_pitch(spectra)
         if _is_device(out):
-            self._check_device_tensor(out, "float32", "out")
+            _check_device_tensor(out, "float32", "out")
             assert out.ndim == 2 and int(out.shape[0]) == batch and int(out.shape[1]) == n_out
             out_pitch = int(out.stride(0)) if batch > 1 else 0
-            self._bind_torch_stream(out)
-        elif dev_in:
-            self._bind_torch_stream(spectra)
+        self._bind(out, spectra)
         st = self.lib.vv_dsp_stft_batch_inverse(self._h, _ptr(keep), DEVICE if dev_in else HOST, batch, frames, spec_pitch,
-                                                _ptr(out), DEVICE if _is_device(out) else HOST, n_out, out_pitch, int(normalise))
+                                                _ptr(out), _space(out), n_out, out_pitch, int(normalise))
         _check(self.lib, st, "vv_dsp_stft_batch_inverse")
         return out
 
@@ -621,11 +672,11 @@ class Stft:
         """Synthesis of one frame-range shard of a longer stream (include/vv_dsp/b200.h): spectra = CUDA tensor
         [halo_frames + own frames, bins], out = CUDA tensor [n_out] (the shard's owned samples)."""
         import torch
-        self._check_device_tensor(spectra, "complex64", "spectra")
+        _check_device_tensor(spectra, "complex64", "spectra")
         assert spectra.ndim == 2 and spectra.shape[1] == self.bins and spectra.is_contiguous()
         if out is None:
             out = torch.empty(n_out, device=spectra.device, dtype=torch.float32)
-        self._check_device_tensor(out, "float32", "out")
+        _check_device_tensor(out, "float32", "out")
         self._bind_torch_stream(out)
         st = self.lib.vv_dsp_stft_shard_inverse(self._h, _ptr(spectra), int(spectra.shape[0]), int(halo_frames), int(bool(is_first)),
                                                 int(bool(is_last)), _ptr(out), int(n_out))
@@ -725,187 +776,70 @@ class StftStream:
 
 
 # ----------------------------------------------------------------------------- FIR filtering
-class FirFilter:
+class FirFilter(_StreamHandle):
     """vv_dsp_fir handle (include/vv_dsp/b200.h): batched FIR filtering by FFT convolution on the device.
     out[b][i] = sum_j h_b[j] x_b[i - j] for i < n_out; n_out = n is lfilter(h, 1, x), n + num_taps - 1 the full convolution."""
 
+    _prefix = "fir"
+    _f = property(lambda self: self._h)        # the handle's name before the handles shared a base class
+
     def __init__(self, num_taps, lib: Library | None = None):
-        self.lib = lib or default_library()
+        super().__init__(lib)
         self.num_taps = int(num_taps)
-        self._f = _vp()
-        _check(self.lib, self.lib.vv_dsp_fir_create(self.num_taps, C.byref(self._f)), "vv_dsp_fir_create")
+        _check(self.lib, self.lib.vv_dsp_fir_create(self.num_taps, C.byref(self._h)), "vv_dsp_fir_create")
         n, p = _sz(0), _sz(0)
-        _check(self.lib, self.lib.vv_dsp_fir_get_config(self._f, C.byref(n), C.byref(p)), "vv_dsp_fir_get_config")
+        _check(self.lib, self.lib.vv_dsp_fir_get_config(self._h, C.byref(n), C.byref(p)), "vv_dsp_fir_get_config")
         self.fft_size, self.partitions = int(n.value), int(p.value)
-        self._stream_pinned = False
-        self._bound_stream = None
-
-    def close(self):
-        if getattr(self, "_f", None) is not None and self._f.value:
-            self.lib.vv_dsp_fir_destroy(self._f)
-            self._f = _vp()
-
-    __del__ = close
-
-    def __enter__(self):
-        return self
-
-    def __exit__(self, *exc):
-        self.close()
-
-    def set_stream(self, cuda_stream):
-        """Pin the handle to a stream (a cudaStream_t as an integer; 0 = the legacy default stream); None = its own
-        stream and back to automatic binding to torch's current stream (see Stft.set_stream)."""
-        self._stream_pinned = cuda_stream is not None
-        self._set_stream_raw(cuda_stream)
-
-    def _set_stream_raw(self, cuda_stream):
-        arg = None if cuda_stream is None else _vp(int(cuda_stream) or 1)
-        _check(self.lib, self.lib.vv_dsp_fir_set_stream(self._f, arg), "vv_dsp_fir_set_stream")
-        self._bound_stream = None if cuda_stream is None else (int(cuda_stream) or 1)
-
-    def _bind_torch_stream(self, tensor):
-        """device calls are enqueued on torch's current stream of the tensor's device, as Stft._bind_torch_stream does"""
-        if self._stream_pinned:
-            return
-        import torch
-        cur = int(torch.cuda.current_stream(tensor.device).cuda_stream) or 1
-        if cur != self._bound_stream:
-            self._set_stream_raw(cur)
-
-    def synchronize(self):
-        _check(self.lib, self.lib.vv_dsp_fir_synchronize(self._f), "vv_dsp_fir_synchronize")
-
-    @staticmethod
-    def _rows(a, what):
-        """(container, rows, row length, row pitch in elements); device tensors keep their layout (odd pitches of views
-        included), host arrays are made dense float32"""
-        if _is_device(a):
-            Stft._check_device_tensor(a, "float32", what)
-            if a.ndim != 2:
-                raise ValueError(f"{what}: expected a 2-D tensor")
-            return a, int(a.shape[0]), int(a.shape[1]), (int(a.stride(0)) if a.shape[0] > 1 else 0)
-        a = np.ascontiguousarray(a, np.float32)
-        if a.ndim != 2:
-            raise ValueError(f"{what}: expected a 2-D array")
-        return a, int(a.shape[0]), int(a.shape[1]), 0
 
     def filter(self, filters, signals, n_out=None, out=None):
         """filters: [1 or batch, num_taps], signals: [batch, n] float32 (numpy, or torch CUDA tensors).  Returns
         [batch, n_out] float32 (default n_out = n) in the container of `signals` unless `out` is given."""
-        filters, nf, taps, fpitch = self._rows(filters, "filters")
-        signals, batch, n, spitch = self._rows(signals, "signals")
+        filters, nf, taps, fpitch = _rows(filters, "filters")
+        signals, batch, n, spitch = _rows(signals, "signals")
         if taps != self.num_taps:
             raise ValueError(f"filters: rows of {taps} taps, the handle was created for {self.num_taps}")
         n_out = n if n_out is None else int(n_out)
-        if out is None:
-            if _is_device(signals):
-                import torch
-                out = torch.empty((batch, n_out), device=signals.device, dtype=torch.float32)
-            else:
-                out = np.empty((batch, n_out), np.float32)
-        elif not _is_device(out):
-            assert out.dtype == np.float32 and out.flags.c_contiguous
-        opitch = 0
-        if _is_device(out):
-            Stft._check_device_tensor(out, "float32", "out")
-            assert out.ndim == 2 and int(out.shape[0]) == batch and int(out.shape[1]) == n_out
-            opitch = int(out.stride(0)) if batch > 1 else 0
-        dev = next((t for t in (out, signals, filters) if _is_device(t)), None)
-        if dev is not None:
-            self._bind_torch_stream(dev)
-        st = self.lib.vv_dsp_fir_filter_batch(self._f, _ptr(filters), DEVICE if _is_device(filters) else HOST, nf, fpitch,
-                                              _ptr(signals), DEVICE if _is_device(signals) else HOST, batch, n, spitch,
-                                              _ptr(out), DEVICE if _is_device(out) else HOST, n_out, opitch)
+        out, opitch = _out_rows(out, signals, batch, n_out)
+        self._bind(out, signals, filters)
+        st = self.lib.vv_dsp_fir_filter_batch(self._h, _ptr(filters), _space(filters), nf, fpitch, _ptr(signals), _space(signals),
+                                              batch, n, spitch, _ptr(out), _space(out), n_out, opitch)
         _check(self.lib, st, "vv_dsp_fir_filter_batch")
         return out
 
 
 # ----------------------------------------------------------------------------- resampling
-class Resampler:
+class Resampler(_StreamHandle):
     """vv_dsp_resample_poly handle (include/vv_dsp/b200.h): batched rational-ratio resampling by a polyphase FIR on the
     device, scipy.signal.resample_poly(x, up, down, window=taps, padtype='constant') row by row.  taps=None designs scipy's
     default Kaiser (beta 5) filter; up / down are reduced by their gcd."""
 
+    _prefix = "resample_poly"
+    _r = property(lambda self: self._h)        # the handle's name before the handles shared a base class
+
     def __init__(self, up, down, taps=None, lib: Library | None = None):
-        self.lib = lib or default_library()
-        self._r = _vp()
+        super().__init__(lib)
         t = None if taps is None else np.ascontiguousarray(np.asarray(taps, np.float32).ravel())
         st = self.lib.vv_dsp_resample_poly_create(int(up), int(down), None if t is None else t.ctypes.data_as(_vp),
-                                                  0 if t is None else t.size, C.byref(self._r))
+                                                  0 if t is None else t.size, C.byref(self._h))
         _check(self.lib, st, "vv_dsp_resample_poly_create")
         u, d, k, tp = _sz(0), _sz(0), _sz(0), _sz(0)
-        _check(self.lib, self.lib.vv_dsp_resample_poly_get_config(self._r, C.byref(u), C.byref(d), C.byref(k), C.byref(tp)),
+        _check(self.lib, self.lib.vv_dsp_resample_poly_get_config(self._h, C.byref(u), C.byref(d), C.byref(k), C.byref(tp)),
                "vv_dsp_resample_poly_get_config")
         self.up, self.down, self.num_taps, self.taps_per_phase = int(u.value), int(d.value), int(k.value), int(tp.value)
-        self._stream_pinned = False
-        self._bound_stream = None
-
-    def close(self):
-        if getattr(self, "_r", None) is not None and self._r.value:
-            self.lib.vv_dsp_resample_poly_destroy(self._r)
-            self._r = _vp()
-
-    __del__ = close
-
-    def __enter__(self):
-        return self
-
-    def __exit__(self, *exc):
-        self.close()
 
     def output_length(self, n) -> int:
         """ceil(n up / down)"""
-        return int(self.lib.vv_dsp_resample_poly_output_length(self._r, int(n)))
-
-    def set_stream(self, cuda_stream):
-        """Pin the handle to a stream (a cudaStream_t as an integer; 0 = the legacy default stream); None = its own
-        stream and back to automatic binding to torch's current stream (see Stft.set_stream)."""
-        self._stream_pinned = cuda_stream is not None
-        self._set_stream_raw(cuda_stream)
-
-    def _set_stream_raw(self, cuda_stream):
-        arg = None if cuda_stream is None else _vp(int(cuda_stream) or 1)
-        _check(self.lib, self.lib.vv_dsp_resample_poly_set_stream(self._r, arg), "vv_dsp_resample_poly_set_stream")
-        self._bound_stream = None if cuda_stream is None else (int(cuda_stream) or 1)
-
-    def _bind_torch_stream(self, tensor):
-        if self._stream_pinned:
-            return
-        import torch
-        cur = int(torch.cuda.current_stream(tensor.device).cuda_stream) or 1
-        if cur != self._bound_stream:
-            self._set_stream_raw(cur)
-
-    def synchronize(self):
-        _check(self.lib, self.lib.vv_dsp_resample_poly_synchronize(self._r), "vv_dsp_resample_poly_synchronize")
+        return int(self.lib.vv_dsp_resample_poly_output_length(self._h, int(n)))
 
     def resample(self, signals, out=None):
         """signals: [batch, n] float32 (numpy, or a torch CUDA tensor, views with a row pitch included).  Returns
         [batch, output_length(n)] float32 in the container of `signals` unless `out` is given."""
-        signals, batch, n, spitch = FirFilter._rows(signals, "signals")
-        n_out = self.output_length(n)
-        if out is None:
-            if _is_device(signals):
-                import torch
-                out = torch.empty((batch, n_out), device=signals.device, dtype=torch.float32)
-            else:
-                out = np.empty((batch, n_out), np.float32)
-        elif not _is_device(out):
-            if not (isinstance(out, np.ndarray) and out.dtype == np.float32 and out.flags.c_contiguous):
-                raise ValueError("out: expected a C-contiguous float32 numpy array")
-        opitch = 0
-        if _is_device(out):
-            Stft._check_device_tensor(out, "float32", "out")
-            opitch = int(out.stride(0)) if batch > 1 else 0
-        if tuple(out.shape) != (batch, n_out):
-            raise ValueError(f"out: expected shape {(batch, n_out)}, got {tuple(out.shape)}")
-        dev = next((t for t in (out, signals) if _is_device(t)), None)
-        if dev is not None:
-            self._bind_torch_stream(dev)
+        signals, batch, n, spitch = _rows(signals, "signals")
+        out, opitch = _out_rows(out, signals, batch, self.output_length(n))
+        self._bind(out, signals)
         got = _sz(0)
-        st = self.lib.vv_dsp_resample_poly_batch(self._r, _ptr(signals), DEVICE if _is_device(signals) else HOST, batch, n, spitch,
-                                                 _ptr(out), DEVICE if _is_device(out) else HOST, opitch, C.byref(got))
+        st = self.lib.vv_dsp_resample_poly_batch(self._h, _ptr(signals), _space(signals), batch, n, spitch, _ptr(out), _space(out),
+                                                 opitch, C.byref(got))
         _check(self.lib, st, "vv_dsp_resample_poly_batch")
         return out
 
@@ -914,14 +848,15 @@ class Resampler:
 PADTYPES = {None: 0, "none": 0, "odd": 1, "even": 2, "constant": 3}
 
 
-class SosFilter:
+class SosFilter(_StreamHandle):
     """vv_dsp_sos handle (include/vv_dsp/b200.h): batched IIR filtering by a cascade of second-order sections on the
     device, scipy.signal.sosfilt / sosfiltfilt row by row.  sos: [S][6] rows (b0, b1, b2, 1, a1, a2), rounded to float32
     once; every section must have its poles strictly inside the unit circle."""
 
+    _prefix = "sos"
+
     def __init__(self, sos, lib: Library | None = None):
-        self.lib = lib or default_library()
-        self._h = _vp()
+        super().__init__(lib)
         s = np.ascontiguousarray(np.asarray(sos, np.float32))
         if s.ndim != 2 or s.shape[1] != 6:
             raise ValueError("sos: expected an array of shape (n_sections, 6)")
@@ -929,67 +864,11 @@ class SosFilter:
         ns, seg = _sz(0), _sz(0)
         _check(self.lib, self.lib.vv_dsp_sos_get_config(self._h, C.byref(ns), C.byref(seg)), "vv_dsp_sos_get_config")
         self.n_sections, self.segment_length = int(ns.value), int(seg.value)
-        self._stream_pinned = False
-        self._bound_stream = None
-
-    def close(self):
-        if getattr(self, "_h", None) is not None and self._h.value:
-            self.lib.vv_dsp_sos_destroy(self._h)
-            self._h = _vp()
-
-    __del__ = close
-
-    def __enter__(self):
-        return self
-
-    def __exit__(self, *exc):
-        self.close()
-
-    def set_stream(self, cuda_stream):
-        """Pin the handle to a stream (a cudaStream_t as an integer; 0 = the legacy default stream); None = its own
-        stream and back to automatic binding to torch's current stream (see Stft.set_stream)."""
-        self._stream_pinned = cuda_stream is not None
-        self._set_stream_raw(cuda_stream)
-
-    def _set_stream_raw(self, cuda_stream):
-        arg = None if cuda_stream is None else _vp(int(cuda_stream) or 1)
-        _check(self.lib, self.lib.vv_dsp_sos_set_stream(self._h, arg), "vv_dsp_sos_set_stream")
-        self._bound_stream = None if cuda_stream is None else (int(cuda_stream) or 1)
-
-    def _bind_torch_stream(self, tensor):
-        if self._stream_pinned:
-            return
-        import torch
-        cur = int(torch.cuda.current_stream(tensor.device).cuda_stream) or 1
-        if cur != self._bound_stream:
-            self._set_stream_raw(cur)
-
-    def synchronize(self):
-        _check(self.lib, self.lib.vv_dsp_sos_synchronize(self._h), "vv_dsp_sos_synchronize")
-
-    def _out(self, signals, batch, n, out):
-        """the output container ([batch, n] float32 like `signals` unless given) and its row pitch"""
-        if out is None:
-            if _is_device(signals):
-                import torch
-                out = torch.empty((batch, n), device=signals.device, dtype=torch.float32)
-            else:
-                out = np.empty((batch, n), np.float32)
-        elif not _is_device(out):
-            if not (isinstance(out, np.ndarray) and out.dtype == np.float32 and out.flags.c_contiguous):
-                raise ValueError("out: expected a C-contiguous float32 numpy array")
-        opitch = 0
-        if _is_device(out):
-            Stft._check_device_tensor(out, "float32", "out")
-            opitch = int(out.stride(0)) if batch > 1 else 0
-        if tuple(out.shape) != (batch, n):
-            raise ValueError(f"out: expected shape {(batch, n)}, got {tuple(out.shape)}")
-        return out, opitch
 
     def _state(self, z, batch, what):
         """a [S, batch, 2] float32 state in either space, dense"""
         if _is_device(z):
-            Stft._check_device_tensor(z, "float32", what)
+            _check_device_tensor(z, "float32", what)
             if not z.is_contiguous():
                 raise ValueError(f"{what}: expected a contiguous tensor")
         else:
@@ -1002,8 +881,8 @@ class SosFilter:
         """scipy.signal.sosfilt(sos, signals, zi=zi) row by row.  signals: [batch, n] float32 (numpy, or a torch CUDA
         tensor, views with a row pitch included); zi: [S, batch, 2] or None (zero state).  Returns the output in the
         container of `signals` unless `out` is given, and (output, zf) when return_zf."""
-        signals, batch, n, spitch = FirFilter._rows(signals, "signals")
-        out, opitch = self._out(signals, batch, n, out)
+        signals, batch, n, spitch = _rows(signals, "signals")
+        out, opitch = _out_rows(out, signals, batch, n)
         if zi is not None:
             zi = self._state(zi, batch, "zi")
         zf = None
@@ -1013,14 +892,9 @@ class SosFilter:
                 zf = torch.empty((self.n_sections, batch, 2), device=signals.device, dtype=torch.float32)
             else:
                 zf = np.empty((self.n_sections, batch, 2), np.float32)
-        dev = next((t for t in (out, signals, zi, zf) if t is not None and _is_device(t)), None)
-        if dev is not None:
-            self._bind_torch_stream(dev)
-        space = lambda t: DEVICE if t is not None and _is_device(t) else HOST      # noqa: E731
-        st = self.lib.vv_dsp_sos_filter_batch(self._h, _ptr(signals), space(signals), batch, n, spitch,
-                                              None if zi is None else _ptr(zi), space(zi),
-                                              None if zf is None else _ptr(zf), space(zf),
-                                              _ptr(out), space(out), opitch)
+        self._bind(out, signals, zi, zf)
+        st = self.lib.vv_dsp_sos_filter_batch(self._h, _ptr(signals), _space(signals), batch, n, spitch, _ptr(zi), _space(zi),
+                                              _ptr(zf), _space(zf), _ptr(out), _space(out), opitch)
         _check(self.lib, st, "vv_dsp_sos_filter_batch")
         return (out, zf) if return_zf else out
 
@@ -1029,14 +903,11 @@ class SosFilter:
         default.  Returns the output in the container of `signals` unless `out` is given."""
         if padtype not in PADTYPES:
             raise ValueError(f"padtype: expected one of {sorted(k for k in PADTYPES if k)} or None")
-        signals, batch, n, spitch = FirFilter._rows(signals, "signals")
-        out, opitch = self._out(signals, batch, n, out)
-        dev = next((t for t in (out, signals) if _is_device(t)), None)
-        if dev is not None:
-            self._bind_torch_stream(dev)
-        st = self.lib.vv_dsp_sos_filtfilt_batch(self._h, _ptr(signals), DEVICE if _is_device(signals) else HOST, batch, n,
-                                                spitch, PADTYPES[padtype], (1 << 64) - 1 if padlen is None else int(padlen),
-                                                _ptr(out), DEVICE if _is_device(out) else HOST, opitch)
+        signals, batch, n, spitch = _rows(signals, "signals")
+        out, opitch = _out_rows(out, signals, batch, n)
+        self._bind(out, signals)
+        st = self.lib.vv_dsp_sos_filtfilt_batch(self._h, _ptr(signals), _space(signals), batch, n, spitch, PADTYPES[padtype],
+                                                (1 << 64) - 1 if padlen is None else int(padlen), _ptr(out), _space(out), opitch)
         _check(self.lib, st, "vv_dsp_sos_filtfilt_batch")
         return out
 
@@ -1078,7 +949,7 @@ class FftPlan:
             else:
                 out = np.empty(oshape, np.float32 if self.type == FFT_C2R else np.complex64)
         st = self.lib.vv_dsp_fft_execute_batch(self._p, _ptr(x), DEVICE if dev else HOST, _ptr(out),
-                                               DEVICE if _is_device(out) else HOST, batch,
+                                               _space(out), batch,
                                                _vp(int(stream) or 1) if stream is not None else None)
         _check(self.lib, st, "vv_dsp_fft_execute_batch")
         return out

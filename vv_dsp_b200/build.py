@@ -17,7 +17,10 @@ ROOT = os.path.dirname(PKG)
 INC = os.path.join(ROOT, "include")
 LIB = os.path.join(PKG, "lib", "libvvdsp_b200.so")
 OBJ = os.path.join(PKG, "lib", "obj")
-HOST_SRCS = [os.path.join(PKG, "csrc", "host", f) for f in ("window.c", "framing.c", "fft.c", "stft.c", "stream.c", "mel.c", "pcm.c", "fir.c", "resample.c", "sos.c")]
+HOST_DIR = os.path.join(PKG, "csrc", "host")
+# the one list of C99 host units (the emulator build of tests/emu imports it) and the headers they share
+HOST_SRCS = sorted(os.path.join(HOST_DIR, f) for f in os.listdir(HOST_DIR) if f.endswith(".c"))
+HOST_DEPS = sorted(os.path.join(HOST_DIR, f) for f in os.listdir(HOST_DIR) if f.endswith(".h"))
 CUDA_DIR = os.path.join(PKG, "csrc", "cuda")
 # one kernel family per translation unit (vvb_tu_*.cu) + the C-ABI / runtime unit: compiled in parallel
 CUDA_SRCS = sorted(os.path.join(CUDA_DIR, f) for f in os.listdir(CUDA_DIR) if f.endswith(".cu"))
@@ -59,7 +62,7 @@ def build(force: bool = False, verbose: bool = False) -> str:
     objs = []
     for src in HOST_SRCS:
         o = os.path.join(OBJ, os.path.basename(src) + ".o")
-        if force or _stale(o, [src] + hdrs):
+        if force or _stale(o, [src] + HOST_DEPS + hdrs):
             _run(["gcc", "-std=c99", "-O2", "-fPIC", "-Wall", "-Wextra", "-I" + INC, "-c", src, "-o", o], verbose)
         objs.append(o)
     # VVB_NVCC_EXTRA: extra nvcc flags for A/B builds (e.g. "-DVVB_INV_BASETW=0")

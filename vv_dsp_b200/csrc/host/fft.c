@@ -18,6 +18,7 @@
 #include "vv_dsp/spectral/fft.h"
 #include "vv_dsp/b200.h"
 #include "vvb200_cuda.h"
+#include "internal.h"
 
 struct vv_dsp_fft_plan {
     size_t n;
@@ -132,8 +133,7 @@ vv_dsp_status vv_dsp_fft_execute_batch(const vv_dsp_fft_plan* plan, const void* 
     if (batch == 0) return VV_DSP_OK;
     stream = cuda_stream ? cuda_stream : plan->stream;
     if (in_space == VV_DSP_MEM_DEVICE && out_space == VV_DSP_MEM_DEVICE) {
-        st = vvb_fft_exec(plan->eng, in, out, batch, stream);
-        return st == 0 ? VV_DSP_OK : (st >= 1 && st <= 6 ? (vv_dsp_status)st : VV_DSP_ERROR_INTERNAL);
+        return vvdsp_internal_status(vvb_fft_exec(plan->eng, in, out, batch, stream));
     }
     if (in_space == VV_DSP_MEM_HOST) {
         st = vvb_malloc(&d_in, plan->in_bytes * batch);
@@ -144,7 +144,7 @@ vv_dsp_status vv_dsp_fft_execute_batch(const vv_dsp_fft_plan* plan, const void* 
     if (!st && out_space == VV_DSP_MEM_HOST) st = vvb_memcpy_d2h(out, d_out, plan->out_bytes * batch, stream);
     { int s2 = vvb_stream_sync(stream); if (!st) st = s2; }
     vvb_free(d_in); vvb_free(d_out);
-    if (st) return (st >= 1 && st <= 6) ? (vv_dsp_status)st : VV_DSP_ERROR_INTERNAL;
+    if (st) return vvdsp_internal_status(st);
     if (out_space == VV_DSP_MEM_HOST && plan->type == VV_DSP_FFT_R2C && plan->n % 2 == 0 && plan->n > 1) {
         size_t b, bins = plan->n / 2 + 1;
         for (b = 0; b < batch; ++b) ((vv_dsp_cpx*)out)[b * bins + plan->n / 2].im = 0.0f;

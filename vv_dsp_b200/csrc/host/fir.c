@@ -6,9 +6,8 @@
 #include <stdlib.h>
 #include "vv_dsp/b200.h"
 #include "vvb200_cuda.h"
+#include "internal.h"
 
-/* staging bytes per chunk of HOST signals (as in stft.c; VVB_STAGE_TARGET_BYTES overrides it) */
-#define FIR_STAGE_TARGET_BYTES ((size_t)96 << 20)
 /* bound of the handle's filter-spectra scratch: per-signal filters beyond it are processed in chunks of signals */
 #define FIR_SPEC_TARGET_BYTES ((size_t)128 << 20)
 #define FIR_MIN_FFT 128
@@ -17,31 +16,13 @@
 
 struct vv_dsp_fir {
     size_t taps, fft_size, parts, lp;
-    int device;                       /* the CUDA device the handle was created on: every entry point runs there */
+    handle_core core;
     vvb_fir_engine* eng;
-    void* own_stream;
-    void* stream;                     /* own_stream or the caller's */
-    size_t stage_target;
     float* d_h;     size_t h_bytes;   /* filters staged from HOST */
     vvb_cpx* d_spec; size_t spec_bytes;
     float* d_x;     size_t x_bytes;   /* signals staged from HOST */
     float* d_y;     size_t y_bytes;   /* output staged for HOST */
 };
-
-static vv_dsp_status map_status(int st)
-{
-    if (st == 0) return VV_DSP_OK;
-    if (st >= 1 && st <= 6 && st != 5) return (vv_dsp_status)st;
-    return VV_DSP_ERROR_INTERNAL;
-}
-
-static int dev_enter(const vv_dsp_fir* f)
-{
-    int cur = -1;
-    if (vvb_get_device(&cur) != 0 || cur == f->device) return -1;
-    return vvb_set_device(f->device) == 0 ? cur : -1;
-}
-static void dev_leave(int prev) { if (prev >= 0) vvb_set_device(prev); }
 
 /* The plan rule (documented in b200.h): over transform sizes N = 128 ... 8192 and partition counts P with
  * Lp = ceil(M / P) <= N, the smallest P N log2(N) / (N - Lp + 1); ties to the smaller N, then the fewer passes.
@@ -71,7 +52,7 @@ static void fir_free(vv_dsp_fir* f)
     if (!f) return;
     vvb_free(f->d_h); vvb_free(f->d_spec); vvb_free(f->d_x); vvb_free(f->d_y);
     vvb_fir_engine_destroy(f->eng);
-    if (f->own_stream) vvb_stream_destroy(f->own_stream);
+    vvdsp_internal_core_free(&f->core);
     free(f);
 }
 
@@ -87,16 +68,8 @@ vv_dsp_status vv_dsp_fir_create(size_t num_taps, vv_dsp_fir** out)
     f->taps = num_taps;
     fir_plan(num_taps, &f->fft_size, &f->parts);
     f->lp = (num_taps + f->parts - 1) / f->parts;
-    f->stage_target = FIR_STAGE_TARGET_BYTES;
-    {   /* a small staging size makes a modest batch span many chunks (tests) */
-        const char* env = getenv("VVB_STAGE_TARGET_BYTES");
-        if (env && atol(env) > 0) f->stage_target = (size_t)atol(env);
-    }
-    st = vvb_device_ready();                      /* 6 = no usable device: reported as UNSUPPORTED, never a CPU fallback */
-    if (!st) st = vvb_get_device(&f->device);
+    st = vvdsp_internal_core_init(&f->core);
     if (!st) st = vvb_fir_engine_create(f->fft_size, &f->eng);
-    if (!st) st = vvb_stream_create(&f->own_stream);
-    f->stream = f->own_stream;
     if (st) { fir_free(f); return st == 6 ? VV_DSP_ERROR_UNSUPPORTED : VV_DSP_ERROR_INTERNAL; }
     *out = f;
     return VV_DSP_OK;
@@ -106,27 +79,20 @@ vv_dsp_status vv_dsp_fir_destroy(vv_dsp_fir* f)
 {
     int prev;
     if (!f) return VV_DSP_ERROR_NULL_POINTER;
-    prev = dev_enter(f);
+    prev = vvdsp_internal_enter(&f->core);
     fir_free(f);
-    dev_leave(prev);
+    vvdsp_internal_leave(prev);
     return VV_DSP_OK;
 }
 
 vv_dsp_status vv_dsp_fir_set_stream(vv_dsp_fir* f, void* cuda_stream)
 {
-    if (!f) return VV_DSP_ERROR_NULL_POINTER;
-    f->stream = cuda_stream ? cuda_stream : f->own_stream;
-    return VV_DSP_OK;
+    return vvdsp_internal_set_stream(f ? &f->core : NULL, cuda_stream);
 }
 
 vv_dsp_status vv_dsp_fir_synchronize(vv_dsp_fir* f)
 {
-    int prev, st;
-    if (!f) return VV_DSP_ERROR_NULL_POINTER;
-    prev = dev_enter(f);
-    st = vvb_stream_sync(f->stream);
-    dev_leave(prev);
-    return map_status(st);
+    return vvdsp_internal_synchronize(f ? &f->core : NULL);
 }
 
 vv_dsp_status vv_dsp_fir_get_config(const vv_dsp_fir* f, size_t* fft_size, size_t* partitions)
@@ -137,27 +103,16 @@ vv_dsp_status vv_dsp_fir_get_config(const vv_dsp_fir* f, size_t* fft_size, size_
     return VV_DSP_OK;
 }
 
-/* grow a device scratch to `bytes`; work already enqueued may still use the old one */
-static int reserve(vv_dsp_fir* f, void** buf, size_t* have, size_t bytes)
-{
-    int st;
-    if (bytes <= *have) return 0;
-    st = vvb_stream_sync(f->stream);
-    vvb_free(*buf); *buf = NULL; *have = 0;
-    if (!st) st = vvb_malloc(buf, bytes);
-    if (!st) *have = bytes;
-    return st;
-}
-
 /* filter spectra of `count` filters (rows of `filters` at `pitch`) into d_spec */
 static int make_spectra(vv_dsp_fir* f, const vv_dsp_real* filters, vv_dsp_mem_space space, size_t count, size_t pitch)
 {
     int st = 0;
     if (space == VV_DSP_MEM_HOST) {
-        st = vvb_memcpy2d_h2d(f->d_h, f->taps * sizeof(float), filters, pitch * sizeof(float), f->taps * sizeof(float), count, f->stream);
+        st = vvb_memcpy2d_h2d(f->d_h, f->taps * sizeof(float), filters, pitch * sizeof(float), f->taps * sizeof(float), count,
+                              f->core.stream);
         filters = f->d_h; pitch = f->taps;
     }
-    if (!st) st = vvb_fir_spectra(f->eng, filters, count, pitch, f->taps, f->lp, f->parts, f->d_spec, f->stream);
+    if (!st) st = vvb_fir_spectra(f->eng, filters, count, pitch, f->taps, f->lp, f->parts, f->d_spec, f->core.stream);
     return st;
 }
 
@@ -172,16 +127,17 @@ static int filter_impl(vv_dsp_fir* f, const vv_dsp_real* filters, vv_dsp_mem_spa
     const size_t h_per = (!shared && filters_space == VV_DSP_MEM_HOST) ? f->taps * sizeof(float) : 0;
     const size_t stage_per = (x_per > y_per ? x_per : y_per) + h_per;
     const int any_host = signals_space == VV_DSP_MEM_HOST || out_space == VV_DSP_MEM_HOST || filters_space == VV_DSP_MEM_HOST;
-    size_t cs = batch, done;
+    size_t cs = vvdsp_internal_chunk_rows(&f->core, batch, stage_per), done;
     int st = 0;
-    if (stage_per && f->stage_target / stage_per < cs) cs = f->stage_target / stage_per;
     if (!shared && FIR_SPEC_TARGET_BYTES / spec_per < cs) cs = FIR_SPEC_TARGET_BYTES / spec_per;
     if (cs < 1) cs = 1;
-    st = reserve(f, (void**)&f->d_spec, &f->spec_bytes, (shared ? 1 : cs) * spec_per);
-    if (!st && filters_space == VV_DSP_MEM_HOST) st = reserve(f, (void**)&f->d_h, &f->h_bytes, (shared ? 1 : cs) * f->taps * sizeof(float));
-    if (!st && x_per) st = reserve(f, (void**)&f->d_x, &f->x_bytes, cs * x_per);
-    if (!st && signals_space == VV_DSP_MEM_HOST && !f->d_x) st = reserve(f, (void**)&f->d_x, &f->x_bytes, sizeof(float));   /* n == 0 */
-    if (!st && y_per) st = reserve(f, (void**)&f->d_y, &f->y_bytes, cs * y_per);
+    st = vvdsp_internal_reserve(&f->core, (void**)&f->d_spec, &f->spec_bytes, (shared ? 1 : cs) * spec_per);
+    if (!st && filters_space == VV_DSP_MEM_HOST)
+        st = vvdsp_internal_reserve(&f->core, (void**)&f->d_h, &f->h_bytes, (shared ? 1 : cs) * f->taps * sizeof(float));
+    if (!st && x_per) st = vvdsp_internal_reserve(&f->core, (void**)&f->d_x, &f->x_bytes, cs * x_per);
+    if (!st && signals_space == VV_DSP_MEM_HOST && !f->d_x)                                               /* n == 0 */
+        st = vvdsp_internal_reserve(&f->core, (void**)&f->d_x, &f->x_bytes, sizeof(float));
+    if (!st && y_per) st = vvdsp_internal_reserve(&f->core, (void**)&f->d_y, &f->y_bytes, cs * y_per);
     if (!st && shared) st = make_spectra(f, filters, filters_space, 1, filter_pitch);
     /* every chunk runs on the handle's stream, so stream order keeps the scratch buffers of consecutive chunks apart */
     for (done = 0; done < batch && !st; done += cs) {
@@ -191,18 +147,19 @@ static int filter_impl(vv_dsp_fir* f, const vv_dsp_real* filters, vv_dsp_mem_spa
         size_t xp = signal_pitch, yp = out_pitch;
         if (!shared) st = make_spectra(f, filters + done * filter_pitch, filters_space, nb, filter_pitch);
         if (!st && signals_space == VV_DSP_MEM_HOST) {
-            if (n) st = vvb_memcpy2d_h2d(f->d_x, n * sizeof(float), d_x, signal_pitch * sizeof(float), n * sizeof(float), nb, f->stream);
+            if (n)
+                st = vvb_memcpy2d_h2d(f->d_x, n * sizeof(float), d_x, signal_pitch * sizeof(float), n * sizeof(float), nb,
+                                      f->core.stream);
             d_x = f->d_x; xp = n;
         }
         if (out_space == VV_DSP_MEM_HOST) { d_y = f->d_y; yp = n_out; }
         if (!st) st = vvb_fir_filter(f->eng, f->d_spec, shared ? 0 : f->parts * f->fft_size, f->taps, f->lp, f->parts, d_x, nb, n, xp,
-                                     d_y, n_out, yp, f->stream);
+                                     d_y, n_out, yp, f->core.stream);
         if (!st && out_space == VV_DSP_MEM_HOST)
             st = vvb_memcpy2d_d2h(out + done * out_pitch, out_pitch * sizeof(float), f->d_y, n_out * sizeof(float), n_out * sizeof(float),
-                                  nb, f->stream);
+                                  nb, f->core.stream);
     }
-    if (any_host) { int s2 = vvb_stream_sync(f->stream); if (!st) st = s2; }
-    return st;
+    return vvdsp_internal_finish(&f->core, st, any_host);
 }
 
 vv_dsp_status vv_dsp_fir_filter_batch(vv_dsp_fir* f, const vv_dsp_real* filters, vv_dsp_mem_space filters_space, size_t num_filters,
@@ -220,9 +177,9 @@ vv_dsp_status vv_dsp_fir_filter_batch(vv_dsp_fir* f, const vv_dsp_real* filters,
         return VV_DSP_ERROR_INVALID_SIZE;
     if ((const void*)out == (const void*)signals) return VV_DSP_ERROR_UNSUPPORTED;      /* no in-place filtering */
     if (batch == 0 || n_out == 0) return VV_DSP_OK;
-    prev = dev_enter(f);
+    prev = vvdsp_internal_enter(&f->core);
     st = filter_impl(f, filters, filters_space, num_filters, filter_pitch, signals, signals_space, batch, n, signal_pitch, out, out_space,
                      n_out, out_pitch);
-    dev_leave(prev);
-    return map_status(st);
+    vvdsp_internal_leave(prev);
+    return vvdsp_internal_status(st);
 }

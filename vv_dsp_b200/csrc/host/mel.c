@@ -451,12 +451,6 @@ int vvdsp_internal_logmel(const mel_device* md, const float* d_power, size_t fra
     return vvb_logmel(d_power, frames, bins, bins, md->d_meta, md->d_w, n_mels, md->n_groups, eps, d_out, stream);
 }
 
-static vv_dsp_status to_status(int st)
-{
-    if (st == 0) return VV_DSP_OK;
-    return (st >= 1 && st <= 6 && st != 5) ? (vv_dsp_status)st : VV_DSP_ERROR_INTERNAL;
-}
-
 vv_dsp_status vv_dsp_compute_log_mel_spectrogram(const vv_dsp_real* power_spectrogram, size_t num_frames, size_t n_fft_bins,
                                                  const vv_dsp_real* filterbank_weights, size_t n_mels, vv_dsp_real log_epsilon,
                                                  vv_dsp_real* out_log_mel_spectrogram)
@@ -470,7 +464,7 @@ vv_dsp_status vv_dsp_compute_log_mel_spectrogram(const vv_dsp_real* power_spectr
     if (log_epsilon < 0.0f) return VV_DSP_ERROR_OUT_OF_RANGE;
     memset(&md, 0, sizeof(md));
     st = vvb_device_ready();                         /* no CUDA device -> UNSUPPORTED, never a CPU computation */
-    if (st) return to_status(st);
+    if (st) return vvdsp_internal_status(st);
     st = vvb_stream_create(&stream);
     if (!st) st = vvdsp_internal_mel_device_build(filterbank_weights, n_mels, n_fft_bins, stream, &md);
     if (!st) st = vvb_malloc((void**)&d_p, num_frames * n_fft_bins * sizeof(float));
@@ -481,7 +475,7 @@ vv_dsp_status vv_dsp_compute_log_mel_spectrogram(const vv_dsp_real* power_spectr
     if (stream) { int s2 = vvb_stream_sync(stream); if (!st) st = s2; }
     vvb_free(d_p); vvb_free(d_o); vvdsp_internal_mel_device_free(&md);
     if (stream) vvb_stream_destroy(stream);
-    return to_status(st);
+    return vvdsp_internal_status(st);
 }
 
 /* ------------------------------------------------------------------ MFCC (src/features/mel.c:249-461) */
@@ -539,7 +533,7 @@ vv_dsp_status vv_dsp_mfcc(const vv_dsp_real* log_mel_spectrogram, size_t num_fra
     if (v != VV_DSP_OK) return v;
     md.d_table = NULL; md.d_lifter = NULL;
     st = vvb_device_ready();
-    if (st) return to_status(st);
+    if (st) return vvdsp_internal_status(st);
     st = vvb_stream_create(&stream);
     if (!st) st = vvdsp_internal_mfcc_device_build(n_mels, num_mfcc_coeffs, lifter_coeff, stream, &md);
     if (!st) st = vvb_malloc((void**)&d_in, num_frames * n_mels * sizeof(float));
@@ -550,7 +544,7 @@ vv_dsp_status vv_dsp_mfcc(const vv_dsp_real* log_mel_spectrogram, size_t num_fra
     if (stream) { int s2 = vvb_stream_sync(stream); if (!st) st = s2; }
     vvb_free(d_in); vvb_free(d_out); vvdsp_internal_mfcc_device_free(&md);
     if (stream) vvb_stream_destroy(stream);
-    return to_status(st);
+    return vvdsp_internal_status(st);
 }
 
 struct vv_dsp_mfcc_plan {
@@ -595,7 +589,7 @@ vv_dsp_status vv_dsp_mfcc_process(const vv_dsp_mfcc_plan* plan, const vv_dsp_rea
     v = mfcc_validate(num_frames, p->n_mels, p->n_coeffs, p->dct_type, p->lifter);
     if (v != VV_DSP_OK) return v;
     st = vvb_device_ready();
-    if (st) return to_status(st);
+    if (st) return vvdsp_internal_status(st);
     if (!p->on_device) {
         st = vvb_stream_create(&p->stream);
         if (!st) st = vvdsp_internal_mel_device_build(p->weights, p->n_mels, p->bins, p->stream, &p->mel);
@@ -603,7 +597,7 @@ vv_dsp_status vv_dsp_mfcc_process(const vv_dsp_mfcc_plan* plan, const vv_dsp_rea
         if (st) {
             vvdsp_internal_mel_device_free(&p->mel); vvdsp_internal_mfcc_device_free(&p->mfcc);
             if (p->stream) { vvb_stream_destroy(p->stream); p->stream = NULL; }
-            return to_status(st);
+            return vvdsp_internal_status(st);
         }
         p->on_device = 1;
     }
@@ -617,7 +611,7 @@ vv_dsp_status vv_dsp_mfcc_process(const vv_dsp_mfcc_plan* plan, const vv_dsp_rea
     if (!st) st = vvb_memcpy_d2h(out_mfcc_coeffs, d_o, num_frames * p->n_coeffs * sizeof(float), p->stream);
     { int s2 = vvb_stream_sync(p->stream); if (!st) st = s2; }
     vvb_free(d_p); vvb_free(d_lm); vvb_free(d_o);
-    return to_status(st);
+    return vvdsp_internal_status(st);
 }
 
 vv_dsp_status vv_dsp_mfcc_destroy(vv_dsp_mfcc_plan* plan)

@@ -6,12 +6,7 @@
 #include <stdlib.h>
 #include "vv_dsp/b200.h"
 #include "vvb200_cuda.h"
-
-static vv_dsp_status to_status(int st)
-{
-    if (st == 0) return VV_DSP_OK;
-    return (st >= 1 && st <= 6 && st != 5) ? (vv_dsp_status)st : VV_DSP_ERROR_INTERNAL;
-}
+#include "internal.h"
 
 vv_dsp_status vv_dsp_b200_pcm_to_planar(const void* interleaved, vv_dsp_mem_space in_space, int format, size_t num_samples,
                                         size_t channels, vv_dsp_real* planar, vv_dsp_mem_space out_space, size_t planar_pitch,
@@ -29,7 +24,7 @@ vv_dsp_status vv_dsp_b200_pcm_to_planar(const void* interleaved, vv_dsp_mem_spac
     if (planar_pitch == 0) planar_pitch = num_samples;
     if (planar_pitch < num_samples) return VV_DSP_ERROR_INVALID_SIZE;
     st = vvb_device_ready();                 /* no CUDA device -> UNSUPPORTED, never a CPU conversion */
-    if (st) return to_status(st);
+    if (st) return vvdsp_internal_status(st);
     if (!stream && (in_space == VV_DSP_MEM_HOST || out_space == VV_DSP_MEM_HOST)) { st = vvb_stream_create(&own); stream = own; }
     if (!st && in_space == VV_DSP_MEM_HOST) {
         st = vvb_malloc(&d_tmp_in, num_samples * channels * bytes_per);
@@ -50,5 +45,5 @@ vv_dsp_status vv_dsp_b200_pcm_to_planar(const void* interleaved, vv_dsp_mem_spac
         vvb_free(d_tmp_in); vvb_free(d_tmp_out);
     }
     if (own) vvb_stream_destroy(own);
-    return to_status(st);
+    return vvdsp_internal_status(st);
 }

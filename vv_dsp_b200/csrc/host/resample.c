@@ -9,38 +9,19 @@
 #include <string.h>
 #include "vv_dsp/b200.h"
 #include "vvb200_cuda.h"
+#include "internal.h"
 
-/* staging bytes per chunk of HOST rows (as in fir.c; VVB_STAGE_TARGET_BYTES overrides it) */
-#define RS_STAGE_TARGET_BYTES ((size_t)96 << 20)
 #define RS_MAX_BANK ((size_t)65536)             /* up T: the default design of every pair of standard rates fits */
 #define RS_MAX_RATIO ((size_t)0x7fffffff)       /* up and down after reduction: keeps the kernel's index products in range */
 #define RS_MAX_UPSAMPLED ((size_t)1 << 62)      /* n up */
 
 struct vv_dsp_resample_poly {
     size_t up, down, taps, per_phase, half;
-    int device;                       /* the CUDA device the handle was created on: every entry point runs there */
+    handle_core core;
     float* d_bank;                    /* [per_phase][up], NULL for the identity ratio */
-    void* own_stream;
-    void* stream;                     /* own_stream or the caller's */
-    size_t stage_target;
     float* d_x;     size_t x_bytes;   /* signals staged from HOST */
     float* d_y;     size_t y_bytes;   /* output staged for HOST */
 };
-
-static vv_dsp_status map_status(int st)
-{
-    if (st == 0) return VV_DSP_OK;
-    if (st >= 1 && st <= 6 && st != 5) return (vv_dsp_status)st;
-    return VV_DSP_ERROR_INTERNAL;
-}
-
-static int dev_enter(const vv_dsp_resample_poly* r)
-{
-    int cur = -1;
-    if (vvb_get_device(&cur) != 0 || cur == r->device) return -1;
-    return vvb_set_device(r->device) == 0 ? cur : -1;
-}
-static void dev_leave(int prev) { if (prev >= 0) vvb_set_device(prev); }
 
 static size_t gcd(size_t a, size_t b)
 {
@@ -86,7 +67,7 @@ static void rs_free(vv_dsp_resample_poly* r)
 {
     if (!r) return;
     vvb_free(r->d_bank); vvb_free(r->d_x); vvb_free(r->d_y);
-    if (r->own_stream) vvb_stream_destroy(r->own_stream);
+    vvdsp_internal_core_free(&r->core);
     free(r);
 }
 
@@ -110,15 +91,7 @@ vv_dsp_status vv_dsp_resample_poly_create(size_t up, size_t down, const vv_dsp_r
     r->half = (r->taps - 1) / 2;
     r->per_phase = (r->taps + up - 1) / up;
     if (!(up == 1 && down == 1) && (r->per_phase > RS_MAX_BANK / up)) { free(r); return VV_DSP_ERROR_INVALID_SIZE; }
-    r->stage_target = RS_STAGE_TARGET_BYTES;
-    {   /* a small staging size makes a modest batch span many chunks (tests) */
-        const char* env = getenv("VVB_STAGE_TARGET_BYTES");
-        if (env && atol(env) > 0) r->stage_target = (size_t)atol(env);
-    }
-    st = vvb_device_ready();                      /* 6 = no usable device: reported as UNSUPPORTED, never a CPU fallback */
-    if (!st) st = vvb_get_device(&r->device);
-    if (!st) st = vvb_stream_create(&r->own_stream);
-    r->stream = r->own_stream;
+    st = vvdsp_internal_core_init(&r->core);
     if (!st && !(up == 1 && down == 1)) {        /* the identity ratio copies: no filter, no bank */
         const size_t bank_n = up * r->per_phase;
         double* h = (double*)malloc(r->taps * sizeof(double));
@@ -135,8 +108,8 @@ vv_dsp_status vv_dsp_resample_poly_create(size_t up, size_t down, const vv_dsp_r
                     bank[j * up + phi] = k < r->taps ? (float)((double)up * h[k]) : 0.0f;
                 }
             st = vvb_malloc((void**)&r->d_bank, bank_n * sizeof(float));
-            if (!st) st = vvb_memcpy_h2d(r->d_bank, bank, bank_n * sizeof(float), r->stream);
-            if (!st) st = vvb_stream_sync(r->stream);
+            if (!st) st = vvb_memcpy_h2d(r->d_bank, bank, bank_n * sizeof(float), r->core.stream);
+            if (!st) st = vvb_stream_sync(r->core.stream);
         }
         free(h); free(bank);
     }
@@ -149,27 +122,20 @@ vv_dsp_status vv_dsp_resample_poly_destroy(vv_dsp_resample_poly* r)
 {
     int prev;
     if (!r) return VV_DSP_ERROR_NULL_POINTER;
-    prev = dev_enter(r);
+    prev = vvdsp_internal_enter(&r->core);
     rs_free(r);
-    dev_leave(prev);
+    vvdsp_internal_leave(prev);
     return VV_DSP_OK;
 }
 
 vv_dsp_status vv_dsp_resample_poly_set_stream(vv_dsp_resample_poly* r, void* cuda_stream)
 {
-    if (!r) return VV_DSP_ERROR_NULL_POINTER;
-    r->stream = cuda_stream ? cuda_stream : r->own_stream;
-    return VV_DSP_OK;
+    return vvdsp_internal_set_stream(r ? &r->core : NULL, cuda_stream);
 }
 
 vv_dsp_status vv_dsp_resample_poly_synchronize(vv_dsp_resample_poly* r)
 {
-    int prev, st;
-    if (!r) return VV_DSP_ERROR_NULL_POINTER;
-    prev = dev_enter(r);
-    st = vvb_stream_sync(r->stream);
-    dev_leave(prev);
-    return map_status(st);
+    return vvdsp_internal_synchronize(r ? &r->core : NULL);
 }
 
 vv_dsp_status vv_dsp_resample_poly_get_config(const vv_dsp_resample_poly* r, size_t* up, size_t* down, size_t* num_taps,
@@ -187,18 +153,6 @@ size_t vv_dsp_resample_poly_output_length(const vv_dsp_resample_poly* r, size_t 
     return (n / r->down) * r->up + ((n % r->down) * r->up + r->down - 1) / r->down;
 }
 
-/* grow a device scratch to `bytes`; work already enqueued may still use the old one */
-static int reserve(vv_dsp_resample_poly* r, void** buf, size_t* have, size_t bytes)
-{
-    int st;
-    if (bytes <= *have) return 0;
-    st = vvb_stream_sync(r->stream);
-    vvb_free(*buf); *buf = NULL; *have = 0;
-    if (!st) st = vvb_malloc(buf, bytes);
-    if (!st) *have = bytes;
-    return st;
-}
-
 static int copy_rows(vv_dsp_resample_poly* r, const vv_dsp_real* src, vv_dsp_mem_space ss, size_t sp, vv_dsp_real* dst,
                      vv_dsp_mem_space ds, size_t dp, size_t rows, size_t n)
 {
@@ -208,9 +162,9 @@ static int copy_rows(vv_dsp_resample_poly* r, const vv_dsp_real* src, vv_dsp_mem
         for (b = 0; b < rows; ++b) memcpy(dst + b * dp, src + b * sp, w);
         return 0;
     }
-    if (ss == VV_DSP_MEM_HOST) return vvb_memcpy2d_h2d(dst, dp * sizeof(float), src, sp * sizeof(float), w, rows, r->stream);
-    if (ds == VV_DSP_MEM_HOST) return vvb_memcpy2d_d2h(dst, dp * sizeof(float), src, sp * sizeof(float), w, rows, r->stream);
-    return vvb_memcpy2d_d2d(dst, dp * sizeof(float), src, sp * sizeof(float), w, rows, r->stream);
+    if (ss == VV_DSP_MEM_HOST) return vvb_memcpy2d_h2d(dst, dp * sizeof(float), src, sp * sizeof(float), w, rows, r->core.stream);
+    if (ds == VV_DSP_MEM_HOST) return vvb_memcpy2d_d2h(dst, dp * sizeof(float), src, sp * sizeof(float), w, rows, r->core.stream);
+    return vvb_memcpy2d_d2d(dst, dp * sizeof(float), src, sp * sizeof(float), w, rows, r->core.stream);
 }
 
 static int resample_impl(vv_dsp_resample_poly* r, const vv_dsp_real* signals, vv_dsp_mem_space signals_space, size_t batch,
@@ -219,19 +173,16 @@ static int resample_impl(vv_dsp_resample_poly* r, const vv_dsp_real* signals, vv
 {
     const size_t x_per = signals_space == VV_DSP_MEM_HOST ? n * sizeof(float) : 0;
     const size_t y_per = out_space == VV_DSP_MEM_HOST ? n_out * sizeof(float) : 0;
-    const size_t stage_per = x_per > y_per ? x_per : y_per;
+    const size_t cs = vvdsp_internal_chunk_rows(&r->core, batch, x_per > y_per ? x_per : y_per);
     const int any_host = signals_space == VV_DSP_MEM_HOST || out_space == VV_DSP_MEM_HOST;
-    size_t cs = batch, done;
+    size_t done;
     int st = 0;
     if (!r->d_bank) {                             /* identity ratio: a copy, bit for bit */
         st = copy_rows(r, signals, signals_space, signal_pitch, out, out_space, out_pitch, batch, n);
-        if (any_host) { int s2 = vvb_stream_sync(r->stream); if (!st) st = s2; }
-        return st;
+        return vvdsp_internal_finish(&r->core, st, any_host);
     }
-    if (stage_per && r->stage_target / stage_per < cs) cs = r->stage_target / stage_per;
-    if (cs < 1) cs = 1;
-    if (x_per) st = reserve(r, (void**)&r->d_x, &r->x_bytes, cs * x_per);
-    if (!st && y_per) st = reserve(r, (void**)&r->d_y, &r->y_bytes, cs * y_per);
+    if (x_per) st = vvdsp_internal_reserve(&r->core, (void**)&r->d_x, &r->x_bytes, cs * x_per);
+    if (!st && y_per) st = vvdsp_internal_reserve(&r->core, (void**)&r->d_y, &r->y_bytes, cs * y_per);
     /* every chunk runs on the handle's stream, so stream order keeps the scratch buffers of consecutive chunks apart */
     for (done = 0; done < batch && !st; done += cs) {
         const size_t nb = batch - done < cs ? batch - done : cs;
@@ -239,17 +190,17 @@ static int resample_impl(vv_dsp_resample_poly* r, const vv_dsp_real* signals, vv
         float* d_y = out + done * out_pitch;
         size_t xp = signal_pitch, yp = out_pitch;
         if (signals_space == VV_DSP_MEM_HOST) {
-            st = vvb_memcpy2d_h2d(r->d_x, n * sizeof(float), d_x, signal_pitch * sizeof(float), n * sizeof(float), nb, r->stream);
+            st = vvb_memcpy2d_h2d(r->d_x, n * sizeof(float), d_x, signal_pitch * sizeof(float), n * sizeof(float), nb, r->core.stream);
             d_x = r->d_x; xp = n;
         }
         if (out_space == VV_DSP_MEM_HOST) { d_y = r->d_y; yp = n_out; }
-        if (!st) st = vvb_resample_poly(r->d_bank, r->up, r->down, r->per_phase, r->half, d_x, nb, n, xp, d_y, n_out, yp, r->stream);
+        if (!st)
+            st = vvb_resample_poly(r->d_bank, r->up, r->down, r->per_phase, r->half, d_x, nb, n, xp, d_y, n_out, yp, r->core.stream);
         if (!st && out_space == VV_DSP_MEM_HOST)
             st = vvb_memcpy2d_d2h(out + done * out_pitch, out_pitch * sizeof(float), r->d_y, n_out * sizeof(float), n_out * sizeof(float),
-                                  nb, r->stream);
+                                  nb, r->core.stream);
     }
-    if (any_host) { int s2 = vvb_stream_sync(r->stream); if (!st) st = s2; }
-    return st;
+    return vvdsp_internal_finish(&r->core, st, any_host);
 }
 
 vv_dsp_status vv_dsp_resample_poly_batch(vv_dsp_resample_poly* r, const vv_dsp_real* signals, vv_dsp_mem_space signals_space,
@@ -268,8 +219,8 @@ vv_dsp_status vv_dsp_resample_poly_batch(vv_dsp_resample_poly* r, const vv_dsp_r
     if ((const void*)out == (const void*)signals) return VV_DSP_ERROR_UNSUPPORTED;      /* no in-place resampling */
     *out_len = n_out;
     if (batch == 0 || n == 0) return VV_DSP_OK;
-    prev = dev_enter(r);
+    prev = vvdsp_internal_enter(&r->core);
     st = resample_impl(r, signals, signals_space, batch, n, signal_pitch, out, out_space, n_out, out_pitch);
-    dev_leave(prev);
-    return map_status(st);
+    vvdsp_internal_leave(prev);
+    return vvdsp_internal_status(st);
 }

@@ -9,22 +9,18 @@
 #include <string.h>
 #include "vv_dsp/b200.h"
 #include "vvb200_cuda.h"
+#include "internal.h"
 
-/* staging bytes per chunk of HOST rows (as in resample.c; VVB_STAGE_TARGET_BYTES overrides it) */
-#define SOS_STAGE_TARGET_BYTES ((size_t)96 << 20)
 typedef char sos_tile_is_the_kernels[(VV_DSP_SOS_TILE == VVB_IIR_THREADS * VVB_IIR_RUN) ? 1 : -1];
 typedef char sos_chain_fits[(2 * VV_DSP_SOS_MAX_SECTIONS <= 128) ? 1 : -1];
 
 struct vv_dsp_sos {
     size_t sections, segment;
     size_t default_padlen;            /* scipy's 3 (2S + 1 - min(#{b2 == 0}, #{a2 == 0})) */
-    int device;                       /* the CUDA device the handle was created on: every entry point runs there */
+    handle_core core;
     double* d_table;                  /* [S][VVB_IIR_TABLE] */
     float* d_phi;                     /* [2S][2S] */
     float* d_zi_unit;                 /* [S][2]: sosfilt_zi(sos) */
-    void* own_stream;
-    void* stream;                     /* own_stream or the caller's */
-    size_t stage_target;
     float* d_x;     size_t x_bytes;   /* signals staged from HOST */
     float* d_y;     size_t y_bytes;   /* output staged for HOST */
     float* d_fwd;   size_t fwd_bytes; /* filtfilt: the forward pass over the padded rows */
@@ -32,21 +28,6 @@ struct vv_dsp_sos {
     float* d_zi;    size_t zi_bytes;  /* zi staged from HOST */
     float* d_zf;    size_t zf_bytes;  /* zf staged for HOST */
 };
-
-static vv_dsp_status map_status(int st)
-{
-    if (st == 0) return VV_DSP_OK;
-    if (st >= 1 && st <= 6 && st != 5) return (vv_dsp_status)st;
-    return VV_DSP_ERROR_INTERNAL;
-}
-
-static int dev_enter(const vv_dsp_sos* h)
-{
-    int cur = -1;
-    if (vvb_get_device(&cur) != 0 || cur == h->device) return -1;
-    return vvb_set_device(h->device) == 0 ? cur : -1;
-}
-static void dev_leave(int prev) { if (prev >= 0) vvb_set_device(prev); }
 
 /* c = a b, n x n row-major; c may not alias a or b */
 static void matmul(const double* a, const double* b, double* c, size_t n)
@@ -133,7 +114,7 @@ static void sos_free(vv_dsp_sos* h)
     if (!h) return;
     vvb_free(h->d_table); vvb_free(h->d_phi); vvb_free(h->d_zi_unit);
     vvb_free(h->d_x); vvb_free(h->d_y); vvb_free(h->d_fwd); vvb_free(h->d_seg); vvb_free(h->d_zi); vvb_free(h->d_zf);
-    if (h->own_stream) vvb_stream_destroy(h->own_stream);
+    vvdsp_internal_core_free(&h->core);
     free(h);
 }
 
@@ -165,15 +146,7 @@ vv_dsp_status vv_dsp_sos_create(const vv_dsp_real* sos, size_t n_sections, vv_ds
         const char* env = getenv("VVB_IIR_SEGMENT");
         if (env && atol(env) > 0) h->segment = ((size_t)atol(env) + VV_DSP_SOS_TILE - 1) / VV_DSP_SOS_TILE * VV_DSP_SOS_TILE;
     }
-    h->stage_target = SOS_STAGE_TARGET_BYTES;
-    {   /* a small staging size makes a modest batch span many chunks (tests) */
-        const char* env = getenv("VVB_STAGE_TARGET_BYTES");
-        if (env && atol(env) > 0) h->stage_target = (size_t)atol(env);
-    }
-    st = vvb_device_ready();                      /* 6 = no usable device: reported as UNSUPPORTED, never a CPU fallback */
-    if (!st) st = vvb_get_device(&h->device);
-    if (!st) st = vvb_stream_create(&h->own_stream);
-    h->stream = h->own_stream;
+    st = vvdsp_internal_core_init(&h->core);
     if (!st) {
         const size_t S = n_sections, nt = S * VVB_IIR_TABLE, np = 4 * S * S;
         double* table = (double*)malloc(nt * sizeof(double));
@@ -183,10 +156,10 @@ vv_dsp_status vv_dsp_sos_create(const vv_dsp_real* sos, size_t n_sections, vv_ds
         if (!st) st = vvb_malloc((void**)&h->d_table, nt * sizeof(double));
         if (!st) st = vvb_malloc((void**)&h->d_phi, np * sizeof(float));
         if (!st) st = vvb_malloc((void**)&h->d_zi_unit, 2 * S * sizeof(float));
-        if (!st) st = vvb_memcpy_h2d(h->d_table, table, nt * sizeof(double), h->stream);
-        if (!st) st = vvb_memcpy_h2d(h->d_phi, phi, np * sizeof(float), h->stream);
-        if (!st) st = vvb_memcpy_h2d(h->d_zi_unit, zi, 2 * S * sizeof(float), h->stream);
-        if (!st) st = vvb_stream_sync(h->stream);
+        if (!st) st = vvb_memcpy_h2d(h->d_table, table, nt * sizeof(double), h->core.stream);
+        if (!st) st = vvb_memcpy_h2d(h->d_phi, phi, np * sizeof(float), h->core.stream);
+        if (!st) st = vvb_memcpy_h2d(h->d_zi_unit, zi, 2 * S * sizeof(float), h->core.stream);
+        if (!st) st = vvb_stream_sync(h->core.stream);
         free(table); free(phi); free(zi);
     }
     if (st) { sos_free(h); return st == 6 ? VV_DSP_ERROR_UNSUPPORTED : VV_DSP_ERROR_INTERNAL; }
@@ -198,27 +171,20 @@ vv_dsp_status vv_dsp_sos_destroy(vv_dsp_sos* h)
 {
     int prev;
     if (!h) return VV_DSP_ERROR_NULL_POINTER;
-    prev = dev_enter(h);
+    prev = vvdsp_internal_enter(&h->core);
     sos_free(h);
-    dev_leave(prev);
+    vvdsp_internal_leave(prev);
     return VV_DSP_OK;
 }
 
 vv_dsp_status vv_dsp_sos_set_stream(vv_dsp_sos* h, void* cuda_stream)
 {
-    if (!h) return VV_DSP_ERROR_NULL_POINTER;
-    h->stream = cuda_stream ? cuda_stream : h->own_stream;
-    return VV_DSP_OK;
+    return vvdsp_internal_set_stream(h ? &h->core : NULL, cuda_stream);
 }
 
 vv_dsp_status vv_dsp_sos_synchronize(vv_dsp_sos* h)
 {
-    int prev, st;
-    if (!h) return VV_DSP_ERROR_NULL_POINTER;
-    prev = dev_enter(h);
-    st = vvb_stream_sync(h->stream);
-    dev_leave(prev);
-    return map_status(st);
+    return vvdsp_internal_synchronize(h ? &h->core : NULL);
 }
 
 vv_dsp_status vv_dsp_sos_get_config(const vv_dsp_sos* h, size_t* n_sections, size_t* segment_length)
@@ -229,31 +195,12 @@ vv_dsp_status vv_dsp_sos_get_config(const vv_dsp_sos* h, size_t* n_sections, siz
     return VV_DSP_OK;
 }
 
-/* grow a device scratch to `bytes`; work already enqueued may still use the old one */
-static int reserve(vv_dsp_sos* h, float** buf, size_t* have, size_t bytes)
-{
-    int st;
-    if (bytes <= *have) return 0;
-    st = vvb_stream_sync(h->stream);
-    vvb_free(*buf); *buf = NULL; *have = 0;
-    if (!st) st = vvb_malloc((void**)buf, bytes);
-    if (!st) *have = bytes;
-    return st;
-}
-
-/* rows of `batch` signals per chunk: every chunk's HOST staging fits the target */
-static size_t chunk_rows(const vv_dsp_sos* h, size_t batch, size_t stage_per)
-{
-    size_t cs = batch;
-    if (stage_per && h->stage_target / stage_per < cs) cs = h->stage_target / stage_per;
-    return cs < 1 ? 1 : cs;
-}
-
 /* the segment-state scratch of nb rows of nv samples (none when a row fits one segment) */
 static int reserve_segments(vv_dsp_sos* h, size_t nb, size_t nv)
 {
     const size_t segs = (nv + h->segment - 1) / h->segment;
-    return segs > 1 ? reserve(h, &h->d_seg, &h->seg_bytes, nb * segs * 2 * h->sections * sizeof(float)) : 0;
+    if (segs < 2) return 0;
+    return vvdsp_internal_reserve(&h->core, (void**)&h->d_seg, &h->seg_bytes, nb * segs * 2 * h->sections * sizeof(float));
 }
 
 static void call_init(const vv_dsp_sos* h, vvb_iir_call* c)
@@ -272,12 +219,12 @@ static int pass_state(vv_dsp_sos* h, const vv_dsp_real* zi, vv_dsp_mem_space zi_
     const size_t bytes = 2 * h->sections * batch * sizeof(float);
     int st = 0;
     if (!zf || (const void*)zf == (const void*)zi) return 0;
-    if (!zi) st = zf_space == VV_DSP_MEM_HOST ? (memset(zf, 0, bytes), 0) : vvb_memset(zf, 0, bytes, h->stream);
+    if (!zi) st = zf_space == VV_DSP_MEM_HOST ? (memset(zf, 0, bytes), 0) : vvb_memset(zf, 0, bytes, h->core.stream);
     else if (zi_space == VV_DSP_MEM_HOST && zf_space == VV_DSP_MEM_HOST) memcpy(zf, zi, bytes);
-    else if (zi_space == VV_DSP_MEM_HOST) st = vvb_memcpy_h2d(zf, zi, bytes, h->stream);
-    else if (zf_space == VV_DSP_MEM_HOST) st = vvb_memcpy_d2h(zf, zi, bytes, h->stream);
-    else st = vvb_memcpy2d_d2d(zf, bytes, zi, bytes, bytes, 1, h->stream);
-    if (!st && (zi_space == VV_DSP_MEM_HOST || zf_space == VV_DSP_MEM_HOST)) st = vvb_stream_sync(h->stream);
+    else if (zi_space == VV_DSP_MEM_HOST) st = vvb_memcpy_h2d(zf, zi, bytes, h->core.stream);
+    else if (zf_space == VV_DSP_MEM_HOST) st = vvb_memcpy_d2h(zf, zi, bytes, h->core.stream);
+    else st = vvb_memcpy2d_d2d(zf, bytes, zi, bytes, bytes, 1, h->core.stream);
+    if (!st && (zi_space == VV_DSP_MEM_HOST || zf_space == VV_DSP_MEM_HOST)) st = vvb_stream_sync(h->core.stream);
     return st;
 }
 
@@ -290,13 +237,13 @@ static int filter_impl(vv_dsp_sos* h, const vv_dsp_real* signals, vv_dsp_mem_spa
     const size_t y_per = out_space == VV_DSP_MEM_HOST ? row_bytes : 0;
     const int zi_host = zi && zi_space == VV_DSP_MEM_HOST, zf_host = zf && zf_space == VV_DSP_MEM_HOST;
     const int any_host = x_per || y_per || zi_host || zf_host;
-    const size_t cs = chunk_rows(h, batch, x_per > y_per ? x_per : y_per);
+    const size_t cs = vvdsp_internal_chunk_rows(&h->core, batch, x_per > y_per ? x_per : y_per);
     size_t done;
     int st = 0;
-    if (x_per) st = reserve(h, &h->d_x, &h->x_bytes, cs * x_per);
-    if (!st && y_per) st = reserve(h, &h->d_y, &h->y_bytes, cs * y_per);
-    if (!st && zi_host) st = reserve(h, &h->d_zi, &h->zi_bytes, cs * state_row);
-    if (!st && zf_host) st = reserve(h, &h->d_zf, &h->zf_bytes, cs * state_row);
+    if (x_per) st = vvdsp_internal_reserve(&h->core, (void**)&h->d_x, &h->x_bytes, cs * x_per);
+    if (!st && y_per) st = vvdsp_internal_reserve(&h->core, (void**)&h->d_y, &h->y_bytes, cs * y_per);
+    if (!st && zi_host) st = vvdsp_internal_reserve(&h->core, (void**)&h->d_zi, &h->zi_bytes, cs * state_row);
+    if (!st && zf_host) st = vvdsp_internal_reserve(&h->core, (void**)&h->d_zf, &h->zf_bytes, cs * state_row);
     if (!st) st = reserve_segments(h, cs, n);
     /* every chunk runs on the handle's stream, so stream order keeps the scratch buffers of consecutive chunks apart */
     for (done = 0; done < batch && !st; done += cs) {
@@ -307,7 +254,7 @@ static int filter_impl(vv_dsp_sos* h, const vv_dsp_real* signals, vv_dsp_mem_spa
         c.y = out + done * out_pitch; c.y_pitch = out_pitch; c.out_mode = VVB_IIR_OUT_DIRECT;
         c.batch = nb;
         if (x_per) {
-            st = vvb_memcpy2d_h2d(h->d_x, row_bytes, c.x, signal_pitch * sizeof(float), row_bytes, nb, h->stream);
+            st = vvb_memcpy2d_h2d(h->d_x, row_bytes, c.x, signal_pitch * sizeof(float), row_bytes, nb, h->core.stream);
             c.x = h->d_x; c.x_pitch = n;
         }
         if (y_per) { c.y = h->d_y; c.y_pitch = n; }
@@ -315,7 +262,7 @@ static int filter_impl(vv_dsp_sos* h, const vv_dsp_real* signals, vv_dsp_mem_spa
             c.zi = zi + 2 * done; c.zi_sstride = 2 * batch; c.zi_rstride = 2;
             if (zi_host && !st) {
                 st = vvb_memcpy2d_h2d(h->d_zi, 2 * nb * sizeof(float), c.zi, 2 * batch * sizeof(float), 2 * nb * sizeof(float),
-                                      S, h->stream);
+                                      S, h->core.stream);
                 c.zi = h->d_zi; c.zi_sstride = 2 * nb;
             }
         }
@@ -323,15 +270,15 @@ static int filter_impl(vv_dsp_sos* h, const vv_dsp_real* signals, vv_dsp_mem_spa
             c.zf = zf_host ? h->d_zf : zf + 2 * done;
             c.zf_sstride = zf_host ? 2 * nb : 2 * batch;
         }
-        if (!st) st = vvb_iir_sos(&c, h->stream);
+        if (!st) st = vvb_iir_sos(&c, h->core.stream);
         if (!st && y_per)
-            st = vvb_memcpy2d_d2h(out + done * out_pitch, out_pitch * sizeof(float), h->d_y, row_bytes, row_bytes, nb, h->stream);
+            st = vvb_memcpy2d_d2h(out + done * out_pitch, out_pitch * sizeof(float), h->d_y, row_bytes, row_bytes, nb,
+                                  h->core.stream);
         if (!st && zf_host)
             st = vvb_memcpy2d_d2h(zf + 2 * done, 2 * batch * sizeof(float), h->d_zf, 2 * nb * sizeof(float),
-                                  2 * nb * sizeof(float), S, h->stream);
+                                  2 * nb * sizeof(float), S, h->core.stream);
     }
-    if (any_host) { int s2 = vvb_stream_sync(h->stream); if (!st) st = s2; }
-    return st;
+    return vvdsp_internal_finish(&h->core, st, any_host);
 }
 
 vv_dsp_status vv_dsp_sos_filter_batch(vv_dsp_sos* h, const vv_dsp_real* signals, vv_dsp_mem_space signals_space, size_t batch,
@@ -348,12 +295,12 @@ vv_dsp_status vv_dsp_sos_filter_batch(vv_dsp_sos* h, const vv_dsp_real* signals,
     if (signal_pitch < n || out_pitch < n) return VV_DSP_ERROR_INVALID_SIZE;
     if ((const void*)out == (const void*)signals) return VV_DSP_ERROR_UNSUPPORTED;      /* no in-place filtering */
     if (batch == 0) return VV_DSP_OK;
-    prev = dev_enter(h);
+    prev = vvdsp_internal_enter(&h->core);
     st = n == 0 ? pass_state(h, zi, zi_space, zf, zf_space, batch)
                 : filter_impl(h, signals, signals_space, batch, n, signal_pitch, zi, zi_space, zf, zf_space, out, out_space,
                               out_pitch);
-    dev_leave(prev);
-    return map_status(st);
+    vvdsp_internal_leave(prev);
+    return vvdsp_internal_status(st);
 }
 
 static int filtfilt_impl(vv_dsp_sos* h, const vv_dsp_real* signals, vv_dsp_mem_space signals_space, size_t batch, size_t n,
@@ -363,12 +310,12 @@ static int filtfilt_impl(vv_dsp_sos* h, const vv_dsp_real* signals, vv_dsp_mem_s
     const size_t nv = n + 2 * pad, row_bytes = n * sizeof(float);
     const size_t x_per = signals_space == VV_DSP_MEM_HOST ? row_bytes : 0;
     const size_t y_per = out_space == VV_DSP_MEM_HOST ? row_bytes : 0;
-    const size_t cs = chunk_rows(h, batch, x_per > y_per ? x_per : y_per);
+    const size_t cs = vvdsp_internal_chunk_rows(&h->core, batch, x_per > y_per ? x_per : y_per);
     size_t done;
     int st = 0;
-    if (x_per) st = reserve(h, &h->d_x, &h->x_bytes, cs * x_per);
-    if (!st && y_per) st = reserve(h, &h->d_y, &h->y_bytes, cs * y_per);
-    if (!st) st = reserve(h, &h->d_fwd, &h->fwd_bytes, cs * nv * sizeof(float));
+    if (x_per) st = vvdsp_internal_reserve(&h->core, (void**)&h->d_x, &h->x_bytes, cs * x_per);
+    if (!st && y_per) st = vvdsp_internal_reserve(&h->core, (void**)&h->d_y, &h->y_bytes, cs * y_per);
+    if (!st) st = vvdsp_internal_reserve(&h->core, (void**)&h->d_fwd, &h->fwd_bytes, cs * nv * sizeof(float));
     if (!st) st = reserve_segments(h, cs, nv);
     for (done = 0; done < batch && !st; done += cs) {
         const size_t nb = batch - done < cs ? batch - done : cs;
@@ -376,7 +323,7 @@ static int filtfilt_impl(vv_dsp_sos* h, const vv_dsp_real* signals, vv_dsp_mem_s
         const float* x = signals + done * signal_pitch;
         size_t xp = signal_pitch;
         if (x_per) {
-            st = vvb_memcpy2d_h2d(h->d_x, row_bytes, x, signal_pitch * sizeof(float), row_bytes, nb, h->stream);
+            st = vvb_memcpy2d_h2d(h->d_x, row_bytes, x, signal_pitch * sizeof(float), row_bytes, nb, h->core.stream);
             x = h->d_x; xp = n;
         }
         /* forward over the padded rows, from sosfilt_zi x_ext[0], into the scratch */
@@ -385,16 +332,16 @@ static int filtfilt_impl(vv_dsp_sos* h, const vv_dsp_real* signals, vv_dsp_mem_s
         c.y = h->d_fwd; c.y_pitch = nv; c.out_mode = VVB_IIR_OUT_DIRECT;
         c.zi = h->d_zi_unit; c.zi_sstride = 2; c.zi_rstride = 0; c.zi_scale_first = 1;
         c.batch = nb;
-        if (!st) st = vvb_iir_sos(&c, h->stream);
+        if (!st) st = vvb_iir_sos(&c, h->core.stream);
         /* backward over the reversed scratch, from sosfilt_zi y_fwd[last], reversed again and trimmed into out */
         c.x = h->d_fwd; c.x_pitch = nv; c.in_mode = VVB_IIR_IN_REV;
         c.y = y_per ? h->d_y : out + done * out_pitch; c.y_pitch = y_per ? n : out_pitch; c.out_mode = VVB_IIR_OUT_REVTRIM;
-        if (!st) st = vvb_iir_sos(&c, h->stream);
+        if (!st) st = vvb_iir_sos(&c, h->core.stream);
         if (!st && y_per)
-            st = vvb_memcpy2d_d2h(out + done * out_pitch, out_pitch * sizeof(float), h->d_y, row_bytes, row_bytes, nb, h->stream);
+            st = vvb_memcpy2d_d2h(out + done * out_pitch, out_pitch * sizeof(float), h->d_y, row_bytes, row_bytes, nb,
+                                  h->core.stream);
     }
-    if (x_per || y_per) { int s2 = vvb_stream_sync(h->stream); if (!st) st = s2; }
-    return st;
+    return vvdsp_internal_finish(&h->core, st, x_per || y_per);
 }
 
 vv_dsp_status vv_dsp_sos_filtfilt_batch(vv_dsp_sos* h, const vv_dsp_real* signals, vv_dsp_mem_space signals_space,
@@ -414,8 +361,8 @@ vv_dsp_status vv_dsp_sos_filtfilt_batch(vv_dsp_sos* h, const vv_dsp_real* signal
     if (n > 0 && n <= pad) return VV_DSP_ERROR_INVALID_SIZE;
     if ((const void*)out == (const void*)signals) return VV_DSP_ERROR_UNSUPPORTED;
     if (batch == 0 || n == 0) return VV_DSP_OK;
-    prev = dev_enter(h);
+    prev = vvdsp_internal_enter(&h->core);
     st = filtfilt_impl(h, signals, signals_space, batch, n, signal_pitch, padtype, pad, out, out_space, out_pitch);
-    dev_leave(prev);
-    return map_status(st);
+    vvdsp_internal_leave(prev);
+    return vvdsp_internal_status(st);
 }

@@ -22,9 +22,6 @@
 #define NORM_CACHE 4
 #define NSLOT 4            /* slots 0,1: analysis (host -> device staging); slots 2,3: synthesis (device -> host) */
 #define NDEP 64            /* per-chunk completion events of the last stream-ordered analysis call */
-/* per slot and direction (default; see stage_target below).  e2e step of the headline shape against the chunk size, same box:
- * 192 MB 45.8 ms, 96 MB 44.9, 48 MB 45.2, 24 MB 47.3 (the first chunk's upload and the last chunk's download are not overlapped) */
-#define STAGE_TARGET_BYTES ((size_t)96 << 20)
 
 typedef struct stage_slot {
     void* stream;
@@ -38,9 +35,7 @@ struct vv_dsp_stft {
     vv_dsp_stft_window win_type;
     vv_dsp_real* win;                 /* host copy of the window (bit-identical to the reference's) */
     vvb_engine* eng;
-    int device;                       /* the CUDA device the handle was created on: every entry point runs there */
-    void* own_stream;
-    void* stream;                     /* own_stream or the caller's */
+    handle_core core;
     /* per-frame staging */
     float* h_in;   vvb_cpx* h_spec;   float* h_frame;   /* pinned */
     float* d_in;   vvb_cpx* d_spec;   float* d_frame;
@@ -52,7 +47,6 @@ struct vv_dsp_stft {
     int zero_copy;                    /* per-frame calls: the kernels read / write the pinned staging buffers directly */
     struct { const char* lo; const char* hi; void* ev; int valid; } dep[NDEP];
     int dep_next;
-    size_t stage_target;              /* staging bytes per slot and direction */
     /* log-mel chain: power scratch (grown on demand) and the last filterbank in device-sparse form */
     float* d_mel_scratch; size_t mel_scratch_bytes;
     mel_device mel; const float* mel_key_ptr; size_t mel_key_n; unsigned long long mel_key_hash;
@@ -64,28 +58,14 @@ struct vv_dsp_stft {
     int norm_next;
 };
 
-static vv_dsp_status map_status(int st)
-{
-    if (st == 0) return VV_DSP_OK;
-    if (st >= 1 && st <= 6 && st != 5) return (vv_dsp_status)st;
-    return VV_DSP_ERROR_INTERNAL;
-}
-
-/* A handle lives on the device that was current when it was created.  Entry points switch to it when the caller's
- * current device is another one and switch back before returning (multi-device callers: csrc/host/stream.c). */
-static int dev_enter(const vv_dsp_stft* h)
-{
-    int cur = -1;
-    if (!h || vvb_get_device(&cur) != 0 || cur == h->device) return -1;
-    return vvb_set_device(h->device) == 0 ? cur : -1;
-}
-static void dev_leave(int prev) { if (prev >= 0) vvb_set_device(prev); }
-
 const char* vv_dsp_b200_version(void) { return "vv-dsp_b200 0.1.0 (sm_100a)"; }
 const char* vv_dsp_b200_last_error(void) { return vvb_last_error(); }
 unsigned long long vv_dsp_b200_kernel_launches(void) { return vvb_kernel_launches(); }
-vv_dsp_status vv_dsp_b200_fp32_peak(int packed, double* tflops) { return map_status(vvb_fp32_peak(packed, tflops)); }
-vv_dsp_status vv_dsp_b200_sm_clock_mhz(void* cuda_stream, double* mhz) { return map_status(vvb_sm_clock_mhz(cuda_stream, mhz)); }
+vv_dsp_status vv_dsp_b200_fp32_peak(int packed, double* tflops) { return vvdsp_internal_status(vvb_fp32_peak(packed, tflops)); }
+vv_dsp_status vv_dsp_b200_sm_clock_mhz(void* cuda_stream, double* mhz)
+{
+    return vvdsp_internal_status(vvb_sm_clock_mhz(cuda_stream, mhz));
+}
 
 /* ---------------------------------------------------------------- create / destroy */
 static void handle_free(vv_dsp_stft* h)
@@ -103,7 +83,7 @@ static void handle_free(vv_dsp_stft* h)
     vvb_host_free(h->h_in); vvb_host_free(h->h_spec); vvb_host_free(h->h_frame);
     vvb_free(h->d_in); vvb_free(h->d_spec); vvb_free(h->d_frame);
     vvb_engine_destroy(h->eng);
-    if (h->own_stream) vvb_stream_destroy(h->own_stream);
+    vvdsp_internal_core_free(&h->core);
     free(h->win);
     free(h);
 }
@@ -121,11 +101,6 @@ vv_dsp_status vv_dsp_stft_create(const vv_dsp_stft_params* params, vv_dsp_stft**
     if (!h) return VV_DSP_ERROR_INTERNAL;
     h->nfft = params->fft_size; h->hop = params->hop_size; h->bins = h->nfft / 2 + 1;
     h->win_type = params->window;
-    h->stage_target = STAGE_TARGET_BYTES;
-    {   /* test hook: a small staging size makes a modest batch span many chunks (tests/test_gpu_parity.py) */
-        const char* env = getenv("VVB_STAGE_TARGET_BYTES");
-        if (env && atol(env) > 0) h->stage_target = (size_t)atol(env);
-    }
     h->win = (vv_dsp_real*)malloc(h->nfft * sizeof(vv_dsp_real));
     if (!h->win) { handle_free(h); return VV_DSP_ERROR_INTERNAL; }
     switch (params->window) {
@@ -135,11 +110,8 @@ vv_dsp_status vv_dsp_stft_create(const vv_dsp_stft_params* params, vv_dsp_stft**
     default: ws = VV_DSP_ERROR_OUT_OF_RANGE; break;
     }
     if (ws != VV_DSP_OK) { handle_free(h); return ws; }
-    st = vvb_device_ready();                      /* 6 = no usable device: reported as UNSUPPORTED, never a CPU fallback */
-    if (!st) st = vvb_get_device(&h->device);
+    st = vvdsp_internal_core_init(&h->core);
     if (!st) st = vvb_engine_create(h->nfft, h->hop, h->win, &h->eng);
-    if (!st) st = vvb_stream_create(&h->own_stream);
-    h->stream = h->own_stream;
     if (!st) st = vvb_host_alloc((void**)&h->h_in, h->nfft * sizeof(float));
     if (!st) st = vvb_host_alloc((void**)&h->h_spec, h->bins * sizeof(vvb_cpx));
     if (!st) st = vvb_host_alloc((void**)&h->h_frame, h->nfft * sizeof(float));
@@ -170,15 +142,16 @@ static vv_dsp_status process_impl(vv_dsp_stft* h, const vv_dsp_real* in, vv_dsp_
     if (h->zero_copy) {
         /* one launch instead of copy + launch + copy: the pinned staging buffers are mapped into the device's address
          * space (unified addressing), so the kernel reads the frame and writes the spectrum over the host link itself */
-        st = vvb_stft_forward(h->eng, h->h_in, 1, h->nfft, h->nfft, 1, VVB_PAD_ZERO, VVB_OUT_COMPLEX, h->h_spec, h->bins, h->stream);
+        st = vvb_stft_forward(h->eng, h->h_in, 1, h->nfft, h->nfft, 1, VVB_PAD_ZERO, VVB_OUT_COMPLEX, h->h_spec, h->bins,
+                              h->core.stream);
     } else {
-        st = vvb_memcpy_h2d(h->d_in, h->h_in, h->nfft * sizeof(float), h->stream);
+        st = vvb_memcpy_h2d(h->d_in, h->h_in, h->nfft * sizeof(float), h->core.stream);
         if (!st) st = vvb_stft_forward(h->eng, h->d_in, 1, h->nfft, h->nfft, 1, VVB_PAD_ZERO, VVB_OUT_COMPLEX,
-                                       h->d_spec, h->bins, h->stream);
-        if (!st) st = vvb_memcpy_d2h(h->h_spec, h->d_spec, h->bins * sizeof(vvb_cpx), h->stream);
+                                       h->d_spec, h->bins, h->core.stream);
+        if (!st) st = vvb_memcpy_d2h(h->h_spec, h->d_spec, h->bins * sizeof(vvb_cpx), h->core.stream);
     }
-    if (!st) st = vvb_stream_sync(h->stream);
-    if (st) return map_status(st);
+    if (!st) st = vvb_stream_sync(h->core.stream);
+    if (st) return vvdsp_internal_status(st);
     /* bins 0..nfft/2 from the device; the rest is the conjugate mirror of a real input's spectrum */
     for (k = 0; k < h->bins; ++k) { out[k].re = h->h_spec[k].re; out[k].im = h->h_spec[k].im; }
     for (k = 1; k < h->bins; ++k)
@@ -199,14 +172,14 @@ static vv_dsp_status reconstruct_impl(vv_dsp_stft* h, const vv_dsp_cpx* in, vv_d
         h->h_spec[k].im = 0.5f * (a.im - b.im);
     }
     if (h->zero_copy) {
-        st = vvb_stft_inverse_frames(h->eng, h->h_spec, 1, h->bins, h->h_frame, h->stream);
+        st = vvb_stft_inverse_frames(h->eng, h->h_spec, 1, h->bins, h->h_frame, h->core.stream);
     } else {
-        st = vvb_memcpy_h2d(h->d_spec, h->h_spec, h->bins * sizeof(vvb_cpx), h->stream);
-        if (!st) st = vvb_stft_inverse_frames(h->eng, h->d_spec, 1, h->bins, h->d_frame, h->stream);
-        if (!st) st = vvb_memcpy_d2h(h->h_frame, h->d_frame, n * sizeof(float), h->stream);
+        st = vvb_memcpy_h2d(h->d_spec, h->h_spec, h->bins * sizeof(vvb_cpx), h->core.stream);
+        if (!st) st = vvb_stft_inverse_frames(h->eng, h->d_spec, 1, h->bins, h->d_frame, h->core.stream);
+        if (!st) st = vvb_memcpy_d2h(h->h_frame, h->d_frame, n * sizeof(float), h->core.stream);
     }
-    if (!st) st = vvb_stream_sync(h->stream);
-    if (st) return map_status(st);
+    if (!st) st = vvb_stream_sync(h->core.stream);
+    if (st) return vvdsp_internal_status(st);
     for (i = 0; i < n; ++i) {
         out_add[i] += h->h_frame[i];
         if (norm_add) norm_add[i] += h->win[i] * h->win[i];
@@ -231,20 +204,18 @@ size_t vv_dsp_stft_num_frames(const vv_dsp_stft* h, size_t n, vv_dsp_frame_conve
 
 vv_dsp_status vv_dsp_stft_set_stream(vv_dsp_stft* h, void* cuda_stream)
 {
-    if (!h) return VV_DSP_ERROR_NULL_POINTER;
-    h->stream = cuda_stream ? cuda_stream : h->own_stream;
-    return VV_DSP_OK;
+    return vvdsp_internal_set_stream(h ? &h->core : NULL, cuda_stream);
 }
 
 static vv_dsp_status synchronize_impl(vv_dsp_stft* h)
 {
     int i, st;
     if (!h) return VV_DSP_ERROR_NULL_POINTER;
-    st = vvb_stream_sync(h->stream);
+    st = vvb_stream_sync(h->core.stream);
     for (i = 0; i < NSLOT; ++i)
         if (h->slot[i].stream) { int s2 = vvb_stream_sync(h->slot[i].stream); if (!st) st = s2; }
     for (i = 0; i < NDEP; ++i) h->dep[i].valid = 0;
-    return map_status(st);
+    return vvdsp_internal_status(st);
 }
 
 vv_dsp_status vv_dsp_stft_set_async(vv_dsp_stft* h, int enable)
@@ -298,14 +269,6 @@ static int slot_reserve(stage_slot* s, size_t in_bytes, size_t out_bytes)
     return st;
 }
 
-static size_t chunk_signals(const vv_dsp_stft* h, size_t batch, size_t bytes_per_signal)
-{
-    size_t c = bytes_per_signal ? h->stage_target / bytes_per_signal : batch;
-    if (c < 1) c = 1;
-    if (c > batch) c = batch;
-    return c;
-}
-
 /* ------------------------------------------------------------------ batched forward */
 /* pcm_format 0: `signals_v` are float32 samples; 16 / 24 / 32 / -32: HOST rows of little-endian PCM (or float32) samples as
  * they sit in a WAV data chunk (mono, one signal per row, pitch in samples), decoded on the device chunk by chunk with the
@@ -334,15 +297,15 @@ static vv_dsp_status batch_forward_impl(vv_dsp_stft* h, const void* signals_v, i
     esize = (kind == VV_DSP_SPEC_COMPLEX) ? sizeof(vvb_cpx) : sizeof(float);
 
     if (signals_space == VV_DSP_MEM_DEVICE && out_space == VV_DSP_MEM_DEVICE)
-        return map_status(vvb_stft_forward(h->eng, signals, batch, n, signal_pitch, frames, pad, (int)kind, out,
-                                           spec_pitch, h->stream));
+        return vvdsp_internal_status(vvb_stft_forward(h->eng, signals, batch, n, signal_pitch, frames, pad, (int)kind, out,
+                                                      spec_pitch, h->core.stream));
 
     /* at least one side lives in host memory: stream chunks of signals through two slots */
     {
         const size_t in_per = (signals_space == VV_DSP_MEM_HOST) ? (n ? n : 1) * sizeof(float) : 0;
         const size_t out_per = (out_space == VV_DSP_MEM_HOST) ? frames * h->bins * esize : 0;
-        const size_t cs = chunk_signals(h, batch, in_per > out_per ? in_per : out_per);
-        if (!h->async) st = vvb_stream_sync(h->stream);   /* device-side operands may still be in flight */
+        const size_t cs = vvdsp_internal_chunk_rows(&h->core, batch, in_per > out_per ? in_per : out_per);
+        if (!h->async) st = vvb_stream_sync(h->core.stream);   /* device-side operands may still be in flight */
         for (done = 0; done < batch && !st; done += cs, ++c) {
             /* sizes without a Stockham kernel keep per-engine scratch buffers (chirp-z work buffer, synthesis frames):
              * their chunks all run on ONE stream, in order, in both directions */
@@ -391,7 +354,7 @@ static vv_dsp_status batch_forward_impl(vv_dsp_stft* h, const void* signals_v, i
             for (c = 0; c < NSLOT; ++c)
                 if (h->slot[c].stream) { int s2 = vvb_stream_sync(h->slot[c].stream); if (!st) st = s2; }
     }
-    return map_status(st);
+    return vvdsp_internal_status(st);
 }
 
 /* --------------------------------------------------- 1/sum(w^2) tables for the ISTFT */
@@ -431,12 +394,12 @@ static int norm_tables(vv_dsp_stft* h, size_t frames, const float** d_tab)
     }
     for (i = 0; i < edge; ++i) host[edge + h->hop + i] = inv_norm_at(h, frames, frames * h->hop + i);  /* tail */
     k = h->norm_next; h->norm_next = (h->norm_next + 1) % NORM_CACHE;
-    st = vvb_stream_sync(h->stream);                 /* the evicted table may still be in use */
+    st = vvb_stream_sync(h->core.stream);            /* the evicted table may still be in use */
     for (i = 0; i < NSLOT && !st; ++i) if (h->slot[i].stream) st = vvb_stream_sync(h->slot[i].stream);
     vvb_free(h->norm[k].d_tab); h->norm[k].d_tab = NULL; h->norm[k].used = 0;
     if (!st) st = vvb_malloc((void**)&h->norm[k].d_tab, total * sizeof(float));
-    if (!st) st = vvb_memcpy_h2d(h->norm[k].d_tab, host, total * sizeof(float), h->stream);
-    if (!st) st = vvb_stream_sync(h->stream);
+    if (!st) st = vvb_memcpy_h2d(h->norm[k].d_tab, host, total * sizeof(float), h->core.stream);
+    if (!st) st = vvb_stream_sync(h->core.stream);
     free(host);
     if (st) return st;
     h->norm[k].frames = frames; h->norm[k].used = 1;
@@ -459,16 +422,16 @@ static vv_dsp_status batch_inverse_impl(vv_dsp_stft* h, const vv_dsp_cpx* spectr
     if (out_pitch == 0) out_pitch = n_out;
     if (spec_pitch < h->bins || out_pitch < n_out) return VV_DSP_ERROR_INVALID_SIZE;
     if (batch == 0 || n_out == 0) return VV_DSP_OK;
-    if (normalise) { st = norm_tables(h, frames, &d_tab); if (st) return map_status(st); }
+    if (normalise) { st = norm_tables(h, frames, &d_tab); if (st) return vvdsp_internal_status(st); }
 
     if (spectra_space == VV_DSP_MEM_DEVICE && out_space == VV_DSP_MEM_DEVICE)
-        return map_status(vvb_stft_inverse(h->eng, (const vvb_cpx*)spectra, batch, frames, spec_pitch, out, n_out,
-                                           out_pitch, d_tab, h->stream));
+        return vvdsp_internal_status(vvb_stft_inverse(h->eng, (const vvb_cpx*)spectra, batch, frames, spec_pitch, out, n_out,
+                                                      out_pitch, d_tab, h->core.stream));
     {
         const size_t in_per = (spectra_space == VV_DSP_MEM_HOST) ? frames * h->bins * sizeof(vvb_cpx) : 0;
         const size_t out_per = (out_space == VV_DSP_MEM_HOST) ? n_out * sizeof(float) : 0;
-        const size_t cs = chunk_signals(h, batch, in_per > out_per ? in_per : out_per);
-        if (!h->async) st = vvb_stream_sync(h->stream);
+        const size_t cs = vvdsp_internal_chunk_rows(&h->core, batch, in_per > out_per ? in_per : out_per);
+        if (!h->async) st = vvb_stream_sync(h->core.stream);
         for (done = 0; done < batch && !st; done += cs, ++c) {
             stage_slot* s = &h->slot[fast ? 2 + c % 2 : 0];            /* own streams: D2H overlaps the analysis H2D */
             const size_t nb = (batch - done < cs) ? batch - done : cs;
@@ -502,7 +465,7 @@ static vv_dsp_status batch_inverse_impl(vv_dsp_stft* h, const vv_dsp_cpx* spectr
             for (c = 0; c < NSLOT; ++c)
                 if (h->slot[c].stream) { int s2 = vvb_stream_sync(h->slot[c].stream); if (!st) st = s2; }
     }
-    return map_status(st);
+    return vvdsp_internal_status(st);
 }
 
 vv_dsp_status vv_dsp_stft_istft(vv_dsp_stft* h, const vv_dsp_cpx* half_spectra, size_t frames, vv_dsp_real* out, size_t n_out)
@@ -575,7 +538,7 @@ static vv_dsp_status batch_mel_chain(vv_dsp_stft* h, const void* signals_v, int 
     pad = (convention == VV_DSP_FRAMES_CENTER) ? VVB_PAD_REFLECT_CENTER : VVB_PAD_ZERO;
     per_signal = frames * h->bins * sizeof(float);
     cs = scratch_target / per_signal; if (cs < 1) cs = 1; if (cs > batch) cs = batch;
-    stream = h->stream;
+    stream = h->core.stream;
     /* the device-sparse filterbank is cached per handle; fingerprint = pointer, size and an FNV-1a hash of EVERY weight
      * (about 80 k words: negligible next to the kernels, and an in-place edit of any weight is seen) */
     for (i = 0; i < n_mels * h->bins; ++i) {
@@ -600,23 +563,17 @@ static vv_dsp_status batch_mel_chain(vv_dsp_stft* h, const void* signals_v, int 
                                                     : mode ? "one fused kernel, band sums per warp" : "power kernel + log-mel kernel");
     }
     if (fused) {
-        const size_t stage_target = h->stage_target;                   /* VVB_STAGE_TARGET_BYTES applies here too */
         cs = batch;
         if (signals_space == VV_DSP_MEM_HOST || out_space == VV_DSP_MEM_HOST) {
             const size_t per = (n ? n : 1) * sizeof(float) + frames * n_mels * sizeof(float);
-            cs = stage_target / per;
+            cs = h->core.stage_target / per;                            /* VVB_STAGE_TARGET_BYTES applies here too */
         } else if (n_coeffs) {
             cs = scratch_target / (frames * n_mels * sizeof(float));    /* the log-mel rows between the two kernels */
         }
         if (cs < 1) cs = 1;
         if (cs > batch) cs = batch;
     }
-    if (!st && !fused && h->mel_scratch_bytes < cs * per_signal) {
-        st = vvb_stream_sync(stream);
-        vvb_free(h->d_mel_scratch); h->d_mel_scratch = NULL; h->mel_scratch_bytes = 0;
-        if (!st) st = vvb_malloc((void**)&h->d_mel_scratch, cs * per_signal);
-        if (!st) h->mel_scratch_bytes = cs * per_signal;
-    }
+    if (!st && !fused) st = vvdsp_internal_reserve(&h->core, (void**)&h->d_mel_scratch, &h->mel_scratch_bytes, cs * per_signal);
     d_power = h->d_mel_scratch;
     if (!st && n_coeffs) {
         if (!h->mfcc.d_table || h->mfcc.n_mels != n_mels || h->mfcc.n_coeffs != n_coeffs || h->mfcc.lifter != lifter) {
@@ -624,12 +581,9 @@ static vv_dsp_status batch_mel_chain(vv_dsp_stft* h, const void* signals_v, int 
             vvdsp_internal_mfcc_device_free(&h->mfcc);
             if (!st) st = vvdsp_internal_mfcc_device_build(n_mels, n_coeffs, lifter, stream, &h->mfcc);
         }
-        if (!st && h->logmel_scratch_bytes < cs * frames * n_mels * sizeof(float)) {
-            st = vvb_stream_sync(stream);
-            vvb_free(h->d_logmel_scratch); h->d_logmel_scratch = NULL; h->logmel_scratch_bytes = 0;
-            if (!st) st = vvb_malloc((void**)&h->d_logmel_scratch, cs * frames * n_mels * sizeof(float));
-            if (!st) h->logmel_scratch_bytes = cs * frames * n_mels * sizeof(float);
-        }
+        if (!st)
+            st = vvdsp_internal_reserve(&h->core, (void**)&h->d_logmel_scratch, &h->logmel_scratch_bytes,
+                                        cs * frames * n_mels * sizeof(float));
     }
     if (!st && fused && signals_space == VV_DSP_MEM_HOST && batch > cs) {
         /* host signals through the fused kernel, more than one chunk: two staging sets on the handle's two slot streams, so
@@ -671,7 +625,7 @@ static vv_dsp_status batch_mel_chain(vv_dsp_stft* h, const void* signals_v, int 
             if (ps[k]) { int s2 = vvb_stream_sync(ps[k]); if (!st) st = s2; }
             vvb_free(px[k]); vvb_free(po[k]); vvb_free(pl[k]); vvb_free(pr[k]);
         }
-        return map_status(st);
+        return vvdsp_internal_status(st);
     }
     if (!st && signals_space == VV_DSP_MEM_HOST) st = vvb_malloc((void**)&d_x, cs * (n ? n : 1) * sizeof(float));
     if (!st && pcm_format) st = vvb_malloc(&d_raw, cs * (n ? n : 1) * bps);
@@ -712,7 +666,7 @@ static vv_dsp_status batch_mel_chain(vv_dsp_stft* h, const void* signals_v, int 
         int s2 = vvb_stream_sync(stream); if (!st) st = s2;
         vvb_free(d_x); vvb_free(d_o); vvb_free(d_raw);
     }
-    return map_status(st);
+    return vvdsp_internal_status(st);
 }
 
 vv_dsp_status vv_dsp_stft_batch_logmel_pcm(vv_dsp_stft* h, const void* pcm, int format, size_t batch, size_t n, size_t signal_pitch,
@@ -722,10 +676,10 @@ vv_dsp_status vv_dsp_stft_batch_logmel_pcm(vv_dsp_stft* h, const void* pcm, int 
     int prev;
     vv_dsp_status st;
     if (format != 16 && format != 24 && format != 32 && format != -32) return VV_DSP_ERROR_OUT_OF_RANGE;
-    prev = dev_enter(h);
+    prev = vvdsp_internal_enter(h ? &h->core : NULL);
     st = batch_mel_chain(h, pcm, format, VV_DSP_MEM_HOST, batch, n, signal_pitch, convention, filterbank_weights, n_mels, log_epsilon, 0, 0.0f,
                          out, out_space, out_frames);
-    dev_leave(prev);
+    vvdsp_internal_leave(prev);
     return st;
 }
 
@@ -734,10 +688,10 @@ vv_dsp_status vv_dsp_stft_batch_logmel(vv_dsp_stft* h, const vv_dsp_real* signal
                                        const vv_dsp_real* filterbank_weights, size_t n_mels, vv_dsp_real log_epsilon,
                                        vv_dsp_real* out, vv_dsp_mem_space out_space, size_t* out_frames)
 {
-    const int prev = dev_enter(h);
+    const int prev = vvdsp_internal_enter(h ? &h->core : NULL);
     const vv_dsp_status st = batch_mel_chain(h, signals, 0, signals_space, batch, n, signal_pitch, convention, filterbank_weights, n_mels,
                                              log_epsilon, 0, 0.0f, out, out_space, out_frames);
-    dev_leave(prev);
+    vvdsp_internal_leave(prev);
     return st;
 }
 
@@ -750,10 +704,10 @@ vv_dsp_status vv_dsp_stft_batch_mfcc(vv_dsp_stft* h, const vv_dsp_real* signals,
     int prev;
     vv_dsp_status st;
     if (num_mfcc_coeffs == 0) return VV_DSP_ERROR_INVALID_SIZE;
-    prev = dev_enter(h);
+    prev = vvdsp_internal_enter(h ? &h->core : NULL);
     st = batch_mel_chain(h, signals, 0, signals_space, batch, n, signal_pitch, convention, filterbank_weights, n_mels, log_epsilon,
                          num_mfcc_coeffs, lifter_coeff, out, out_space, out_frames);
-    dev_leave(prev);
+    vvdsp_internal_leave(prev);
     return st;
 }
 
@@ -772,37 +726,37 @@ static vv_dsp_status shard_inverse_impl(vv_dsp_stft* h, const vv_dsp_cpx* spectr
     if (!is_first && local_frames - halo_frames < h->nfft / h->hop - 1) return VV_DSP_ERROR_INVALID_SIZE;
     st = norm_tables(h, local_frames, &d_tab);
     if (!st) st = vvb_stft_inverse_shard(h->eng, (const vvb_cpx*)spectra, local_frames, halo_frames, is_first, is_last, h->bins,
-                                         out, n_out, d_tab, h->stream);
-    return map_status(st);
+                                         out, n_out, d_tab, h->core.stream);
+    return vvdsp_internal_status(st);
 }
 
 /* ------------------------------------------------- public entry points: run on the handle's device */
 vv_dsp_status vv_dsp_stft_destroy(vv_dsp_stft* h)
 {
-    const int prev = dev_enter(h);
+    const int prev = vvdsp_internal_enter(h ? &h->core : NULL);
     const vv_dsp_status st = destroy_impl(h);
-    dev_leave(prev);
+    vvdsp_internal_leave(prev);
     return st;
 }
 vv_dsp_status vv_dsp_stft_process(vv_dsp_stft* h, const vv_dsp_real* in, vv_dsp_cpx* out)
 {
-    const int prev = dev_enter(h);
+    const int prev = vvdsp_internal_enter(h ? &h->core : NULL);
     const vv_dsp_status st = process_impl(h, in, out);
-    dev_leave(prev);
+    vvdsp_internal_leave(prev);
     return st;
 }
 vv_dsp_status vv_dsp_stft_reconstruct(vv_dsp_stft* h, const vv_dsp_cpx* in, vv_dsp_real* out_add, vv_dsp_real* norm_add)
 {
-    const int prev = dev_enter(h);
+    const int prev = vvdsp_internal_enter(h ? &h->core : NULL);
     const vv_dsp_status st = reconstruct_impl(h, in, out_add, norm_add);
-    dev_leave(prev);
+    vvdsp_internal_leave(prev);
     return st;
 }
 vv_dsp_status vv_dsp_stft_synchronize(vv_dsp_stft* h)
 {
-    const int prev = dev_enter(h);
+    const int prev = vvdsp_internal_enter(h ? &h->core : NULL);
     const vv_dsp_status st = synchronize_impl(h);
-    dev_leave(prev);
+    vvdsp_internal_leave(prev);
     return st;
 }
 vv_dsp_status vv_dsp_stft_batch_forward(vv_dsp_stft* h, const vv_dsp_real* signals, vv_dsp_mem_space signals_space,
@@ -810,10 +764,10 @@ vv_dsp_status vv_dsp_stft_batch_forward(vv_dsp_stft* h, const vv_dsp_real* signa
                                         vv_dsp_frame_convention convention, vv_dsp_spec_kind kind, void* out,
                                         vv_dsp_mem_space out_space, size_t spec_pitch, size_t* out_frames)
 {
-    const int prev = dev_enter(h);
+    const int prev = vvdsp_internal_enter(h ? &h->core : NULL);
     const vv_dsp_status st = batch_forward_impl(h, signals, 0, signals_space, batch, n, signal_pitch, convention, kind, out, out_space,
                                                 spec_pitch, out_frames);
-    dev_leave(prev);
+    vvdsp_internal_leave(prev);
     return st;
 }
 vv_dsp_status vv_dsp_stft_batch_forward_pcm(vv_dsp_stft* h, const void* pcm, int format, size_t batch, size_t n, size_t signal_pitch,
@@ -823,29 +777,29 @@ vv_dsp_status vv_dsp_stft_batch_forward_pcm(vv_dsp_stft* h, const void* pcm, int
     int prev;
     vv_dsp_status st;
     if (format != 16 && format != 24 && format != 32 && format != -32) return VV_DSP_ERROR_OUT_OF_RANGE;
-    prev = dev_enter(h);
+    prev = vvdsp_internal_enter(h ? &h->core : NULL);
     st = batch_forward_impl(h, pcm, format, VV_DSP_MEM_HOST, batch, n, signal_pitch, convention, kind, out, out_space, spec_pitch, out_frames);
-    dev_leave(prev);
+    vvdsp_internal_leave(prev);
     return st;
 }
 vv_dsp_status vv_dsp_stft_batch_inverse(vv_dsp_stft* h, const vv_dsp_cpx* spectra, vv_dsp_mem_space spectra_space,
                                         size_t batch, size_t frames, size_t spec_pitch, vv_dsp_real* out,
                                         vv_dsp_mem_space out_space, size_t n_out, size_t out_pitch, int normalise)
 {
-    const int prev = dev_enter(h);
+    const int prev = vvdsp_internal_enter(h ? &h->core : NULL);
     const vv_dsp_status st = batch_inverse_impl(h, spectra, spectra_space, batch, frames, spec_pitch, out, out_space, n_out, out_pitch,
                                                 normalise);
-    dev_leave(prev);
+    vvdsp_internal_leave(prev);
     return st;
 }
 vv_dsp_status vv_dsp_stft_shard_inverse(vv_dsp_stft* h, const vv_dsp_cpx* spectra, size_t local_frames, size_t halo_frames,
                                         int is_first, int is_last, vv_dsp_real* out, size_t n_out)
 {
-    const int prev = dev_enter(h);
+    const int prev = vvdsp_internal_enter(h ? &h->core : NULL);
     const vv_dsp_status st = shard_inverse_impl(h, spectra, local_frames, halo_frames, is_first, is_last, out, n_out);
-    dev_leave(prev);
+    vvdsp_internal_leave(prev);
     return st;
 }
-int vv_dsp_stft_device(const vv_dsp_stft* h) { return h ? h->device : -1; }
-void* vv_dsp_stft_get_stream(const vv_dsp_stft* h) { return h ? h->stream : NULL; }
+int vv_dsp_stft_device(const vv_dsp_stft* h) { return h ? h->core.device : -1; }
+void* vv_dsp_stft_get_stream(const vv_dsp_stft* h) { return h ? h->core.stream : NULL; }
 const vv_dsp_real* vv_dsp_stft_window_ptr(const vv_dsp_stft* h) { return h ? h->win : NULL; }

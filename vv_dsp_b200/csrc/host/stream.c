@@ -19,6 +19,7 @@
 #include <string.h>
 #include "vv_dsp/b200.h"
 #include "vvb200_cuda.h"
+#include "internal.h"
 
 typedef struct shard {
     int device;
@@ -37,13 +38,6 @@ struct vv_dsp_stft_stream {
     shard* sh;
     int graphs_tried;
 };
-
-static vv_dsp_status map_status(int st)
-{
-    if (st == 0) return VV_DSP_OK;
-    if (st >= 1 && st <= 6 && st != 5) return (vv_dsp_status)st;
-    return VV_DSP_ERROR_INTERNAL;
-}
 
 static void stream_free(vv_dsp_stft_stream* s)
 {
@@ -79,7 +73,7 @@ vv_dsp_status vv_dsp_stft_stream_create(const vv_dsp_stft_params* params, size_t
     if (params->fft_size % params->hop_size) return VV_DSP_ERROR_UNSUPPORTED;       /* halo frames need hop | fft_size */
     if (n < params->fft_size) return VV_DSP_ERROR_INVALID_SIZE;
     st = vvb_device_count(&count);
-    if (st) return map_status(st);
+    if (st) return vvdsp_internal_status(st);
     for (d = 0; d < num_devices; ++d) {
         const int id = device_ids ? device_ids[d] : (int)d;
         if (id < 0 || id >= count) return VV_DSP_ERROR_OUT_OF_RANGE;
@@ -125,7 +119,7 @@ vv_dsp_status vv_dsp_stft_stream_create(const vv_dsp_stft_params* params, size_t
         if (!st) st = vvb_enable_peer_access(s->sh[d + 1].device, s->sh[d].device);
     }
     vvb_set_device(cur);
-    if (st) { stream_free(s); return map_status(st); }
+    if (st) { stream_free(s); return vvdsp_internal_status(st); }
     *out = s;
     return VV_DSP_OK;
 }
@@ -165,7 +159,7 @@ vv_dsp_status vv_dsp_stft_stream_synchronize(vv_dsp_stft_stream* s)
         if (!st) st = s2;
     }
     vvb_set_device(cur);
-    return map_status(st);
+    return vvdsp_internal_status(st);
 }
 
 vv_dsp_status vv_dsp_stft_stream_upload(vv_dsp_stft_stream* s, const vv_dsp_real* signal)
@@ -180,7 +174,7 @@ vv_dsp_status vv_dsp_stft_stream_upload(vv_dsp_stft_stream* s, const vv_dsp_real
         if (!st) st = vvb_memcpy_h2d(k->d_x + k->lh, signal + k->s0, (k->s1 - k->s0) * sizeof(float), k->stream);
     }
     vvb_set_device(cur);
-    if (st) return map_status(st);
+    if (st) return vvdsp_internal_status(st);
     return vv_dsp_stft_stream_synchronize(s);
 }
 
@@ -234,7 +228,7 @@ static vv_dsp_status for_each_device(vv_dsp_stft_stream* s, enqueue_fn a, enqueu
         if (!st && b) st = b(s, d);
     }
     vvb_set_device(cur);
-    return map_status(st);
+    return vvdsp_internal_status(st);
 }
 
 vv_dsp_status vv_dsp_stft_stream_forward(vv_dsp_stft_stream* s) { return for_each_device(s, enqueue_forward, NULL); }
@@ -304,7 +298,7 @@ vv_dsp_status vv_dsp_stft_stream_download(vv_dsp_stft_stream* s, vv_dsp_real* ou
         if (!st) st = vvb_memcpy_d2h(out + k->s0, k->d_y, (k->s1 - k->s0) * sizeof(float), k->stream);
     }
     vvb_set_device(cur);
-    if (st) return map_status(st);
+    if (st) return vvdsp_internal_status(st);
     return vv_dsp_stft_stream_synchronize(s);
 }
 
@@ -321,7 +315,7 @@ vv_dsp_status vv_dsp_stft_stream_download_spectra(vv_dsp_stft_stream* s, vv_dsp_
                                      (k->f1 - k->f0) * s->bins * sizeof(vvb_cpx), k->stream);
     }
     vvb_set_device(cur);
-    if (st) return map_status(st);
+    if (st) return vvdsp_internal_status(st);
     return vv_dsp_stft_stream_synchronize(s);
 }
 
@@ -361,7 +355,7 @@ vv_dsp_status vv_dsp_stft_stream_time_roundtrip(vv_dsp_stft_stream* s, size_t wa
         if ((double)ms > worst) worst = (double)ms;
     }
     vvb_set_device(cur);
-    if (st) return map_status(st);
+    if (st) return vvdsp_internal_status(st);
     *ms_per_step = worst / (double)steps;
     return VV_DSP_OK;
 }
